@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- Krotov iterations/s and state-timesteps/s of the B200 hot path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--samples S] [--n-grid G]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--samples S] [--n-grid G] [--dump-outputs DIR]
 
 A "step" is ONE Krotov iteration (backward sweep + sequential update + forward sweep,
 src/optimize.jl:279-371 of the reference) over the whole workload.  The workload is BASELINE.json's
@@ -17,6 +17,8 @@ e2e    = the same metric through the public API `optimize(problem, method=Krotov
 --impl reference times the CPU restatement of the reference (oracle/krotov_oracle.c, OpenMP over
 trajectories like the reference's @threadsif) on a bounded sample of the same workload: Julia is not
 installed in this image, so the reference itself cannot run (see DESIGN.md).
+--dump-outputs DIR writes what the last timed iteration returned (see dump_outputs) as float64 .npy files; the
+inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -216,6 +218,32 @@ def extra_configs(K, to_problem, peaks):
     return out
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(folder, pulses, g_a_int, res):
+    """The arrays a caller of the timed path receives from its last iteration, as float64 .npy files (complex arrays
+    with a trailing [re, im] axis): the new pulses (L, N_T), the g_a integrals (L,), tau (N, 2), the forward-propagated
+    final states (N, d, 2) and J_T (1,).  Beyond DUMP_BYTES in all, tau and the states are cut to a fixed, seeded
+    sample of trajectories whose indices go to trajectory_index.npy."""
+    def re_im(a):
+        a = np.asarray(a, np.complex128)
+        return np.stack([a.real, a.imag], axis=-1)
+
+    out = {"pulses": np.asarray(pulses, np.float64), "g_a_int": np.asarray(g_a_int, np.float64),
+           "tau": re_im(res.tau_vals), "states": re_im(np.array(res.states)), "J_T": np.array([res.J_T], np.float64)}
+    n = out["states"].shape[0]
+    per_traj = out["states"][0].nbytes + out["tau"][0].nbytes + 8
+    keep = (DUMP_BYTES - out["pulses"].nbytes - 4096) // per_traj
+    if keep < n:
+        rows = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+        out["tau"], out["states"] = out["tau"][rows], out["states"][rows]
+        out["trajectory_index"] = rows.astype(np.float64)
+    os.makedirs(folder, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(folder, name + ".npy"), np.ascontiguousarray(a))
+
+
 def run_reference(args):
     """`--impl reference`: CPU restatement on the host cores (rank 0 only)."""
     rank = int(os.environ.get("RANK", "0"))
@@ -273,7 +301,12 @@ def main():
                     help="several ranks: shard the trajectories (per-step exchange) or replicate the forward sweep")
     ap.add_argument("--scaling", choices=["strong", "weak"], default="strong",
                     help="strong: the BASELINE ensemble sharded over the ranks; weak: --samples per rank")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed iteration to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path; --impl reference has none")
     if args.impl == "reference":
         run_reference(args)
         return
@@ -336,6 +369,9 @@ def main():
             barrier()
             marks["t1"] = time.perf_counter()
             marks["clocks"] = sampler.stop()
+            if args.dump_outputs:
+                marks["pulses"] = np.array([np.array(e) for e in eps_new])
+                marks["g_a_int"] = np.array(wrk.g_a_int)
         marks["J_T"] = wrk.result.J_T
         marks["m_fw"] = int(wrk.fw_settings.coeff_count.max())
         marks["m_bw"] = int(wrk.bw_settings.coeff_count.max())
@@ -345,6 +381,8 @@ def main():
     res = K.optimize(problem, method=K.Krotov, comm=comm)
     if res.message.startswith("Exception"):
         raise SystemExit(f"optimisation failed: {res.message}")
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, marks["pulses"], marks["g_a_int"], res)
 
     timed_ms = np.array(dev_ms[warmup:warmup + steps])
     dev_total_ms = float(timed_ms.sum())

@@ -238,6 +238,36 @@ def test_reference_arm_uses_all_cores_even_under_torchrun_env():
     assert out.returncode == 0 and out.stdout.strip() == ""
 
 
+def test_bench_dump_outputs_float64_within_budget(tmp_path, monkeypatch):
+    """`bench.py --dump-outputs`: every array as float64 .npy, complex ones with a trailing [re, im] axis; beyond the
+    byte budget tau and the states are cut to the same seeded sample of trajectories on every run."""
+    import types
+
+    import bench
+
+    rng = np.random.default_rng(3)
+    n, d = 64, 5
+    states = rng.standard_normal((n, d)) + 1j * rng.standard_normal((n, d))
+    res = types.SimpleNamespace(tau_vals=states[:, 0].copy(), states=list(states), J_T=0.25)
+    pulses, ga = rng.standard_normal((2, 30)), rng.standard_normal(2)
+    bench.dump_outputs(str(tmp_path / "full"), pulses, ga, res)
+    got = {f[:-4]: np.load(tmp_path / "full" / f) for f in os.listdir(tmp_path / "full")}
+    assert set(got) == {"pulses", "g_a_int", "tau", "states", "J_T"}
+    assert all(a.dtype == np.float64 for a in got.values())
+    assert np.array_equal(got["pulses"], pulses) and np.array_equal(got["g_a_int"], ga) and got["J_T"].tolist() == [0.25]
+    assert np.array_equal(got["states"][..., 0] + 1j * got["states"][..., 1], states)
+    assert np.array_equal(got["tau"][:, 0] + 1j * got["tau"][:, 1], states[:, 0])
+
+    monkeypatch.setattr(bench, "DUMP_BYTES", pulses.nbytes + 4096 + 20 * (d * 16 + 16 + 8))
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), pulses, ga, res)
+        assert sum(os.path.getsize(tmp_path / run / f) for f in os.listdir(tmp_path / run)) <= bench.DUMP_BYTES
+    rows = np.load(tmp_path / "a" / "trajectory_index.npy").astype(int)
+    assert len(rows) == 20 and np.array_equal(rows, np.load(tmp_path / "b" / "trajectory_index.npy"))
+    sampled = np.load(tmp_path / "a" / "states.npy")
+    assert np.array_equal(sampled[..., 0] + 1j * sampled[..., 1], states[rows])
+
+
 def _gloo_worker(rank, world, port, out):
     import torch.distributed as dist
 
