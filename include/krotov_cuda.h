@@ -143,6 +143,10 @@ int krotov_destroy(krotov_handle h);
  * the calling thread).  Never NULL. */
 const char *krotov_last_error(krotov_handle h);
 int krotov_get_info(krotov_handle h, krotov_info *out);
+/* Device allocations and peer mappings the library currently owns, over all handles of the process.  Every
+ * krotov_destroy (and every failed krotov_create) gives back what its handle took, so a test can check for leaks
+ * by comparing this count before and after, which device-wide free memory cannot show on a shared GPU. */
+int64_t krotov_live_device_objects(void);
 
 /* ---- propagator settings --------------------------------------------------------------
  * Chebyshev polynomial of one direction.  Replaces what init_prop/reinit_prop! leave in

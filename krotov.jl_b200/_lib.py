@@ -21,7 +21,8 @@ CHI_HOST, CHI_SM, CHI_SS, CHI_RE = 0, 1, 2, 3
 PATH_WARP, PATH_DENSE, PATH_SPARSE = 1, 2, 3
 COMM_DESC_BYTES = 256
 
-# every symbol include/krotov_cuda.h declares (tests check the .so exports all of them)
+# every symbol include/krotov_cuda.h declares that returns a status code or a string (tests check the .so exports all
+# of them); krotov_live_device_objects returns a count and is bound below
 EXPORTS = [
     "krotov_abi_version", "krotov_create", "krotov_destroy", "krotov_last_error", "krotov_get_info",
     "krotov_set_cheby", "krotov_set_amplitudes", "krotov_forward", "krotov_set_chi", "krotov_set_chi_coeffs", "krotov_iterate",
@@ -103,6 +104,8 @@ def lib():
         if name not in ("krotov_last_error",):
             getattr(L, name).restype = i32
     L.krotov_last_error.restype = C.c_char_p
+    L.krotov_live_device_objects.argtypes = []
+    L.krotov_live_device_objects.restype = C.c_int64
     _lib = L
     return L
 

@@ -21,6 +21,7 @@
 //   -> m-1 GEMMs;
 // the pulse value never visits the host.
 #include "dense_kernel.cuh"
+#include "device_buffer.cuh"
 
 #include <cooperative_groups.h>
 
@@ -30,6 +31,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <memory>
 
 namespace kr {
 
@@ -980,11 +982,10 @@ struct DenseEngine {
     std::vector<Block> blocks;
     int n_partial = 0;
     // device
-    double2 *Hf = nullptr, *Hb = nullptr, *G = nullptr;
-    double2 *V[3] = {nullptr, nullptr, nullptr}, *OUT = nullptr, *PSI = nullptr, *PSI0 = nullptr, *TGT = nullptr,
-            *CHI = nullptr, *X = nullptr, *PHI = nullptr;
-    double *partial = nullptr;
-    int *d_col_of_traj = nullptr, *d_traj_of_col = nullptr;
+    DevBuf Hf, Hb, G;                                            // double2
+    DevBuf V[3], OUT, PSI, PSI0, TGT, CHI, X, PHI;               // double2
+    DevBuf partial;                                              // double
+    DevBuf d_col_of_traj, d_traj_of_col;                         // int
     bool chi_from_host = false;
     Cheb ch[2];
     size_t slab = 0;  // elements per time slot
@@ -995,16 +996,16 @@ struct DenseEngine {
     // sparse mode (ELL): shared pattern, values per generator and term for both directions
     bool sparse = false;
     int W = 0;
-    int *ell_cols = nullptr;
-    double2 *Pvf = nullptr, *Pvb = nullptr, *Gv = nullptr;  // [g][1+L][dp*W], [g][dp*W]
+    DevBuf ell_cols;      // int
+    DevBuf Pvf, Pvb, Gv;  // double2: [g][1+L][dp*W], [g][dp*W]
     std::vector<int> sp_part_off;  // offset of every column block's CTA partials
     int nnz_union = 0;
     bool x_contig = false;   // single column block stored with ld = 8 nt + 2: a B tile is one bulk copy
     size_t gmat = 0;         // elements of one tile-major generator: (dp/BM) (dp/BK) BM A_STRIDE
     // stream-K GEMM (fewer row blocks than SMs): partial tiles, ready flags
     bool streamk = false;
-    double2 *sk_ws = nullptr;
-    unsigned *sk_flags = nullptr;
+    DevBuf sk_ws;     // double2
+    DevBuf sk_flags;  // unsigned
     // whole-iteration CUDA graph (launch-bound problems): captured the second time an identical iteration is asked for
     unsigned long long cheb_version = 0;
     struct GraphKey {
@@ -1021,26 +1022,30 @@ struct DenseEngine {
     // persistent sweep (sparse path): launch shape and device copies of the small tables
     bool sweep = false;
     int sw_grid = 0, sw_K = 0, sw_items = 0, sw_R = 4;
-    unsigned *sw_bar = nullptr;
+    DevBuf sw_bar;  // unsigned
     size_t sw_smem = 0;
-    int *sw_blk = nullptr, *sw_m[2] = {nullptr, nullptr}, *sw_dtc[2] = {nullptr, nullptr};
-    double *sw_partial = nullptr, *sw_coef[2] = {nullptr, nullptr}, *sw_Emin[2] = {nullptr, nullptr},
-           *sw_Delta[2] = {nullptr, nullptr};
-    double2 *sw_phase[2] = {nullptr, nullptr};
+    DevBuf sw_blk, sw_m[2], sw_dtc[2];                       // int
+    DevBuf sw_partial, sw_coef[2], sw_Emin[2], sw_Delta[2];  // double
+    DevBuf sw_phase[2];                                      // double2
     long long sweep_launches = 0;
     // persistent cluster sweep for moderate dense generators (dense_sweep.cuh)
     bool dsweep = false;
     int ds_units = 0, ds_R = 0, ds_gpad = 0;
     size_t ds_smem = 0;
-    int *ds_units_dev = nullptr;
-    long long *ds_prof = nullptr;
+    DevBuf ds_units_dev;  // int
+    DevBuf ds_prof;       // long long
+
+    ~DenseEngine() {
+        if (graph_exec) cudaGraphExecDestroy(graph_exec);
+    }
 };
 
 namespace {
 
+// b holds n elements of T (at least one) afterwards
 template <typename T>
-bool dalloc(T *&p, size_t n, std::string &err) {
-    cudaError_t e = cudaMalloc((void **)&p, std::max<size_t>(n, 1) * sizeof(T));
+bool dalloc(DevBuf &b, size_t n, std::string &err) {
+    const cudaError_t e = b.allocate(std::max<size_t>(n, 1) * sizeof(T));
     if (e != cudaSuccess) {
         err = std::string("cudaMalloc of ") + std::to_string(n * sizeof(T)) + " bytes: " + cudaGetErrorString(e);
         return false;
@@ -1056,8 +1061,8 @@ bool launch_gemm(DenseEngine *e, const Block &b, GemmParams p, std::string &err)
     p.col0 = b.col0;
     p.streamk = e->streamk ? 1 : 0;
     p.x_contig = e->x_contig ? 1 : 0;
-    p.ws = e->sk_ws;
-    p.flags = e->sk_flags;
+    p.ws = e->sk_ws.get<double2>();
+    p.flags = e->sk_flags.get<unsigned>();
     dim3 grid(e->streamk ? e->sm_count : e->dp / BM), block(GEMM_THREADS);
     const size_t smem = gemm_smem_bytes();
     static bool attr_set = false;
@@ -1087,7 +1092,7 @@ bool launch_spmm(DenseEngine *e, const Block &b, const double2 *Gv, GemmParams p
     p.col0 = b.col0;
     if (p.partial) p.partial += n_partial_off;
     sp.e = p;
-    sp.cols = e->ell_cols;
+    sp.cols = e->ell_cols.get<int>();
     sp.Gv = Gv;
     sp.W = e->W;
     sp.ncols = b.nt * 8;
@@ -1147,12 +1152,12 @@ bool sweep_configure(DenseEngine *e) {
     cudaGetLastError();
     if (!e->sweep) return true;
     std::string err;
-    if (!dalloc(e->sw_blk, blk.size(), err) || !dalloc(e->sw_partial, (size_t)kMaxL * e->sw_grid, err) ||
-        !dalloc(e->sw_bar, 1, err)) {
+    if (!dalloc<int>(e->sw_blk, blk.size(), err) || !dalloc<double>(e->sw_partial, (size_t)kMaxL * e->sw_grid, err) ||
+        !dalloc<unsigned>(e->sw_bar, 1, err)) {
         e->sweep = false;
         return false;
     }
-    cudaMemcpy(e->sw_blk, blk.data(), blk.size() * 4, cudaMemcpyHostToDevice);
+    cudaMemcpy(e->sw_blk.get<int>(), blk.data(), blk.size() * 4, cudaMemcpyHostToDevice);
     return true;
 }
 
@@ -1203,10 +1208,10 @@ bool dsweep_configure(DenseEngine *e) {
         }
     }
     std::string err;
-    if (!dalloc(e->ds_units_dev, units.size(), err) || !dalloc(e->sw_partial, (size_t)kMaxL * n_units * kDsCluster, err) ||
-        !dalloc(e->sw_bar, 1, err))
+    if (!dalloc<int>(e->ds_units_dev, units.size(), err) ||
+        !dalloc<double>(e->sw_partial, (size_t)kMaxL * n_units * kDsCluster, err) || !dalloc<unsigned>(e->sw_bar, 1, err))
         return false;
-    cudaMemcpy(e->ds_units_dev, units.data(), units.size() * 4, cudaMemcpyHostToDevice);
+    cudaMemcpy(e->ds_units_dev.get<int>(), units.data(), units.size() * 4, cudaMemcpyHostToDevice);
     e->ds_units = n_units;
     e->dsweep = true;
     return true;
@@ -1217,23 +1222,25 @@ bool launch_dsweep(DenseEngine *e, int mode, const double *d_eps_old, double *d_
     DSweepParams p;
     memset(&p, 0, sizeof(p));
     p.d = e->d; p.dp = e->dp; p.ld = e->ld; p.L = e->L; p.N_T = e->N_T; p.mode = mode; p.store_fw = e->store_fw;
-    p.n_units = e->ds_units; p.R = e->ds_R; p.gpad = e->ds_gpad; p.units = e->ds_units_dev;
-    p.H[0] = e->Hf;
-    p.H[1] = e->hermitian ? e->Hf : e->Hb;
+    p.n_units = e->ds_units; p.R = e->ds_R; p.gpad = e->ds_gpad; p.units = e->ds_units_dev.get<int>();
+    p.H[0] = e->Hf.get<double2>();
+    p.H[1] = e->hermitian ? e->Hf.get<double2>() : e->Hb.get<double2>();
     for (int dir = 0; dir < 2; ++dir) {
-        p.coef[dir] = e->sw_coef[dir]; p.m[dir] = e->sw_m[dir]; p.phase[dir] = e->sw_phase[dir]; p.dtc[dir] = e->sw_dtc[dir];
-        p.E_min[dir] = e->sw_Emin[dir]; p.Delta[dir] = e->sw_Delta[dir];
+        p.coef[dir] = e->sw_coef[dir].get<double>(); p.m[dir] = e->sw_m[dir].get<int>();
+        p.phase[dir] = e->sw_phase[dir].get<double2>(); p.dtc[dir] = e->sw_dtc[dir].get<int>();
+        p.E_min[dir] = e->sw_Emin[dir].get<double>(); p.Delta[dir] = e->sw_Delta[dir].get<double>();
         p.ndtc[dir] = e->ch[dir].ndtc; p.mmax[dir] = e->ch[dir].mmax;
     }
-    p.PSI = e->PSI; p.X = e->X; p.PHI = e->PHI; p.VX[0] = e->V[0]; p.VX[1] = e->V[1];
-    p.PSI0 = e->PSI0; p.CHI = e->CHI; p.slab = e->slab;
+    p.PSI = e->PSI.get<double2>(); p.X = e->X.get<double2>(); p.PHI = e->PHI.get<double2>();
+    p.VX[0] = e->V[0].get<double2>(); p.VX[1] = e->V[1].get<double2>();
+    p.PSI0 = e->PSI0.get<double2>(); p.CHI = e->CHI.get<double2>(); p.slab = e->slab;
     p.eps_old = d_eps_old; p.eps_new = d_eps_new; p.alpha = d_alpha; p.dt = d_dt; p.ga = d_ga;
     p.amp_old = gen_coeffs_old(e, d_eps_old); p.am = e->amp; p.cm = e->comm;
-    p.partial = e->sw_partial;
-    p.bar = e->sw_bar;
-    if (getenv("KROTOV_PROF") && !e->ds_prof) dalloc(e->ds_prof, 8, err);
-    p.prof = getenv("KROTOV_PROF") ? e->ds_prof : nullptr;
-    DK_CHECK(cudaMemsetAsync(e->sw_bar, 0, sizeof(unsigned), e->stream));
+    p.partial = e->sw_partial.get<double>();
+    p.bar = e->sw_bar.get<unsigned>();
+    if (getenv("KROTOV_PROF") && !e->ds_prof) dalloc<long long>(e->ds_prof, 8, err);
+    p.prof = getenv("KROTOV_PROF") ? e->ds_prof.get<long long>() : nullptr;
+    DK_CHECK(cudaMemsetAsync(e->sw_bar.get<unsigned>(), 0, sizeof(unsigned), e->stream));
     DK_CHECK(cudaFuncSetAttribute((const void *)dense_cluster_sweep_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                   (int)e->ds_smem));
     cudaLaunchConfig_t cfg;
@@ -1257,7 +1264,7 @@ bool launch_dsweep(DenseEngine *e, int mode, const double *d_eps_old, double *d_
     if (p.prof) {  // diagnostics: where CTA 0 spent its cycles (us per time step of the sweep)
         long long h[6];
         DK_CHECK(cudaStreamSynchronize(e->stream));
-        DK_CHECK(cudaMemcpy(h, e->ds_prof, sizeof(h), cudaMemcpyDeviceToHost));
+        DK_CHECK(cudaMemcpy(h, e->ds_prof.get<long long>(), sizeof(h), cudaMemcpyDeviceToHost));
         const double f = 1.0 / 1965.0 / e->N_T;
         fprintf(stderr, "[dense sweep, mode %d, d=%d, %d clusters] us per time step (both sweeps of an iteration summed): "
                         "build G %.2f, tiles %.2f, exchange + cluster barrier %.2f, group reload %.2f, overlaps %.2f, "
@@ -1279,11 +1286,9 @@ bool sweep_usable(const DenseEngine *e, int mode) {
 }
 
 template <typename T>
-bool sweep_upload(T *&dst, const std::vector<T> &src, std::string &err) {
-    if (dst) cudaFree(dst);
-    dst = nullptr;
-    if (!dalloc(dst, src.size(), err)) return false;
-    DK_CHECK(cudaMemcpy(dst, src.data(), src.size() * sizeof(T), cudaMemcpyHostToDevice));
+bool sweep_upload(DevBuf &dst, const std::vector<T> &src, std::string &err) {
+    if (!dalloc<T>(dst, src.size(), err)) return false;  // (frees the previous table first)
+    DK_CHECK(cudaMemcpy(dst.get<void>(), src.data(), src.size() * sizeof(T), cudaMemcpyHostToDevice));
     return true;
 }
 
@@ -1294,23 +1299,25 @@ bool launch_sweep(DenseEngine *e, int mode, const double *d_eps_old, double *d_e
     memset(&p, 0, sizeof(p));
     p.dp = e->dp; p.ld = e->ld; p.W = e->W; p.L = e->L; p.N_T = e->N_T; p.n_blocks = (int)e->blocks.size();
     p.n_items = e->sw_items; p.mode = mode; p.store_fw = e->store_fw; p.K = e->sw_K;
-    p.cols = e->ell_cols;
-    p.Pv[0] = e->Pvf;
-    p.Pv[1] = e->hermitian ? e->Pvf : e->Pvb;
-    p.blk = e->sw_blk;
+    p.cols = e->ell_cols.get<int>();
+    p.Pv[0] = e->Pvf.get<double2>();
+    p.Pv[1] = e->hermitian ? e->Pvf.get<double2>() : e->Pvb.get<double2>();
+    p.blk = e->sw_blk.get<int>();
     for (int dir = 0; dir < 2; ++dir) {
-        p.coef[dir] = e->sw_coef[dir]; p.m[dir] = e->sw_m[dir]; p.phase[dir] = e->sw_phase[dir]; p.dtc[dir] = e->sw_dtc[dir];
-        p.E_min[dir] = e->sw_Emin[dir]; p.Delta[dir] = e->sw_Delta[dir];
+        p.coef[dir] = e->sw_coef[dir].get<double>(); p.m[dir] = e->sw_m[dir].get<int>();
+        p.phase[dir] = e->sw_phase[dir].get<double2>(); p.dtc[dir] = e->sw_dtc[dir].get<int>();
+        p.E_min[dir] = e->sw_Emin[dir].get<double>(); p.Delta[dir] = e->sw_Delta[dir].get<double>();
         p.ndtc[dir] = e->ch[dir].ndtc; p.mmax[dir] = e->ch[dir].mmax;
     }
-    p.PSI = e->PSI; p.V[0] = e->V[0]; p.V[1] = e->V[1]; p.V[2] = e->V[2]; p.OUT = e->OUT; p.X = e->X; p.PHI = e->PHI;
-    p.PSI0 = e->PSI0; p.CHI = e->CHI; p.slab = e->slab;
+    p.PSI = e->PSI.get<double2>(); p.V[0] = e->V[0].get<double2>(); p.V[1] = e->V[1].get<double2>();
+    p.V[2] = e->V[2].get<double2>(); p.OUT = e->OUT.get<double2>(); p.X = e->X.get<double2>(); p.PHI = e->PHI.get<double2>();
+    p.PSI0 = e->PSI0.get<double2>(); p.CHI = e->CHI.get<double2>(); p.slab = e->slab;
     p.eps_old = d_eps_old; p.eps_new = d_eps_new; p.alpha = d_alpha; p.dt = d_dt; p.ga = d_ga;
     p.amp_old = gen_coeffs_old(e, d_eps_old); p.am = e->amp; p.cm = e->comm;
-    p.partial = e->sw_partial;
+    p.partial = e->sw_partial.get<double>();
     p.cg_sync = getenv("KROTOV_SWEEP_CGSYNC") ? 1 : 0;
-    p.bar = e->sw_bar;
-    DK_CHECK(cudaMemsetAsync(e->sw_bar, 0, sizeof(unsigned), e->stream));
+    p.bar = e->sw_bar.get<unsigned>();
+    DK_CHECK(cudaMemsetAsync(e->sw_bar.get<unsigned>(), 0, sizeof(unsigned), e->stream));
     const void *fn = sweep_kernel_for(e->sw_R);
     DK_CHECK(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)e->sw_smem));
     void *args[] = {(void *)&p};
@@ -1325,21 +1332,22 @@ bool step(DenseEngine *e, int dir, int n, const double *d_eps, double2 *store, s
     const Cheb &c = e->ch[dir];
     const int dtc = c.dtc_of_step[n];
     const size_t mat = (size_t)e->dp * e->dp;
-    const double2 *H = (dir == KROTOV_FORWARD || e->hermitian) ? e->Hf : e->Hb;
+    const double2 *H = (dir == KROTOV_FORWARD || e->hermitian) ? e->Hf.get<double2>() : e->Hb.get<double2>();
     const size_t nslots = (size_t)e->dp * e->W;
     for (int g = 0; g < e->n_gen; ++g) {
         const double s = 4.0 / c.Delta[g], beta = c.Delta[g] / 2 + c.E_min[g];
         const double2 f = (dir == KROTOV_FORWARD) ? make_double2(0.0, -s) : make_double2(0.0, s);
         if (e->sparse) {
-            const double2 *Pv = (dir == KROTOV_FORWARD || e->hermitian) ? e->Pvf : e->Pvb;
+            const double2 *Pv = (dir == KROTOV_FORWARD || e->hermitian) ? e->Pvf.get<double2>() : e->Pvb.get<double2>();
             build_G_sparse_kernel<<<std::max(1, (int)std::min<size_t>(e->sm_count * 4, (nslots + 255) / 256)), 256, 0,
-                                    e->stream>>>(e->Gv + (size_t)g * nslots, Pv + (size_t)g * (1 + e->L) * nslots, nslots,
-                                                 e->W, e->L, f, beta, d_eps, e->N_T, n);
+                                    e->stream>>>(e->Gv.get<double2>() + (size_t)g * nslots, Pv + (size_t)g * (1 + e->L) * nslots,
+                                                 nslots, e->W, e->L, f, beta, d_eps, e->N_T, n);
             e->launches++;
             continue;
         }
-        build_G_kernel<<<e->sm_count * 4, 256, 0, e->stream>>>(e->G + (size_t)g * e->gmat, H + (size_t)g * (1 + e->L) * mat,
-                                                             e->dp, e->L, f, beta, d_eps, e->N_T, n);
+        build_G_kernel<<<e->sm_count * 4, 256, 0, e->stream>>>(e->G.get<double2>() + (size_t)g * e->gmat,
+                                                             H + (size_t)g * (1 + e->L) * mat, e->dp, e->L, f, beta, d_eps,
+                                                             e->N_T, n);
         e->launches++;
     }
     for (const Block &b : e->blocks) {
@@ -1352,33 +1360,33 @@ bool step(DenseEngine *e, int dir, int n, const double *d_eps, double2 *store, s
             return false;
         }
         // V[0] aliases PSI for j = 1;  ring of three work blocks afterwards
-        const double2 *vprev = e->PSI;  // V_{j-1}
+        const double2 *vprev = e->PSI.get<double2>();  // V_{j-1}
         const double2 *vprev2 = nullptr;
         for (int j = 1; j < m; ++j) {
             GemmParams p;
             memset(&p, 0, sizeof(p));
-            p.A = e->G + (size_t)b.g * e->gmat;
+            p.A = e->G.get<double2>() + (size_t)b.g * e->gmat;
             p.a_tiled = 1;
             p.B = vprev;
             p.epi = 0;
             p.Vold = vprev2;
-            p.Vnew = e->V[j % 3];
-            p.OUT = e->OUT;
+            p.Vnew = e->V[j % 3].get<double2>();
+            p.OUT = e->OUT.get<double2>();
             p.j = j;
             p.last = (j == m - 1);
             p.a0 = a[0];
             p.aj = a[j];
             p.phase = make_double2(ph.real(), ph.imag());
             // the last term must not overwrite PSI while other CTAs still read it as V_0 (only when m == 2)
-            p.PSI = (m == 2) ? e->V[2] : e->PSI;
+            p.PSI = (m == 2) ? e->V[2].get<double2>() : e->PSI.get<double2>();
             p.store = store;
             if (e->sparse) {
-                if (!launch_spmm(e, b, e->Gv + (size_t)b.g * nslots, p, 0, err)) return false;
+                if (!launch_spmm(e, b, e->Gv.get<double2>() + (size_t)b.g * nslots, p, 0, err)) return false;
             } else if (!launch_gemm(e, b, p, err)) {
                 return false;
             }
             vprev2 = vprev;
-            vprev = e->V[j % 3];
+            vprev = e->V[j % 3].get<double2>();
         }
         if (m == 2) {
             err = "m == 2 on the dense path is not supported";
@@ -1397,7 +1405,7 @@ DenseEngine *dense_create(int d, int N, int L, int N_T, int n_gen, const std::ve
         err = "too many controls";
         return nullptr;
     }
-    DenseEngine *e = new DenseEngine();
+    std::unique_ptr<DenseEngine> e(new DenseEngine());
     e->d = d; e->N = N; e->L = L; e->N_T = N_T; e->n_gen = n_gen; e->store_fw = store_fw; e->stream = stream;
     e->dp = (d + BM - 1) / BM * BM;
     int dev = 0;
@@ -1462,46 +1470,45 @@ DenseEngine *dense_create(int d, int N, int L, int N_T, int n_gen, const std::ve
     if (need * 16 > free_b) {
         err = "dense path needs " + std::to_string(need * 16 >> 20) + " MiB of device memory, " +
               std::to_string(free_b >> 20) + " MiB free";
-        delete e;
         return nullptr;
     }
-    bool ok = dalloc(e->Hf, (size_t)n_gen * (1 + L) * mat, err) && dalloc(e->G, (size_t)n_gen * e->gmat, err) &&
-              dalloc(e->V[0], e->slab, err) && dalloc(e->V[1], e->slab, err) && dalloc(e->V[2], e->slab, err) &&
-              dalloc(e->OUT, e->slab, err) && dalloc(e->PSI, e->slab, err) && dalloc(e->PSI0, e->slab, err) &&
-              dalloc(e->TGT, e->slab, err) && dalloc(e->CHI, e->slab, err) &&
-              dalloc(e->X, e->slab * (size_t)(N_T + 1), err) && dalloc(e->partial, (size_t)L * e->n_partial, err) &&
-              dalloc(e->d_col_of_traj, (size_t)N, err) && dalloc(e->d_traj_of_col, (size_t)e->ld, err);
-    if (ok && !e->hermitian && !e->sparse) ok = dalloc(e->Hb, (size_t)n_gen * (1 + L) * mat, err);
-    if (ok && store_fw) ok = dalloc(e->PHI, e->slab * (size_t)(N_T + 1), err);
+    bool ok = dalloc<double2>(e->Hf, (size_t)n_gen * (1 + L) * mat, err) &&
+              dalloc<double2>(e->G, (size_t)n_gen * e->gmat, err) && dalloc<double2>(e->V[0], e->slab, err) &&
+              dalloc<double2>(e->V[1], e->slab, err) && dalloc<double2>(e->V[2], e->slab, err) &&
+              dalloc<double2>(e->OUT, e->slab, err) && dalloc<double2>(e->PSI, e->slab, err) &&
+              dalloc<double2>(e->PSI0, e->slab, err) && dalloc<double2>(e->TGT, e->slab, err) &&
+              dalloc<double2>(e->CHI, e->slab, err) && dalloc<double2>(e->X, e->slab * (size_t)(N_T + 1), err) &&
+              dalloc<double>(e->partial, (size_t)L * e->n_partial, err) && dalloc<int>(e->d_col_of_traj, (size_t)N, err) &&
+              dalloc<int>(e->d_traj_of_col, (size_t)e->ld, err);
+    if (ok && !e->hermitian && !e->sparse) ok = dalloc<double2>(e->Hb, (size_t)n_gen * (1 + L) * mat, err);
+    if (ok && store_fw) ok = dalloc<double2>(e->PHI, e->slab * (size_t)(N_T + 1), err);
     // Stream-K for the DMMA GEMM when the row blocks would leave SMs idle (C5: 128 row blocks on 148 SMs) and K is
     // long enough to split: as many CTAs as SMs, each total/G chunks of the (row block, k) space.
     {
         const int R = e->dp / BM, nk = e->dp / BK, G = e->sm_count;
         e->streamk = !e->sparse && R >= 32 && R < G && nk >= 32 && (G + R - 1) / R + 1 <= kSkParts && !getenv("KROTOV_NO_STREAMK");
         if (ok && e->streamk) {
-            ok = dalloc(e->sk_ws, (size_t)R * kSkParts * BM * 64, err) && dalloc(e->sk_flags, (size_t)R * kSkParts * 4, err);
-            if (ok) cudaMemset(e->sk_flags, 0, (size_t)R * kSkParts * 4 * sizeof(unsigned));
+            ok = dalloc<double2>(e->sk_ws, (size_t)R * kSkParts * BM * 64, err) &&
+                 dalloc<unsigned>(e->sk_flags, (size_t)R * kSkParts * 4, err);
+            if (ok) cudaMemset(e->sk_flags.get<unsigned>(), 0, (size_t)R * kSkParts * 4 * sizeof(unsigned));
         }
     }
     if (ok && e->sparse)
-        ok = dalloc(e->ell_cols, nslots, err) && dalloc(e->Pvf, (size_t)n_gen * (1 + L) * nslots, err) &&
-             dalloc(e->Gv, (size_t)n_gen * nslots, err) &&
-             (e->hermitian || dalloc(e->Pvb, (size_t)n_gen * (1 + L) * nslots, err));
-    if (!ok) {
-        dense_destroy(e);
-        return nullptr;
-    }
+        ok = dalloc<int>(e->ell_cols, nslots, err) && dalloc<double2>(e->Pvf, (size_t)n_gen * (1 + L) * nslots, err) &&
+             dalloc<double2>(e->Gv, (size_t)n_gen * nslots, err) &&
+             (e->hermitian || dalloc<double2>(e->Pvb, (size_t)n_gen * (1 + L) * nslots, err));
+    if (!ok) return nullptr;
     if (e->sparse) {
         // ELL arrays padded to dp rows: padding rows / slots point at their own row with value 0
         std::vector<int> cols(nslots);
         for (size_t i = 0; i < (size_t)e->dp; ++i)
             for (int sl = 0; sl < e->W; ++sl)
                 cols[i * e->W + sl] = (i < (size_t)d) ? (*sp->cols)[i * e->W + sl] : (int)i;
-        cudaMemcpy(e->ell_cols, cols.data(), nslots * 4, cudaMemcpyHostToDevice);
+        cudaMemcpy(e->ell_cols.get<int>(), cols.data(), nslots * 4, cudaMemcpyHostToDevice);
         std::vector<cplx> vbuf(nslots);
         for (int dir = 0; dir < (e->hermitian ? 1 : 2); ++dir) {
             const std::vector<cplx> &src = dir == 0 ? *sp->vals_f : *sp->vals_b;
-            double2 *dst = dir == 0 ? e->Pvf : e->Pvb;
+            double2 *dst = dir == 0 ? e->Pvf.get<double2>() : e->Pvb.get<double2>();
             for (int q = 0; q < n_gen * (1 + L); ++q) {
                 std::fill(vbuf.begin(), vbuf.end(), cplx(0, 0));
                 memcpy(vbuf.data(), &src[(size_t)q * d * e->W], sizeof(cplx) * (size_t)d * e->W);
@@ -1509,9 +1516,8 @@ DenseEngine *dense_create(int d, int N, int L, int N_T, int n_gen, const std::ve
             }
         }
     }
-    if ((e->sparse && !sweep_configure(e)) || (!e->sparse && !dsweep_configure(e))) {
+    if ((e->sparse && !sweep_configure(e.get())) || (!e->sparse && !dsweep_configure(e.get()))) {
         err = "dense_create: allocation for the persistent sweep failed";
-        dense_destroy(e);
         return nullptr;
     }
     // upload padded generator terms (and adjoints), states, targets
@@ -1520,12 +1526,12 @@ DenseEngine *dense_create(int d, int N, int L, int N_T, int n_gen, const std::ve
         const cplx *M = &Hdense[(size_t)q * d * d];
         std::fill(buf.begin(), buf.end(), cplx(0, 0));
         for (int i = 0; i < d; ++i) memcpy(&buf[(size_t)i * e->dp], &M[(size_t)i * d], sizeof(cplx) * d);
-        cudaMemcpy(e->Hf + (size_t)q * mat, buf.data(), mat * 16, cudaMemcpyHostToDevice);
+        cudaMemcpy(e->Hf.get<double2>() + (size_t)q * mat, buf.data(), mat * 16, cudaMemcpyHostToDevice);
         if (!e->hermitian) {
             std::fill(buf.begin(), buf.end(), cplx(0, 0));
             for (int i = 0; i < d; ++i)
                 for (int j = 0; j < d; ++j) buf[(size_t)i * e->dp + j] = std::conj(M[(size_t)j * d + i]);
-            cudaMemcpy(e->Hb + (size_t)q * mat, buf.data(), mat * 16, cudaMemcpyHostToDevice);
+            cudaMemcpy(e->Hb.get<double2>() + (size_t)q * mat, buf.data(), mat * 16, cudaMemcpyHostToDevice);
         }
     }
     auto to_block = [&](const double *src, double2 *dst) {
@@ -1537,34 +1543,22 @@ DenseEngine *dense_create(int d, int N, int L, int N_T, int n_gen, const std::ve
         }
         cudaMemcpy(dst, blk.data(), e->slab * 16, cudaMemcpyHostToDevice);
     };
-    to_block(psi0, e->PSI0);
-    to_block(target, e->TGT);
-    cudaMemset(e->CHI, 0, e->slab * 16);
-    cudaMemset(e->PSI, 0, e->slab * 16);
-    cudaMemcpy(e->d_col_of_traj, e->col_of_traj.data(), (size_t)N * 4, cudaMemcpyHostToDevice);
-    cudaMemcpy(e->d_traj_of_col, e->traj_of_col.data(), (size_t)e->ld * 4, cudaMemcpyHostToDevice);
+    to_block(psi0, e->PSI0.get<double2>());
+    to_block(target, e->TGT.get<double2>());
+    cudaMemset(e->CHI.get<double2>(), 0, e->slab * 16);
+    cudaMemset(e->PSI.get<double2>(), 0, e->slab * 16);
+    cudaMemcpy(e->d_col_of_traj.get<int>(), e->col_of_traj.data(), (size_t)N * 4, cudaMemcpyHostToDevice);
+    cudaMemcpy(e->d_traj_of_col.get<int>(), e->traj_of_col.data(), (size_t)e->ld * 4, cudaMemcpyHostToDevice);
     if (cudaGetLastError() != cudaSuccess) {
         err = "dense_create: upload failed";
-        dense_destroy(e);
         return nullptr;
     }
-    return e;
+    return e.release();
 }
 
 void dense_set_comm(DenseEngine *e, const DenseComm &c) { e->comm = c; }
 
-void dense_destroy(DenseEngine *e) {
-    if (!e) return;
-    void *ptrs[] = {e->Hf, e->Hb, e->G, e->V[0], e->V[1], e->V[2], e->OUT, e->PSI, e->PSI0, e->TGT, e->CHI, e->X,
-                    e->PHI, e->partial, e->d_col_of_traj, e->d_traj_of_col, e->ell_cols, e->Pvf, e->Pvb, e->Gv,
-                    e->sk_ws, e->sk_flags, e->sw_blk, e->sw_partial, e->sw_bar, e->sw_m[0], e->sw_m[1], e->sw_dtc[0], e->sw_dtc[1],
-                    e->sw_coef[0], e->sw_coef[1], e->sw_Emin[0], e->sw_Emin[1], e->sw_Delta[0], e->sw_Delta[1],
-                    e->sw_phase[0], e->sw_phase[1], e->ds_units_dev, e->ds_prof};
-    for (void *p : ptrs)
-        if (p) cudaFree(p);
-    if (e->graph_exec) cudaGraphExecDestroy(e->graph_exec);
-    delete e;
-}
+void dense_destroy(DenseEngine *e) { delete e; }
 
 void dense_set_amp(DenseEngine *e, const AmpDev &a) { e->amp = a; }
 
@@ -1613,7 +1607,8 @@ bool dense_set_cheby(DenseEngine *e, int direction, int ndtc, const std::vector<
 }
 
 static bool finish_sweep(DenseEngine *e, double2 *d_tau, std::string &err) {
-    tau_kernel<<<(e->N + 3) / 4, 128, 0, e->stream>>>(e->PSI, e->TGT, e->d, e->ld, e->d_col_of_traj, e->N, d_tau);
+    tau_kernel<<<(e->N + 3) / 4, 128, 0, e->stream>>>(e->PSI.get<double2>(), e->TGT.get<double2>(), e->d, e->ld,
+                                                      e->d_col_of_traj.get<int>(), e->N, d_tau);
     e->launches++;
     DK_CHECK(cudaGetLastError());
     return true;
@@ -1622,21 +1617,23 @@ static bool finish_sweep(DenseEngine *e, double2 *d_tau, std::string &err) {
 // Psi_k(T) := initial states, tau from them: the state of freshly initialised propagators, which is what the driver
 // reads when `skip_initial_forward_propagation` is set (src/optimize.jl:171-181, :297, :378-381)
 bool dense_seed(DenseEngine *e, double2 *d_tau, std::string &err) {
-    DK_CHECK(cudaMemcpyAsync(e->PSI, e->PSI0, e->slab * 16, cudaMemcpyDeviceToDevice, e->stream));
+    DK_CHECK(cudaMemcpyAsync(e->PSI.get<double2>(), e->PSI0.get<double2>(), e->slab * 16, cudaMemcpyDeviceToDevice, e->stream));
     return finish_sweep(e, d_tau, err);
 }
 
 bool dense_forward(DenseEngine *e, const double *d_eps, double2 *d_tau, long long &launches, std::string &err) {
     e->launches = 0;
-    DK_CHECK(cudaMemcpyAsync(e->PSI, e->PSI0, e->slab * 16, cudaMemcpyDeviceToDevice, e->stream));
+    DK_CHECK(cudaMemcpyAsync(e->PSI.get<double2>(), e->PSI0.get<double2>(), e->slab * 16, cudaMemcpyDeviceToDevice, e->stream));
     if (sweep_usable(e, 0)) {
         if (!launch_sweep(e, 0, d_eps, nullptr, nullptr, nullptr, nullptr, err) || !finish_sweep(e, d_tau, err)) return false;
         launches += e->launches;
         return true;
     }
-    if (e->store_fw) DK_CHECK(cudaMemcpyAsync(e->PHI, e->PSI0, e->slab * 16, cudaMemcpyDeviceToDevice, e->stream));
+    if (e->store_fw)
+        DK_CHECK(cudaMemcpyAsync(e->PHI.get<double2>(), e->PSI0.get<double2>(), e->slab * 16, cudaMemcpyDeviceToDevice, e->stream));
     for (int n = 0; n < e->N_T; ++n)
-        if (!step(e, KROTOV_FORWARD, n, gen_coeffs_old(e, d_eps), e->store_fw ? e->PHI + e->slab * (size_t)(n + 1) : nullptr, err))
+        if (!step(e, KROTOV_FORWARD, n, gen_coeffs_old(e, d_eps),
+                  e->store_fw ? e->PHI.get<double2>() + e->slab * (size_t)(n + 1) : nullptr, err))
             return false;
     if (!finish_sweep(e, d_tau, err)) return false;
     launches += e->launches;
@@ -1720,19 +1717,21 @@ bool iterate_body(DenseEngine *e, const double *d_eps_old, double *d_eps_new, co
     const int N_T = e->N_T;
     // ---- chi(T)
     if (d_chi_coef != nullptr) {
-        chi_from_coef_kernel<<<e->sm_count * 2, 256, 0, e->stream>>>(e->CHI, e->TGT, d_chi_coef, e->d_traj_of_col,
+        chi_from_coef_kernel<<<e->sm_count * 2, 256, 0, e->stream>>>(e->CHI.get<double2>(), e->TGT.get<double2>(), d_chi_coef,
+                                                                     e->d_traj_of_col.get<int>(),
                                                                      e->dp, e->ld);
         e->launches++;
     }
     if (sweep_usable(e, 1))
         return launch_sweep(e, 1, d_eps_old, d_eps_new, d_alpha, d_dt, d_ga, err) && finish_sweep(e, d_tau, err);
     // ---- backward sweep: chi(t_n) for all n into X
-    DK_CHECK(cudaMemcpyAsync(e->PSI, e->CHI, e->slab * 16, cudaMemcpyDeviceToDevice, e->stream));
-    DK_CHECK(cudaMemcpyAsync(e->X + e->slab * (size_t)N_T, e->CHI, e->slab * 16, cudaMemcpyDeviceToDevice, e->stream));
+    DK_CHECK(cudaMemcpyAsync(e->PSI.get<double2>(), e->CHI.get<double2>(), e->slab * 16, cudaMemcpyDeviceToDevice, e->stream));
+    DK_CHECK(cudaMemcpyAsync(e->X.get<double2>() + e->slab * (size_t)N_T, e->CHI.get<double2>(), e->slab * 16,
+                             cudaMemcpyDeviceToDevice, e->stream));
     for (int n = N_T - 1; n >= 0; --n)
-        if (!step(e, KROTOV_BACKWARD, n, gen_coeffs_old(e, d_eps_old), e->X + e->slab * (size_t)n, err)) return false;
+        if (!step(e, KROTOV_BACKWARD, n, gen_coeffs_old(e, d_eps_old), e->X.get<double2>() + e->slab * (size_t)n, err)) return false;
     // ---- forward sweep with sequential update
-    DK_CHECK(cudaMemcpyAsync(e->PSI, e->PSI0, e->slab * 16, cudaMemcpyDeviceToDevice, e->stream));
+    DK_CHECK(cudaMemcpyAsync(e->PSI.get<double2>(), e->PSI0.get<double2>(), e->slab * 16, cudaMemcpyDeviceToDevice, e->stream));
     const size_t mat = (size_t)e->dp * e->dp;
     const int ctas = e->dp / BM;
     for (int n = 0; n < N_T; ++n) {
@@ -1741,24 +1740,25 @@ bool iterate_body(DenseEngine *e, const double *d_eps_old, double *d_eps_new, co
                 const Block &b = e->blocks[bi];
                 GemmParams p;
                 memset(&p, 0, sizeof(p));
-                p.A = e->Hf + ((size_t)b.g * (1 + e->L) + 1 + l) * mat;  // mu_l = H_l (src/optimize.jl:275-276)
-                p.B = e->PSI;
+                p.A = e->Hf.get<double2>() + ((size_t)b.g * (1 + e->L) + 1 + l) * mat;  // mu_l = H_l (src/optimize.jl:275-276)
+                p.B = e->PSI.get<double2>();
                 p.epi = 1;
-                p.CHI = e->X + e->slab * (size_t)n;
+                p.CHI = e->X.get<double2>() + e->slab * (size_t)n;
                 if (e->sparse) {
-                    p.partial = e->partial + (size_t)l * e->n_partial;
-                    const double2 *mu = e->Pvf + ((size_t)b.g * (1 + e->L) + 1 + l) * ((size_t)e->dp * e->W);
+                    p.partial = e->partial.get<double>() + (size_t)l * e->n_partial;
+                    const double2 *mu = e->Pvf.get<double2>() + ((size_t)b.g * (1 + e->L) + 1 + l) * ((size_t)e->dp * e->W);
                     if (!launch_spmm(e, b, mu, p, e->sp_part_off[bi], err)) return false;
                     continue;
                 }
-                p.partial = e->partial + (size_t)l * e->n_partial + bi * ctas;
+                p.partial = e->partial.get<double>() + (size_t)l * e->n_partial + bi * ctas;
                 if (!launch_gemm(e, b, p, err)) return false;
             }
         }
-        update_kernel<<<e->L, 32, 0, e->stream>>>(e->partial, e->n_partial, e->L, d_alpha, d_eps_old, d_eps_new, d_ga,
+        update_kernel<<<e->L, 32, 0, e->stream>>>(e->partial.get<double>(), e->n_partial, e->L, d_alpha, d_eps_old, d_eps_new, d_ga,
                                                  d_dt, N_T, n, e->comm, e->amp);
         e->launches++;
-        if (!step(e, KROTOV_FORWARD, n, gen_coeffs_new(e, d_eps_new), e->store_fw ? e->PHI + e->slab * (size_t)n : nullptr, err))
+        if (!step(e, KROTOV_FORWARD, n, gen_coeffs_new(e, d_eps_new),
+                  e->store_fw ? e->PHI.get<double2>() + e->slab * (size_t)n : nullptr, err))
             return false;
     }
     return finish_sweep(e, d_tau, err);
@@ -1770,14 +1770,14 @@ bool dense_set_chi(DenseEngine *e, const double *chi_host, std::string &err) {
     const cplx *s = reinterpret_cast<const cplx *>(chi_host);
     for (int k = 0; k < e->N; ++k)
         for (int i = 0; i < e->d; ++i) blk[(size_t)i * e->ld + e->col_of_traj[k]] = s[(size_t)k * e->d + i];
-    DK_CHECK(cudaMemcpy(e->CHI, blk.data(), e->slab * 16, cudaMemcpyHostToDevice));
+    DK_CHECK(cudaMemcpy(e->CHI.get<double2>(), blk.data(), e->slab * 16, cudaMemcpyHostToDevice));
     e->chi_from_host = true;
     return true;
 }
 
 bool dense_get_states(DenseEngine *e, double *states_host, std::string &err) {
     std::vector<cplx> blk(e->slab);
-    DK_CHECK(cudaMemcpy(blk.data(), e->PSI, e->slab * 16, cudaMemcpyDeviceToHost));
+    DK_CHECK(cudaMemcpy(blk.data(), e->PSI.get<double2>(), e->slab * 16, cudaMemcpyDeviceToHost));
     cplx *o = reinterpret_cast<cplx *>(states_host);
     for (int k = 0; k < e->N; ++k)
         for (int i = 0; i < e->d; ++i) o[(size_t)k * e->d + i] = blk[(size_t)i * e->ld + e->col_of_traj[k]];
@@ -1785,7 +1785,7 @@ bool dense_get_states(DenseEngine *e, double *states_host, std::string &err) {
 }
 
 bool dense_get_storage(DenseEngine *e, int which, int k, int n0, int n1, double *out_host, std::string &err) {
-    const double2 *S = which == KROTOV_FORWARD ? e->PHI : e->X;
+    const double2 *S = which == KROTOV_FORWARD ? e->PHI.get<double2>() : e->X.get<double2>();
     const int c = e->col_of_traj[k];
     cplx *o = reinterpret_cast<cplx *>(out_host);
     std::vector<cplx> colbuf(e->d);

@@ -15,6 +15,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <map>
+#include <memory>
 #include <set>
 #include <string>
 #include <vector>
@@ -23,6 +24,7 @@
 
 #include "../../include/krotov_cuda.h"
 #include "dense_kernel.cuh"
+#include "device_buffer.cuh"
 #include "warp_kernel.cuh"
 #include "warp2_kernel.cuh"
 #include "tiny_kernel.cuh"
@@ -50,15 +52,7 @@ struct Trace {
     }
 };
 
-struct DevBuf {
-    void *p = nullptr;
-    size_t bytes = 0;
-    void release() {
-        if (p) cudaFree(p);
-        p = nullptr;
-        bytes = 0;
-    }
-};
+using kr::DevBuf;
 
 struct HostSparse {  // ELL description of a sparse generator family (d > 32), slot 0 = diagonal
     int W = 0, nnz_union = 0;
@@ -78,9 +72,20 @@ struct ChebyTables {  // one direction
     std::vector<cplx> phase_host;
 };
 
+// the handle's stream and timing events: a base of krotov_handle_s, so they are destroyed after every member
+struct HandleStream {
+    cudaStream_t stream = nullptr;
+    cudaEvent_t ev0 = nullptr, ev1 = nullptr;
+    ~HandleStream() {
+        if (ev0) cudaEventDestroy(ev0);
+        if (ev1) cudaEventDestroy(ev1);
+        if (stream) cudaStreamDestroy(stream);
+    }
+};
+
 }  // namespace
 
-struct krotov_handle_s {
+struct krotov_handle_s : HandleStream {
     int d = 0, N = 0, L = 0, N_T = 0, n_gen = 0, functional = 0, N_global = 0, store_fw = 0, device = 0;
     int path = 0;
     std::vector<double> tlist, dt;
@@ -124,7 +129,6 @@ struct krotov_handle_s {
     DevBuf d_rfcount;                             // arrival counter of the rank barrier
     double2 *peer_Xbase[kr::kMaxRanks] = {};      // chi trajectories of every rank (parity p at + p * x_slab)
     unsigned long long *peer_flag[kr::kMaxRanks] = {};
-    bool peer_x_opened[kr::kMaxRanks] = {};
     int xchg_last = 0;   // cross-rank protocol of the last launch: 0 none, 1 hier, 2 onehop, 3 mailboxes
     // non-linear control amplitudes (krotov_set_amplitudes)
     bool amp_set = false;
@@ -132,17 +136,22 @@ struct krotov_handle_s {
     std::vector<double> amp_shape;  // [L][N_T] (empty = 1)
     DevBuf d_amp_poly, d_amp_shape, d_amp_old, d_amp_dfac, d_amp_new;
     DevBuf d_emul;       // krotov_group_iterate: per-rank parameter blocks of the emulated multi-rank launch
-    bool peer_opened[kr::kMaxRanks] = {};
     long long iter_count = 0;
+    // the peers' mailboxes and chi trajectories mapped by krotov_comm_connect (peer_mbox / peer_Xbase point into them)
+    std::vector<kr::IpcMapping> peer_maps;
     // dense path
     kr::DenseEngine *dense = nullptr;
     // misc
-    cudaStream_t stream = nullptr;
-    cudaEvent_t ev0 = nullptr, ev1 = nullptr;
     int sm_count = 0;
     long long launches_total = 0, launches_last = 0, fallback_steps = 0;
     double ms_last = 0.0, ms_last_bw = 0.0;
     std::string err;
+
+    // peer mappings first, then the dense engine; the buffers (members) and the stream (base) follow
+    ~krotov_handle_s() {
+        peer_maps.clear();
+        kr::dense_destroy(dense);
+    }
 };
 
 namespace {
@@ -166,7 +175,7 @@ int fail(krotov_handle h, int code, const std::string &msg) {
 
 int dev_alloc(krotov_handle h, DevBuf &b, size_t bytes) {
     if (bytes == 0) bytes = 16;
-    if (b.p != nullptr && b.bytes >= bytes) return KROTOV_OK;  // reuse: cudaFree/cudaMalloc cost up to 100 ms
+    if (b && b.bytes() >= bytes) return KROTOV_OK;  // reuse: cudaFree/cudaMalloc cost up to 100 ms
     // small tables (Chebyshev coefficients, ...) grow by a few entries when a spectral range widens: give them
     // headroom so that a re-derived polynomial never re-allocates in the middle of an optimisation
     if (bytes < (1u << 20)) {
@@ -174,13 +183,11 @@ int dev_alloc(krotov_handle h, DevBuf &b, size_t bytes) {
         while (cap < 2 * bytes) cap <<= 1;
         bytes = cap;
     }
-    b.release();
-    cudaError_t e = cudaMalloc(&b.p, bytes);
+    const cudaError_t e = b.allocate(bytes);
     if (e != cudaSuccess) {
         h->err = std::string("cudaMalloc(") + std::to_string(bytes) + "): " + cudaGetErrorString(e);
         return e == cudaErrorMemoryAllocation ? KROTOV_ERR_NOMEM : KROTOV_ERR_CUDA;
     }
-    b.bytes = bytes;
     return KROTOV_OK;
 }
 
@@ -188,7 +195,7 @@ template <typename T>
 int upload(krotov_handle h, DevBuf &b, const std::vector<T> &v) {
     int rc = dev_alloc(h, b, v.size() * sizeof(T));
     if (rc) return rc;
-    if (!v.empty()) KR_CUDA(h, cudaMemcpy(b.p, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice));
+    if (!v.empty()) KR_CUDA(h, cudaMemcpy(b.get<void>(), v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice));
     return KROTOV_OK;
 }
 
@@ -649,31 +656,31 @@ void fill_warp_params(krotov_handle h, int mode, kr::WarpParams &p) {
     p.wpc = h->wpc; p.tpw = h->tpw; p.nCTA = h->nCTA; p.mode = mode; p.store_fw = h->store_fw;
     p.mu_hermitian = (h->mu_hermitian && !getenv("KROTOV_NO_FAST")) ? 1 : 0;
     p.ndtc_f = h->cheb[0].ndtc; p.ndtc_b = h->cheb[1].set ? h->cheb[1].ndtc : 1; p.mmax_f = h->cheb[0].mmax; p.mmax_b = h->cheb[1].set ? h->cheb[1].mmax : 1;
-    p.gen_of_traj = (const int *)h->d_gen.p;
-    p.cols = (const int *)h->d_cols.p;
-    p.Pf = (const double2 *)h->d_Pf.p; p.Pb = (const double2 *)h->d_Pb.p;
-    p.inv_s_f = (const double *)h->d_inv_s.p;
-    p.coef_f = (const double *)h->cheb[0].coef.p; p.m_f = (const int *)h->cheb[0].m.p;
-    p.phase_f = (const double2 *)h->cheb[0].phase.p;
-    p.coef_b = (const double *)h->cheb[1].coef.p; p.m_b = (const int *)h->cheb[1].m.p;
-    p.phase_b = (const double2 *)h->cheb[1].phase.p;
-    p.dtc_f = (const int *)h->cheb[0].dtc.p; p.dtc_b = (const int *)h->cheb[1].dtc.p; p.dt = (const double *)h->d_dt.p;
-    p.alpha = (const double *)h->d_alpha.p;
-    p.eps_old = (const double *)h->d_eps_old.p; p.eps_new = (double *)h->d_eps_new.p;
-    p.amp_old = h->amp_set ? (const double *)h->d_amp_old.p : p.eps_old;
-    p.amp_dfac = h->amp_set ? (const double *)h->d_amp_dfac.p : nullptr;
-    p.amp_poly = (h->amp_set && !h->amp_poly.empty()) ? (const double *)h->d_amp_poly.p : nullptr;
-    p.amp_shape = (h->amp_set && !h->amp_shape.empty()) ? (const double *)h->d_amp_shape.p : nullptr;
-    p.g_a_int = (double *)h->d_ga.p;
-    p.X = (double2 *)h->d_X.p; p.Phi = (double2 *)h->d_Phi.p;
-    p.psi0 = (const double2 *)h->d_psi0.p;
-    p.target = h->has_target ? (const double2 *)h->d_target.p : nullptr;
-    p.chiT = h->chiT_valid ? (const double2 *)h->d_chiT.p : nullptr;
-    p.chi_coef = (const double2 *)h->d_chicoef.p;
-    p.psi_final = (double2 *)h->d_psif.p; p.tau = (double2 *)h->d_tau.p;
-    p.R = (double *)h->d_R.p;
-    p.E = (double *)h->d_R.p + (size_t)h->N_T * h->nCTA * h->L;
-    p.acc = (h->nCTA > 1 && h->nCTA < 256 && !getenv("KROTOV_NO_ATOMIC_SUM")) ? (unsigned long long *)h->d_acc.p : nullptr;
+    p.gen_of_traj = h->d_gen.get<const int>();
+    p.cols = h->d_cols.get<const int>();
+    p.Pf = h->d_Pf.get<const double2>(); p.Pb = h->d_Pb.get<const double2>();
+    p.inv_s_f = h->d_inv_s.get<const double>();
+    p.coef_f = h->cheb[0].coef.get<const double>(); p.m_f = h->cheb[0].m.get<const int>();
+    p.phase_f = h->cheb[0].phase.get<const double2>();
+    p.coef_b = h->cheb[1].coef.get<const double>(); p.m_b = h->cheb[1].m.get<const int>();
+    p.phase_b = h->cheb[1].phase.get<const double2>();
+    p.dtc_f = h->cheb[0].dtc.get<const int>(); p.dtc_b = h->cheb[1].dtc.get<const int>(); p.dt = h->d_dt.get<const double>();
+    p.alpha = h->d_alpha.get<const double>();
+    p.eps_old = h->d_eps_old.get<const double>(); p.eps_new = h->d_eps_new.get<double>();
+    p.amp_old = h->amp_set ? h->d_amp_old.get<const double>() : p.eps_old;
+    p.amp_dfac = h->amp_set ? h->d_amp_dfac.get<const double>() : nullptr;
+    p.amp_poly = (h->amp_set && !h->amp_poly.empty()) ? h->d_amp_poly.get<const double>() : nullptr;
+    p.amp_shape = (h->amp_set && !h->amp_shape.empty()) ? h->d_amp_shape.get<const double>() : nullptr;
+    p.g_a_int = h->d_ga.get<double>();
+    p.X = h->d_X.get<double2>(); p.Phi = h->d_Phi.get<double2>();
+    p.psi0 = h->d_psi0.get<const double2>();
+    p.target = h->has_target ? h->d_target.get<const double2>() : nullptr;
+    p.chiT = h->chiT_valid ? h->d_chiT.get<const double2>() : nullptr;
+    p.chi_coef = h->d_chicoef.get<const double2>();
+    p.psi_final = h->d_psif.get<double2>(); p.tau = h->d_tau.get<double2>();
+    p.R = h->d_R.get<double>();
+    p.E = h->d_R.get<double>() + (size_t)h->N_T * h->nCTA * h->L;
+    p.acc = (h->nCTA > 1 && h->nCTA < 256 && !getenv("KROTOV_NO_ATOMIC_SUM")) ? h->d_acc.get<unsigned long long>() : nullptr;
     p.rank = h->rank; p.world = h->world;
     // Who polls the rank's mailbox: every CTA (no broadcast hop) while pollers x writers stay few, else the reducer
     // alone, which then broadcasts through E.  Measured on C4 (ms per iteration, all-poll / reducer-poll): 2 GPUs x
@@ -725,7 +732,7 @@ void fill_warp_params(krotov_handle h, int mode, kr::WarpParams &p) {
             p.rf_flag[r] = h->peer_flag[r];
         }
         p.X = p.Xr[h->rank];
-        p.rf_count = (unsigned int *)h->d_rfcount.p;
+        p.rf_count = h->d_rfcount.get<unsigned int>();
         p.rf_iter = (unsigned long long)(h->iter_count + 1);
         p.rf_stride = getenv("KROTOV_RF_STRIDE") ? std::max(1, atoi(getenv("KROTOV_RF_STRIDE"))) : 1;
         p.rf_pack = getenv("KROTOV_RF_PACK") ? (h->bw_hi - h->bw_lo + h->nCTA - 1) / h->nCTA : 0;
@@ -733,8 +740,8 @@ void fill_warp_params(krotov_handle h, int mode, kr::WarpParams &p) {
         p.rf_fwd = (h->lpt == 32 && !getenv("KROTOV_RF_DIRECT")) ? (getenv("KROTOV_RF_SLEEP") ? std::max(1, atoi(getenv("KROTOV_RF_SLEEP"))) : 1000) : 0;
         h->xchg_last = 5;
     }
-    p.err_flag = (int *)h->d_err.p;
-    p.prof = (long long *)h->d_prof.p;
+    p.err_flag = h->d_err.get<int>();
+    p.prof = h->d_prof.get<long long>();
     p.timeout_cycles = 20000000000ll;  // ~10 s
     if (const char *e = getenv("KROTOV_TIMEOUT_CYCLES")) p.timeout_cycles = atoll(e);
 }
@@ -745,8 +752,8 @@ int launch_warp(krotov_handle h, int mode) {
     if (h->tiny && h->world == 1 && !h->amp_set) {
         kr::TinyParams tp;
         tp.w = p;
-        tp.Tf = (const double2 *)h->d_Tf.p;
-        tp.Tb = (const double2 *)h->d_Tb.p;
+        tp.Tf = h->d_Tf.get<const double2>();
+        tp.Tb = h->d_Tb.get<const double2>();
         const int te = (1 + h->L) * h->d * h->d;
         const size_t term_bytes = te <= 12 ? 0 : (size_t)te * 32 * 16;
         const size_t coef_bytes = ((size_t)p.ndtc_f * p.mmax_f + (size_t)p.ndtc_b * p.mmax_b) * 32 * 8;
@@ -792,15 +799,15 @@ int launch_warp(krotov_handle h, int mode) {
 int check_err_flag(krotov_handle h) {
     int flags[4] = {0, 0, 0, 0};  // [0] exchange timed out, [1] time steps redone with the gather protocol,
                                   // [2..3] SM cycles CTA 0 waited at the rank barrier (replicated forward sweep)
-    KR_CUDA(h, cudaMemcpy(flags, h->d_err.p, sizeof(flags), cudaMemcpyDeviceToHost));
+    KR_CUDA(h, cudaMemcpy(flags, h->d_err.get<void>(), sizeof(flags), cudaMemcpyDeviceToHost));
     const int flag = flags[0];
     h->fallback_steps = flags[1];
     long long wait_cycles;
     memcpy(&wait_cycles, flags + 2, 8);
     h->ms_rank_wait = h->rf ? (double)wait_cycles / (double)h->sm_clock_khz : 0.0;
-    if (flags[1]) cudaMemset((int *)h->d_err.p + 1, 0, sizeof(int));
+    if (flags[1]) cudaMemset(h->d_err.get<int>() + 1, 0, sizeof(int));
     if (flag) {
-        cudaMemset(h->d_err.p, 0, sizeof(int));
+        cudaMemset(h->d_err.get<void>(), 0, sizeof(int));
         return fail(h, KROTOV_ERR_TIMEOUT, "in-kernel exchange timed out waiting for a partial sum");
     }
     return KROTOV_OK;
@@ -819,70 +826,21 @@ int krotov_destroy(krotov_handle h) {
     if (!h) return KROTOV_OK;
     cudaSetDevice(h->device);
     if (h->stream) cudaStreamSynchronize(h->stream);
-    for (int r = 0; r < kr::kMaxRanks; ++r) {
-        if (h->peer_opened[r])
-            for (int par = 0; par < 2; ++par)
-                if (h->peer_mbox[par][r]) cudaIpcCloseMemHandle(h->peer_mbox[par][r]);
-        if (h->peer_x_opened[r] && h->peer_Xbase[r]) cudaIpcCloseMemHandle(h->peer_Xbase[r]);
-    }
-    DevBuf *bufs[] = {&h->d_acc, &h->d_Tf, &h->d_Tb, &h->d_cols, &h->d_Pf, &h->d_Pb, &h->d_inv_s, &h->d_gen, &h->d_dt, &h->d_alpha,
-                      &h->d_eps_old, &h->d_eps_new, &h->d_ga, &h->d_X, &h->d_Phi, &h->d_psi0, &h->d_target,
-                      &h->d_chiT, &h->d_chicoef, &h->d_psif, &h->d_tau, &h->d_R, &h->d_err, &h->d_weight, &h->d_prof,
-                      &h->d_mbox[0], &h->d_mbox[1], &h->d_emul,
-                      &h->d_amp_poly, &h->d_amp_shape, &h->d_amp_old, &h->d_amp_dfac, &h->d_amp_new, &h->d_rfcount,
-                      &h->d_rawf, &h->d_rawb, &h->d_rowscale, &h->d_envamps, &h->d_envout};
-    for (DevBuf *b : bufs) b->release();
-    for (int dir = 0; dir < 2; ++dir) {
-        h->cheb[dir].coef.release();
-        h->cheb[dir].m.release();
-        h->cheb[dir].phase.release();
-        h->cheb[dir].dtc.release();
-    }
-    if (h->dense) {
-        kr::dense_destroy(h->dense);
-        h->dense = nullptr;
-    }
-    if (h->ev0) cudaEventDestroy(h->ev0);
-    if (h->ev1) cudaEventDestroy(h->ev1);
-    if (h->stream) cudaStreamDestroy(h->stream);
     delete h;
     return KROTOV_OK;
 }
 
-int krotov_create(const krotov_problem *pb, krotov_handle *out) {
-    if (!pb || !out) return fail(nullptr, KROTOV_ERR_ARG, "null argument");
-    *out = nullptr;
-    if (pb->struct_size != (int32_t)sizeof(krotov_problem))
-        return fail(nullptr, KROTOV_ERR_ARG, "krotov_problem.struct_size mismatch (ABI version?)");
-    if (pb->d < 1 || pb->n_traj < 1 || pb->n_steps < 1 || pb->n_gen < 1)
-        return fail(nullptr, KROTOV_ERR_ARG, "d, n_traj, n_steps, n_gen must be >= 1");
-    if (pb->n_ctrl < 1) return fail(nullptr, KROTOV_ERR_ARG, "no controls in trajectories: cannot optimize");
-    if (pb->n_ctrl > kr::kMaxCtrl) return fail(nullptr, KROTOV_ERR_UNSUPPORTED, "more than 8 controls");
-    if (!pb->tlist || !pb->gen_of_traj || !pb->gen_values || !pb->psi0 || !pb->update_shape || !pb->lambda_a)
-        return fail(nullptr, KROTOV_ERR_ARG, "null array in krotov_problem");
-    if (pb->gen_format == KROTOV_GEN_CSR && (!pb->csr_rowptr || !pb->csr_colind))
-        return fail(nullptr, KROTOV_ERR_ARG, "CSR pattern missing");
-    if (pb->functional != KROTOV_CHI_HOST && !pb->target)
-        return fail(nullptr, KROTOV_ERR_ARG, "built-in functional needs target states");
-    int ndev = 0;
-    cudaError_t ce = cudaGetDeviceCount(&ndev);
-    if (ce != cudaSuccess || ndev == 0)
-        return fail(nullptr, KROTOV_ERR_CUDA, std::string("no CUDA device: ") + cudaGetErrorString(ce));
-    if (pb->device < 0 || pb->device >= ndev) return fail(nullptr, KROTOV_ERR_ARG, "bad device ordinal");
+int64_t krotov_live_device_objects(void) { return kr::g_live_device_objects.load(); }
 
-    krotov_handle h = new krotov_handle_s();
-    auto bail = [&](int rc) {
-        g_create_error = h->err;
-        krotov_destroy(h);
-        return rc;
-    };
+// krotov_create past its argument checks: fills the fresh handle h; on failure h->err holds the message
+static int create_handle(krotov_handle h, const krotov_problem *pb) {
     h->d = pb->d; h->N = pb->n_traj; h->L = pb->n_ctrl; h->N_T = pb->n_steps; h->n_gen = pb->n_gen;
     h->functional = pb->functional;
     h->N_global = pb->n_traj_global > 0 ? pb->n_traj_global : pb->n_traj;
     h->store_fw = pb->store_fw; h->device = pb->device;
     h->rf_wanted = pb->replicated_forward != 0;
     const int d = h->d, N = h->N, L = h->L, N_T = h->N_T;
-    if (cudaSetDevice(h->device) != cudaSuccess) return bail(fail(h, KROTOV_ERR_CUDA, "cudaSetDevice failed"));
+    if (cudaSetDevice(h->device) != cudaSuccess) return fail(h, KROTOV_ERR_CUDA, "cudaSetDevice failed");
     cudaDeviceProp prop;
     cudaGetDeviceProperties(&prop, h->device);
     h->sm_count = prop.multiProcessorCount;
@@ -890,21 +848,21 @@ int krotov_create(const krotov_problem *pb, krotov_handle *out) {
         int khz = 0;
         if (cudaDeviceGetAttribute(&khz, cudaDevAttrClockRate, h->device) == cudaSuccess && khz > 0) h->sm_clock_khz = khz;
     }
-    if (prop.major < 10) return bail(fail(h, KROTOV_ERR_UNSUPPORTED, "libkrotov_cuda is built for sm_100a only"));
+    if (prop.major < 10) return fail(h, KROTOV_ERR_UNSUPPORTED, "libkrotov_cuda is built for sm_100a only");
     if (cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking) != cudaSuccess ||
         cudaEventCreate(&h->ev0) != cudaSuccess || cudaEventCreate(&h->ev1) != cudaSuccess)
-        return bail(fail(h, KROTOV_ERR_CUDA, "stream/event creation failed"));
+        return fail(h, KROTOV_ERR_CUDA, "stream/event creation failed");
 
     h->tlist.assign(pb->tlist, pb->tlist + N_T + 1);
     h->dt.resize(N_T);
     for (int n = 0; n < N_T; ++n) {
         h->dt[n] = h->tlist[n + 1] - h->tlist[n];
-        if (!(h->dt[n] > 0)) return bail(fail(h, KROTOV_ERR_ARG, "tlist must be strictly increasing"));
+        if (!(h->dt[n] > 0)) return fail(h, KROTOV_ERR_ARG, "tlist must be strictly increasing");
     }
     h->gen_of_traj.assign(pb->gen_of_traj, pb->gen_of_traj + N);
     for (int k = 0; k < N; ++k)
         if (h->gen_of_traj[k] < 0 || h->gen_of_traj[k] >= h->n_gen)
-            return bail(fail(h, KROTOV_ERR_ARG, "gen_of_traj out of range"));
+            return fail(h, KROTOV_ERR_ARG, "gen_of_traj out of range");
     h->weight.assign(N, 1.0);
     if (pb->weight) h->weight.assign(pb->weight, pb->weight + N);
     h->has_target = pb->target != nullptr;
@@ -912,11 +870,11 @@ int krotov_create(const krotov_problem *pb, krotov_handle *out) {
     // ---- generator ingestion.  `for_each_entry` walks the non-zeros of term (g, t) in either wire format.
     const cplx *vals = reinterpret_cast<const cplx *>(pb->gen_values);
     if (pb->gen_format != KROTOV_GEN_DENSE_COLMAJOR && pb->gen_format != KROTOV_GEN_CSR)
-        return bail(fail(h, KROTOV_ERR_ARG, "unknown gen_format"));
+        return fail(h, KROTOV_ERR_ARG, "unknown gen_format");
     if (pb->gen_format == KROTOV_GEN_CSR)
         for (int q = 0; q < pb->csr_rowptr[d]; ++q)
             if (pb->csr_colind[q] < 0 || pb->csr_colind[q] >= d)
-                return bail(fail(h, KROTOV_ERR_ARG, "CSR column out of range"));
+                return fail(h, KROTOV_ERR_ARG, "CSR column out of range");
     auto for_each_entry = [&](int g, int t, auto &&fn) {
         if (pb->term_present && !pb->term_present[(size_t)g * (1 + L) + t]) return;
         if (pb->gen_format == KROTOV_GEN_DENSE_COLMAJOR) {
@@ -933,9 +891,9 @@ int krotov_create(const krotov_problem *pb, krotov_handle *out) {
 
     int path = pb->force_path;
     if (path == KROTOV_PATH_WARP && d > 128)
-        return bail(fail(h, KROTOV_ERR_UNSUPPORTED, "warp path needs d <= 128"));
+        return fail(h, KROTOV_ERR_UNSUPPORTED, "warp path needs d <= 128");
     if (path != 0 && path != KROTOV_PATH_WARP && path != KROTOV_PATH_DENSE && path != KROTOV_PATH_SPARSE)
-        return bail(fail(h, KROTOV_ERR_ARG, "bad force_path"));
+        return fail(h, KROTOV_ERR_ARG, "bad force_path");
     auto fill_dense = [&]() {  // dense host copy of every term (row-major)
         h->Hdense.assign((size_t)h->n_gen * (1 + L) * d * d, cplx(0, 0));
         for (int g = 0; g < h->n_gen; ++g)
@@ -955,7 +913,7 @@ int krotov_create(const krotov_problem *pb, krotov_handle *out) {
             path = KROTOV_PATH_WARP;
             pattern_built = true;
         } else if (path == KROTOV_PATH_WARP) {
-            return bail(prc);
+            return prc;
         } else {
             h->err.clear();
         }
@@ -1024,31 +982,31 @@ int krotov_create(const krotov_problem *pb, krotov_handle *out) {
     // ---- buffers common to both paths
     std::vector<double> alpha((size_t)L * N_T);
     for (int l = 0; l < L; ++l) {
-        if (!(pb->lambda_a[l] != 0.0)) return bail(fail(h, KROTOV_ERR_ARG, "lambda_a must be non-zero"));
+        if (!(pb->lambda_a[l] != 0.0)) return fail(h, KROTOV_ERR_ARG, "lambda_a must be non-zero");
         for (int n = 0; n < N_T; ++n) alpha[(size_t)l * N_T + n] = pb->update_shape[(size_t)l * N_T + n] / pb->lambda_a[l];
     }
-    if ((rc = upload(h, h->d_alpha, alpha))) return bail(rc);
-    if ((rc = upload(h, h->d_dt, h->dt))) return bail(rc);
-    if ((rc = upload(h, h->d_gen, h->gen_of_traj))) return bail(rc);
-    if ((rc = upload(h, h->d_weight, h->weight))) return bail(rc);
-    if ((rc = dev_alloc(h, h->d_eps_old, (size_t)L * N_T * 8))) return bail(rc);
-    if ((rc = dev_alloc(h, h->d_eps_new, (size_t)L * N_T * 8))) return bail(rc);
-    if ((rc = dev_alloc(h, h->d_ga, kr::kMaxCtrl * 8))) return bail(rc);
-    if ((rc = dev_alloc(h, h->d_tau, (size_t)N * 16))) return bail(rc);
-    if ((rc = dev_alloc(h, h->d_chicoef, (size_t)N * 16))) return bail(rc);
-    if ((rc = dev_alloc(h, h->d_err, 16))) return bail(rc);
-    cudaMemset(h->d_err.p, 0, 16);
-    cudaMemset(h->d_tau.p, 0, (size_t)N * 16);
+    if ((rc = upload(h, h->d_alpha, alpha))) return rc;
+    if ((rc = upload(h, h->d_dt, h->dt))) return rc;
+    if ((rc = upload(h, h->d_gen, h->gen_of_traj))) return rc;
+    if ((rc = upload(h, h->d_weight, h->weight))) return rc;
+    if ((rc = dev_alloc(h, h->d_eps_old, (size_t)L * N_T * 8))) return rc;
+    if ((rc = dev_alloc(h, h->d_eps_new, (size_t)L * N_T * 8))) return rc;
+    if ((rc = dev_alloc(h, h->d_ga, kr::kMaxCtrl * 8))) return rc;
+    if ((rc = dev_alloc(h, h->d_tau, (size_t)N * 16))) return rc;
+    if ((rc = dev_alloc(h, h->d_chicoef, (size_t)N * 16))) return rc;
+    if ((rc = dev_alloc(h, h->d_err, 16))) return rc;
+    cudaMemset(h->d_err.get<void>(), 0, 16);
+    cudaMemset(h->d_tau.get<void>(), 0, (size_t)N * 16);
     // peer mailboxes for the per-time-step exchange between ranks: [N_T][L][rank], one per iteration parity
     // behind them (warp path): the accumulators of the one-hop cross-rank sum, word stride up to one 128-byte line
     h->mail_bytes = (size_t)N_T * kr::kMaxRanks * L * 8;
     h->xacc_bytes = (path == KROTOV_PATH_WARP && L * kr::kXLimbs <= 32) ? (size_t)N_T * L * kr::kXLimbs * kXaccMaxStride * 8 : 0;
     for (int par = 0; par < 2; ++par) {
-        if ((rc = dev_alloc(h, h->d_mbox[par], h->mail_bytes + h->xacc_bytes + 256))) return bail(rc);
-        cudaMemset((char *)h->d_mbox[par].p + h->mail_bytes + h->xacc_bytes, 0, 256);  // rank-barrier flags (parity 0 only)
-        cudaMemset(h->d_mbox[par].p, 0xFF, h->mail_bytes);
-        if (h->xacc_bytes) cudaMemset((char *)h->d_mbox[par].p + h->mail_bytes, 0, h->xacc_bytes);
-        h->peer_mbox[par][0] = (double *)h->d_mbox[par].p;
+        if ((rc = dev_alloc(h, h->d_mbox[par], h->mail_bytes + h->xacc_bytes + 256))) return rc;
+        cudaMemset(h->d_mbox[par].get<char>() + h->mail_bytes + h->xacc_bytes, 0, 256);  // rank-barrier flags (parity 0 only)
+        cudaMemset(h->d_mbox[par].get<void>(), 0xFF, h->mail_bytes);
+        if (h->xacc_bytes) cudaMemset(h->d_mbox[par].get<char>() + h->mail_bytes, 0, h->xacc_bytes);
+        h->peer_mbox[par][0] = h->d_mbox[par].get<double>();
     }
 
     // are all control terms Hermitian?  (mu_l^dagger = mu_l lets the kernel form mu_l chi ahead of time)
@@ -1062,14 +1020,14 @@ int krotov_create(const krotov_problem *pb, krotov_handle *out) {
                         break;
                     }
     if (path == KROTOV_PATH_WARP) {
-        if (!pattern_built && (rc = build_pattern(h))) return bail(rc);
-        if ((rc = upload(h, h->d_cols, h->cols))) return bail(rc);
+        if (!pattern_built && (rc = build_pattern(h))) return rc;
+        if ((rc = upload(h, h->d_cols, h->cols))) return rc;
         {
             std::vector<cplx> raw;
             build_raw_rows(h, KROTOV_FORWARD, raw);
-            if ((rc = upload(h, h->d_rawf, raw))) return bail(rc);
+            if ((rc = upload(h, h->d_rawf, raw))) return rc;
             build_raw_rows(h, KROTOV_BACKWARD, raw);
-            if ((rc = upload(h, h->d_rawb, raw))) return bail(rc);
+            if ((rc = upload(h, h->d_rawb, raw))) return rc;
         }
         choose_launch(h);
         h->tiny = d >= 2 && d <= 4 && N <= 32 && tiny_kernel_for(d, L) != nullptr && !getenv("KROTOV_NO_TINY");
@@ -1082,22 +1040,22 @@ int krotov_create(const krotov_problem *pb, krotov_handle *out) {
         };
         std::vector<cplx> tmp;
         pad_states(pb->psi0, tmp);
-        if ((rc = upload(h, h->d_psi0, tmp))) return bail(rc);
+        if ((rc = upload(h, h->d_psi0, tmp))) return rc;
         if (h->has_target) {
             pad_states(pb->target, tmp);
-            if ((rc = upload(h, h->d_target, tmp))) return bail(rc);
+            if ((rc = upload(h, h->d_target, tmp))) return rc;
         }
         const size_t slab = (size_t)N * (N_T + 1) * h->lpt * 16;
         h->x_slab = slab / 16;
         // (replicated forward sweep: two chi trajectories, by iteration parity -- a peer that is one iteration ahead
         // writes the other one)
-        if ((rc = dev_alloc(h, h->d_X, slab * (h->rf_wanted ? 2 : 1)))) return bail(rc);
-        if (h->store_fw && (rc = dev_alloc(h, h->d_Phi, slab))) return bail(rc);
-        if ((rc = dev_alloc(h, h->d_chiT, (size_t)N * h->lpt * 16))) return bail(rc);
-        if ((rc = dev_alloc(h, h->d_psif, (size_t)N * h->lpt * 16))) return bail(rc);
+        if ((rc = dev_alloc(h, h->d_X, slab * (h->rf_wanted ? 2 : 1)))) return rc;
+        if (h->store_fw && (rc = dev_alloc(h, h->d_Phi, slab))) return rc;
+        if ((rc = dev_alloc(h, h->d_chiT, (size_t)N * h->lpt * 16))) return rc;
+        if ((rc = dev_alloc(h, h->d_psif, (size_t)N * h->lpt * 16))) return rc;
         // Freshly initialised propagators hold the initial states: that is what `skip_initial_forward_propagation`
         // (src/optimize.jl:171-181) leaves for the first chi(T) (:297) and update_result! (:378-381)
-        cudaMemcpy(h->d_psif.p, h->d_psi0.p, (size_t)N * h->lpt * 16, cudaMemcpyDeviceToDevice);
+        cudaMemcpy(h->d_psif.get<void>(), h->d_psi0.get<void>(), (size_t)N * h->lpt * 16, cudaMemcpyDeviceToDevice);
         if (h->has_target) {
             std::vector<cplx> tau0(N);
             const cplx *s0 = reinterpret_cast<const cplx *>(pb->psi0), *tg = reinterpret_cast<const cplx *>(pb->target);
@@ -1106,14 +1064,14 @@ int krotov_create(const krotov_problem *pb, krotov_handle *out) {
                 for (int i = 0; i < d; ++i) a += std::conj(tg[(size_t)k * d + i]) * s0[(size_t)k * d + i];
                 tau0[k] = a;
             }
-            cudaMemcpy(h->d_tau.p, tau0.data(), (size_t)N * 16, cudaMemcpyHostToDevice);
+            cudaMemcpy(h->d_tau.get<void>(), tau0.data(), (size_t)N * 16, cudaMemcpyHostToDevice);
         }
         h->swept = true;
-        if ((rc = dev_alloc(h, h->d_R, ((size_t)N_T * h->nCTA * L + (size_t)N_T * L) * 8))) return bail(rc);
-        if ((rc = dev_alloc(h, h->d_acc, (size_t)N_T * L * kr::kFixLimbs * 8))) return bail(rc);
+        if ((rc = dev_alloc(h, h->d_R, ((size_t)N_T * h->nCTA * L + (size_t)N_T * L) * 8))) return rc;
+        if ((rc = dev_alloc(h, h->d_acc, (size_t)N_T * L * kr::kFixLimbs * 8))) return rc;
         if (getenv("KROTOV_PROF")) {
-            if ((rc = dev_alloc(h, h->d_prof, (size_t)h->nCTA * 8 * 8))) return bail(rc);
-            cudaMemset(h->d_prof.p, 0, h->d_prof.bytes);
+            if ((rc = dev_alloc(h, h->d_prof, (size_t)h->nCTA * 8 * 8))) return rc;
+            cudaMemset(h->d_prof.get<void>(), 0, h->d_prof.bytes());
         }
     } else {
         kr::SparseDesc sd;
@@ -1124,13 +1082,43 @@ int krotov_create(const krotov_problem *pb, krotov_handle *out) {
         h->dense = kr::dense_create(h->d, h->N, h->L, h->N_T, h->n_gen, h->Hdense, h->gen_of_traj, pb->psi0,
                                     pb->target, h->store_fw, h->stream, h->err,
                                     path == KROTOV_PATH_SPARSE ? &sd : nullptr);
-        if (!h->dense) return bail(KROTOV_ERR_UNSUPPORTED);
+        if (!h->dense) return KROTOV_ERR_UNSUPPORTED;
         std::vector<cplx>().swap(h->Hdense);  // the device holds the generators now
-        if (!kr::dense_seed(h->dense, (double2 *)h->d_tau.p, h->err)) return bail(KROTOV_ERR_CUDA);
+        if (!kr::dense_seed(h->dense, h->d_tau.get<double2>(), h->err)) return KROTOV_ERR_CUDA;
         h->swept = true;
     }
-    if (cudaDeviceSynchronize() != cudaSuccess) return bail(fail(h, KROTOV_ERR_CUDA, "device sync after create failed"));
-    *out = h;
+    if (cudaDeviceSynchronize() != cudaSuccess) return fail(h, KROTOV_ERR_CUDA, "device sync after create failed");
+    return KROTOV_OK;
+}
+
+int krotov_create(const krotov_problem *pb, krotov_handle *out) {
+    if (!pb || !out) return fail(nullptr, KROTOV_ERR_ARG, "null argument");
+    *out = nullptr;
+    if (pb->struct_size != (int32_t)sizeof(krotov_problem))
+        return fail(nullptr, KROTOV_ERR_ARG, "krotov_problem.struct_size mismatch (ABI version?)");
+    if (pb->d < 1 || pb->n_traj < 1 || pb->n_steps < 1 || pb->n_gen < 1)
+        return fail(nullptr, KROTOV_ERR_ARG, "d, n_traj, n_steps, n_gen must be >= 1");
+    if (pb->n_ctrl < 1) return fail(nullptr, KROTOV_ERR_ARG, "no controls in trajectories: cannot optimize");
+    if (pb->n_ctrl > kr::kMaxCtrl) return fail(nullptr, KROTOV_ERR_UNSUPPORTED, "more than 8 controls");
+    if (!pb->tlist || !pb->gen_of_traj || !pb->gen_values || !pb->psi0 || !pb->update_shape || !pb->lambda_a)
+        return fail(nullptr, KROTOV_ERR_ARG, "null array in krotov_problem");
+    if (pb->gen_format == KROTOV_GEN_CSR && (!pb->csr_rowptr || !pb->csr_colind))
+        return fail(nullptr, KROTOV_ERR_ARG, "CSR pattern missing");
+    if (pb->functional != KROTOV_CHI_HOST && !pb->target)
+        return fail(nullptr, KROTOV_ERR_ARG, "built-in functional needs target states");
+    int ndev = 0;
+    cudaError_t ce = cudaGetDeviceCount(&ndev);
+    if (ce != cudaSuccess || ndev == 0)
+        return fail(nullptr, KROTOV_ERR_CUDA, std::string("no CUDA device: ") + cudaGetErrorString(ce));
+    if (pb->device < 0 || pb->device >= ndev) return fail(nullptr, KROTOV_ERR_ARG, "bad device ordinal");
+
+    std::unique_ptr<krotov_handle_s> h(new krotov_handle_s());
+    const int rc = create_handle(h.get(), pb);
+    if (rc != KROTOV_OK) {
+        g_create_error = h->err;
+        return rc;
+    }
+    *out = h.release();
     return KROTOV_OK;
 }
 
@@ -1155,7 +1143,7 @@ int krotov_get_info(krotov_handle h, krotov_info *out) {
     out->launches_last = h->launches_last;
     out->ms_last = h->ms_last;
     out->ms_last_backward = h->ms_last_bw;
-    out->hbm_bytes_state = (int64_t)h->d_X.bytes;
+    out->hbm_bytes_state = (int64_t)h->d_X.bytes();
     out->fallback_steps = h->fallback_steps;
     out->ms_rank_wait = h->ms_rank_wait;
     if (h->dense) kr::dense_info(h->dense, out);
@@ -1212,7 +1200,7 @@ int krotov_set_cheby(krotov_handle h, int direction, int n_dt_class, const int32
         std::vector<cplx> rows;
         DevBuf &dP = direction == KROTOV_FORWARD ? h->d_Pf : h->d_Pb;
         const DevBuf &raw = direction == KROTOV_FORWARD ? h->d_rawf : h->d_rawb;
-        if (raw.p && !getenv("KROTOV_HOST_ROWS")) {
+        if (raw && !getenv("KROTOV_HOST_ROWS")) {
             // rows scaled on the device from the unscaled rows uploaded at krotov_create
             std::vector<double> fb((size_t)2 * h->n_gen);
             for (int g = 0; g < h->n_gen; ++g) {
@@ -1221,11 +1209,11 @@ int krotov_set_cheby(krotov_handle h, int direction, int n_dt_class, const int32
                 fb[2 * g + 1] = Delta[g] / 2 + E_min[g];
             }
             if ((rc = dev_alloc(h, h->d_rowscale, fb.size() * 8))) return rc;
-            KR_CUDA(h, cudaMemcpyAsync(h->d_rowscale.p, fb.data(), fb.size() * 8, cudaMemcpyHostToDevice, h->stream));
+            KR_CUDA(h, cudaMemcpyAsync(h->d_rowscale.get<void>(), fb.data(), fb.size() * 8, cudaMemcpyHostToDevice, h->stream));
             const size_t total = (size_t)h->n_gen * (1 + h->L) * (h->Wt + 1) * h->lpt;
             if ((rc = dev_alloc(h, dP, total * 16))) return rc;
             scale_rows_kernel<<<(unsigned)((total + 255) / 256), 256, 0, h->stream>>>(
-                (const double2 *)raw.p, (const double2 *)h->d_rowscale.p, (double2 *)dP.p, 1 + h->L, h->Wt, h->lpt, h->d, total);
+                raw.get<const double2>(), h->d_rowscale.get<const double2>(), dP.get<double2>(), 1 + h->L, h->Wt, h->lpt, h->d, total);
             KR_CUDA(h, cudaStreamSynchronize(h->stream));  // fb is a local; the next call may rewrite d_rowscale
             h->launches_total += 1;
             tr.lap("rows scaled on the device");
@@ -1306,7 +1294,7 @@ int krotov_forward(krotov_handle h, const double *pulses) {
     if (!h || !pulses) return KROTOV_ERR_ARG;
     if (!h->cheb[0].set) return fail(h, KROTOV_ERR_STATE, "krotov_set_cheby(FORWARD) must be called before krotov_forward");
     cudaSetDevice(h->device);
-    KR_CUDA(h, cudaMemcpyAsync(h->d_eps_old.p, pulses, (size_t)h->L * h->N_T * 8, cudaMemcpyHostToDevice, h->stream));
+    KR_CUDA(h, cudaMemcpyAsync(h->d_eps_old.get<void>(), pulses, (size_t)h->L * h->N_T * 8, cudaMemcpyHostToDevice, h->stream));
     int rc;
     if ((rc = prepare_amplitudes(h, pulses))) return rc;
     if ((rc = begin_timed(h))) return rc;
@@ -1314,7 +1302,7 @@ int krotov_forward(krotov_handle h, const double *pulses) {
         if ((rc = launch_warp(h, 0))) return rc;
     } else {
         std::string e;
-        if (!kr::dense_forward(h->dense, (const double *)h->d_eps_old.p, (double2 *)h->d_tau.p, h->launches_last, e))
+        if (!kr::dense_forward(h->dense, h->d_eps_old.get<const double>(), h->d_tau.get<double2>(), h->launches_last, e))
             return fail(h, KROTOV_ERR_CUDA, e);
     }
     if ((rc = end_timed(h))) return rc;
@@ -1333,7 +1321,7 @@ int krotov_set_chi(krotov_handle h, const double *chi) {
         const cplx *s = reinterpret_cast<const cplx *>(chi);
         for (int k = 0; k < N; ++k)
             for (int i = 0; i < d; ++i) tmp[(size_t)k * h->lpt + i] = s[(size_t)k * d + i];
-        KR_CUDA(h, cudaMemcpy(h->d_chiT.p, tmp.data(), tmp.size() * 16, cudaMemcpyHostToDevice));
+        KR_CUDA(h, cudaMemcpy(h->d_chiT.get<void>(), tmp.data(), tmp.size() * 16, cudaMemcpyHostToDevice));
     } else {
         std::string e;
         if (!kr::dense_set_chi(h->dense, chi, e)) return fail(h, KROTOV_ERR_CUDA, e);
@@ -1346,7 +1334,7 @@ int krotov_set_chi_coeffs(krotov_handle h, const double *coef) {
     if (!h || !coef) return KROTOV_ERR_ARG;
     if (!h->has_target) return fail(h, KROTOV_ERR_STATE, "krotov_set_chi_coeffs needs target states");
     cudaSetDevice(h->device);
-    KR_CUDA(h, cudaMemcpy(h->d_chicoef.p, coef, (size_t)h->N * 16, cudaMemcpyHostToDevice));
+    KR_CUDA(h, cudaMemcpy(h->d_chicoef.get<void>(), coef, (size_t)h->N * 16, cudaMemcpyHostToDevice));
     h->chicoef_valid = true;
     h->chiT_valid = false;
     return KROTOV_OK;
@@ -1367,25 +1355,25 @@ static int iterate_prepare(krotov_handle h, const double *guess_pulses) {
             return fail(h, KROTOV_ERR_STATE, "multi-rank J_T_sm needs krotov_set_chi_coeffs (global sum of tau)");
     }
     const size_t pbytes = (size_t)h->L * h->N_T * 8;
-    KR_CUDA(h, cudaMemcpyAsync(h->d_eps_old.p, guess_pulses, pbytes, cudaMemcpyHostToDevice, h->stream));
+    KR_CUDA(h, cudaMemcpyAsync(h->d_eps_old.get<void>(), guess_pulses, pbytes, cudaMemcpyHostToDevice, h->stream));
     int rc;
     if ((rc = prepare_amplitudes(h, guess_pulses))) return rc;
     if ((rc = begin_timed(h))) return rc;
     if (need_device_coef) {
-        chi_coef_kernel<<<1, 32, 0, h->stream>>>(h->functional, h->N, h->N_global, (const double2 *)h->d_tau.p,
-                                                 (const double *)h->d_weight.p, (double2 *)h->d_chicoef.p);
+        chi_coef_kernel<<<1, 32, 0, h->stream>>>(h->functional, h->N, h->N_global, h->d_tau.get<const double2>(),
+                                                 h->d_weight.get<const double>(), h->d_chicoef.get<double2>());
         h->launches_last += 1;
     }
-    if (h->rf) KR_CUDA(h, cudaMemsetAsync(h->d_rfcount.p, 0, 16, h->stream));
+    if (h->rf) KR_CUDA(h, cudaMemsetAsync(h->d_rfcount.get<void>(), 0, 16, h->stream));
     if (h->world > 1 && !h->rf) {
         // the mailbox of the NEXT iteration's parity is cleared now (peers are at most one iteration ahead)
         const int nxt = (int)((h->iter_count + 1) & 1);
-        KR_CUDA(h, cudaMemsetAsync(h->d_mbox[nxt].p, 0xFF, h->mail_bytes, h->stream));
-        if (h->xacc_bytes) KR_CUDA(h, cudaMemsetAsync((char *)h->d_mbox[nxt].p + h->mail_bytes, 0, h->xacc_bytes, h->stream));
+        KR_CUDA(h, cudaMemsetAsync(h->d_mbox[nxt].get<void>(), 0xFF, h->mail_bytes, h->stream));
+        if (h->xacc_bytes) KR_CUDA(h, cudaMemsetAsync(h->d_mbox[nxt].get<char>() + h->mail_bytes, 0, h->xacc_bytes, h->stream));
     }
     if (h->path == KROTOV_PATH_WARP) {
-        if (h->nCTA > 1 || h->world > 1) KR_CUDA(h, cudaMemsetAsync(h->d_R.p, 0xFF, h->d_R.bytes, h->stream));
-        if (h->nCTA > 1) KR_CUDA(h, cudaMemsetAsync(h->d_acc.p, 0, h->d_acc.bytes, h->stream));
+        if (h->nCTA > 1 || h->world > 1) KR_CUDA(h, cudaMemsetAsync(h->d_R.get<void>(), 0xFF, h->d_R.bytes(), h->stream));
+        if (h->nCTA > 1) KR_CUDA(h, cudaMemsetAsync(h->d_acc.get<void>(), 0, h->d_acc.bytes(), h->stream));
     }
     return KROTOV_OK;
 }
@@ -1395,8 +1383,8 @@ static int iterate_finish(krotov_handle h, double *new_pulses, double *g_a_int) 
     if ((rc = end_timed(h))) return rc;
     h->iter_count += 1;
     if ((rc = check_err_flag(h))) return rc;
-    KR_CUDA(h, cudaMemcpy(new_pulses, h->d_eps_new.p, (size_t)h->L * h->N_T * 8, cudaMemcpyDeviceToHost));
-    KR_CUDA(h, cudaMemcpy(g_a_int, h->d_ga.p, (size_t)h->L * 8, cudaMemcpyDeviceToHost));
+    KR_CUDA(h, cudaMemcpy(new_pulses, h->d_eps_new.get<void>(), (size_t)h->L * h->N_T * 8, cudaMemcpyDeviceToHost));
+    KR_CUDA(h, cudaMemcpy(g_a_int, h->d_ga.get<void>(), (size_t)h->L * 8, cudaMemcpyDeviceToHost));
     h->chiT_valid = false;
     h->chicoef_valid = false;
     h->swept = true;
@@ -1415,13 +1403,13 @@ int krotov_iterate(krotov_handle h, const double *guess_pulses, double *new_puls
         kr::DenseComm dc;
         dc.rank = h->rank;
         dc.world = h->world;
-        dc.err_flag = (int *)h->d_err.p;
+        dc.err_flag = h->d_err.get<int>();
         dc.timeout_cycles = 20000000000ll;
         for (int r = 0; r < kr::kMaxRanks; ++r) dc.mbox[r] = h->peer_mbox[(int)(h->iter_count & 1)][r];
         kr::dense_set_comm(h->dense, dc);
-        if (!kr::dense_iterate(h->dense, (const double *)h->d_eps_old.p, (double *)h->d_eps_new.p,
-                               (const double *)h->d_alpha.p, (const double *)h->d_dt.p, (double *)h->d_ga.p,
-                               h->chiT_valid ? nullptr : (const double2 *)h->d_chicoef.p, (double2 *)h->d_tau.p,
+        if (!kr::dense_iterate(h->dense, h->d_eps_old.get<const double>(), h->d_eps_new.get<double>(),
+                               h->d_alpha.get<const double>(), h->d_dt.get<const double>(), h->d_ga.get<double>(),
+                               h->chiT_valid ? nullptr : h->d_chicoef.get<const double2>(), h->d_tau.get<double2>(),
                                h->launches_last, e))
             return fail(h, KROTOV_ERR_CUDA, e);
         h->ms_last_bw = ms_bw;
@@ -1506,13 +1494,13 @@ int krotov_group_connect(krotov_handle *hs, int world) {
         h->iter_count = 0;
         h->rf = false;
         for (int q = 0; q < world; ++q)
-            for (int par = 0; par < 2; ++par) h->peer_mbox[par][q] = (double *)hs[q]->d_mbox[par].p;
+            for (int par = 0; par < 2; ++par) h->peer_mbox[par][q] = hs[q]->d_mbox[par].get<double>();
         if (rf_all) {
             int rc = rf_prepare(h, r, world);
             if (rc) return rc;
             for (int q = 0; q < world; ++q) {
-                h->peer_Xbase[q] = (double2 *)hs[q]->d_X.p;
-                h->peer_flag[q] = (unsigned long long *)((char *)hs[q]->d_mbox[0].p + hs[q]->mail_bytes + hs[q]->xacc_bytes);
+                h->peer_Xbase[q] = hs[q]->d_X.get<double2>();
+                h->peer_flag[q] = (unsigned long long *)(hs[q]->d_mbox[0].get<char>() + hs[q]->mail_bytes + hs[q]->xacc_bytes);
             }
         }
     }
@@ -1550,7 +1538,7 @@ int krotov_group_iterate(krotov_handle *hs, int world, const double *guess_pulse
     if ((rc = upload(h0, h0->d_emul, pv))) return rc;
     kr::WarpParams p0;
     memset(&p0, 0, sizeof(p0));
-    p0.emul = (const kr::WarpParams *)h0->d_emul.p;
+    p0.emul = h0->d_emul.get<const kr::WarpParams>();
     p0.emul_ranks = world;
     p0.wpc = h0->wpc;
     const KernelKey key{h0->Wt, h0->preg ? h0->L : 0, h0->lpt};
@@ -1568,7 +1556,7 @@ int krotov_group_iterate(krotov_handle *hs, int world, const double *guess_pulse
         void *args1[] = {(void *)&p0};
         KR_CUDA(h0, cudaLaunchCooperativeKernel((const void *)itr->second, grid, block, args1, smem, h0->stream));
         h0->launches_last += 1;
-        p0.emul = (const kr::WarpParams *)h0->d_emul.p + world;
+        p0.emul = h0->d_emul.get<const kr::WarpParams>() + world;
     }
     KR_CUDA(h0, cudaFuncSetAttribute((const void *)it->second, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     void *args[] = {(void *)&p0};
@@ -1610,11 +1598,11 @@ int krotov_set_amplitudes(krotov_handle h, int degree, const double *poly, const
     if (h->dense) {
         kr::AmpDev a;
         if (h->amp_set) {
-            a.amp_old = (const double *)h->d_amp_old.p;
-            a.dfac = (const double *)h->d_amp_dfac.p;
-            a.poly = h->amp_poly.empty() ? nullptr : (const double *)h->d_amp_poly.p;
-            a.shape = h->amp_shape.empty() ? nullptr : (const double *)h->d_amp_shape.p;
-            a.amp_new = (double *)h->d_amp_new.p;
+            a.amp_old = h->d_amp_old.get<const double>();
+            a.dfac = h->d_amp_dfac.get<const double>();
+            a.poly = h->amp_poly.empty() ? nullptr : h->d_amp_poly.get<const double>();
+            a.shape = h->amp_shape.empty() ? nullptr : h->d_amp_shape.get<const double>();
+            a.amp_new = h->d_amp_new.get<double>();
         }
         kr::dense_set_amp(h->dense, a);
     }
@@ -1627,7 +1615,7 @@ int krotov_get_states(krotov_handle h, double *states) {
     const int N = h->N, d = h->d;
     if (h->path == KROTOV_PATH_WARP) {
         std::vector<cplx> tmp((size_t)N * h->lpt);
-        KR_CUDA(h, cudaMemcpy(tmp.data(), h->d_psif.p, tmp.size() * 16, cudaMemcpyDeviceToHost));
+        KR_CUDA(h, cudaMemcpy(tmp.data(), h->d_psif.get<void>(), tmp.size() * 16, cudaMemcpyDeviceToHost));
         cplx *o = reinterpret_cast<cplx *>(states);
         for (int k = 0; k < N; ++k)
             for (int i = 0; i < d; ++i) o[(size_t)k * d + i] = tmp[(size_t)k * h->lpt + i];
@@ -1641,7 +1629,7 @@ int krotov_get_states(krotov_handle h, double *states) {
 int krotov_get_tau(krotov_handle h, double *tau) {
     if (!h || !tau) return KROTOV_ERR_ARG;
     cudaSetDevice(h->device);
-    KR_CUDA(h, cudaMemcpy(tau, h->d_tau.p, (size_t)h->N * 16, cudaMemcpyDeviceToHost));
+    KR_CUDA(h, cudaMemcpy(tau, h->d_tau.get<void>(), (size_t)h->N * 16, cudaMemcpyDeviceToHost));
     return KROTOV_OK;
 }
 
@@ -1654,7 +1642,7 @@ int krotov_get_storage(krotov_handle h, int which, int k, int n0, int n1, double
     if (h->path == KROTOV_PATH_WARP) {
         const DevBuf &b = which == KROTOV_FORWARD ? h->d_Phi : h->d_X;
         std::vector<cplx> tmp((size_t)(n1 - n0) * h->lpt);
-        const char *src = (const char *)b.p + ((size_t)k * (h->N_T + 1) + n0) * h->lpt * 16;
+        const char *src = b.get<const char>() + ((size_t)k * (h->N_T + 1) + n0) * h->lpt * 16;
         if (h->rf && which == KROTOV_BACKWARD && h->iter_count > 0)  // the chi trajectory of the LAST iteration's parity
             src += (size_t)((h->iter_count - 1) & 1) * h->x_slab * 16;
         KR_CUDA(h, cudaMemcpy(tmp.data(), src, tmp.size() * 16, cudaMemcpyDeviceToHost));
@@ -1671,19 +1659,19 @@ int krotov_get_storage(krotov_handle h, int which, int k, int n0, int n1, double
 int krotov_envelope_extremes_device(krotov_handle h, int n_corner, const double *amps, double *e_min, double *e_max) {
     if (!h) return KROTOV_ERR_ARG;
     if (n_corner < 1 || !amps || !e_min || !e_max) return fail(h, KROTOV_ERR_ARG, "bad argument to krotov_envelope_extremes_device");
-    if (h->path != KROTOV_PATH_WARP || h->lpt != 32 || !h->d_rawf.p)
+    if (h->path != KROTOV_PATH_WARP || h->lpt != 32 || !h->d_rawf)
         return fail(h, KROTOV_ERR_UNSUPPORTED, "krotov_envelope_extremes_device: persistent kernel path with d <= 32 only");
     cudaSetDevice(h->device);
     int rc;
     const size_t n_out = (size_t)h->n_gen * n_corner;
     if ((rc = dev_alloc(h, h->d_envamps, (size_t)n_corner * h->L * 8 + 16))) return rc;
     if ((rc = dev_alloc(h, h->d_envout, n_out * 16))) return rc;
-    KR_CUDA(h, cudaMemcpyAsync(h->d_envamps.p, amps, (size_t)n_corner * h->L * 8, cudaMemcpyHostToDevice, h->stream));
-    jacobi_extremes_kernel<<<(unsigned)n_out, 32, 0, h->stream>>>((const double2 *)h->d_rawf.p, (const int *)h->d_cols.p,
-                                                                  (const double *)h->d_envamps.p, (double2 *)h->d_envout.p,
+    KR_CUDA(h, cudaMemcpyAsync(h->d_envamps.get<void>(), amps, (size_t)n_corner * h->L * 8, cudaMemcpyHostToDevice, h->stream));
+    jacobi_extremes_kernel<<<(unsigned)n_out, 32, 0, h->stream>>>(h->d_rawf.get<const double2>(), h->d_cols.get<const int>(),
+                                                                  h->d_envamps.get<const double>(), h->d_envout.get<double2>(),
                                                                   h->L, h->Wt, h->d, n_corner);
     std::vector<double> out(2 * n_out);
-    KR_CUDA(h, cudaMemcpyAsync(out.data(), h->d_envout.p, n_out * 16, cudaMemcpyDeviceToHost, h->stream));
+    KR_CUDA(h, cudaMemcpyAsync(out.data(), h->d_envout.get<void>(), n_out * 16, cudaMemcpyDeviceToHost, h->stream));
     KR_CUDA(h, cudaStreamSynchronize(h->stream));
     h->launches_total += 1;
     for (int g = 0; g < h->n_gen; ++g) {
@@ -1701,10 +1689,10 @@ int krotov_envelope_extremes_device(krotov_handle h, int n_corner, const double 
 int krotov_get_profile(krotov_handle h, int cta, int64_t *out) {
     if (!h || !out) return KROTOV_ERR_ARG;
     for (int i = 0; i < 8; ++i) out[i] = 0;
-    if (!h->d_prof.p) return fail(h, KROTOV_ERR_STATE, "profiling counters are off (set KROTOV_PROF=1 before krotov_create)");
+    if (!h->d_prof) return fail(h, KROTOV_ERR_STATE, "profiling counters are off (set KROTOV_PROF=1 before krotov_create)");
     cudaSetDevice(h->device);
     std::vector<long long> tmp((size_t)h->nCTA * 8);
-    KR_CUDA(h, cudaMemcpy(tmp.data(), h->d_prof.p, tmp.size() * 8, cudaMemcpyDeviceToHost));
+    KR_CUDA(h, cudaMemcpy(tmp.data(), h->d_prof.get<void>(), tmp.size() * 8, cudaMemcpyDeviceToHost));
     if (cta >= h->nCTA) return fail(h, KROTOV_ERR_ARG, "cta out of range");
     for (int c = 0; c < h->nCTA; ++c)
         if (cta < 0 || c == cta)
@@ -1729,8 +1717,8 @@ int krotov_comm_export(krotov_handle h, void *desc) {
     cudaSetDevice(h->device);
     CommDesc cd;
     memset(&cd, 0, sizeof(cd));
-    for (int par = 0; par < 2; ++par) KR_CUDA(h, cudaIpcGetMemHandle(&cd.mh[par], h->d_mbox[par].p));
-    if (h->path == KROTOV_PATH_WARP) KR_CUDA(h, cudaIpcGetMemHandle(&cd.xh, h->d_X.p));
+    for (int par = 0; par < 2; ++par) KR_CUDA(h, cudaIpcGetMemHandle(&cd.mh[par], h->d_mbox[par].get<void>()));
+    if (h->path == KROTOV_PATH_WARP) KR_CUDA(h, cudaIpcGetMemHandle(&cd.xh, h->d_X.get<void>()));
     memset(desc, 0, KROTOV_COMM_DESC_BYTES);
     memcpy(desc, &cd, sizeof(cd));
     CommDescTail tail{h->path == KROTOV_PATH_WARP ? h->nCTA : 0, h->N, h->N_global, rf_eligible(h) ? 1 : 0};
@@ -1742,6 +1730,7 @@ int krotov_comm_connect(krotov_handle h, int rank, int world, const void *descs)
     if (!h || !descs) return KROTOV_ERR_ARG;
     if (world < 1 || world > kr::kMaxRanks || rank < 0 || rank >= world) return fail(h, KROTOV_ERR_ARG, "bad rank/world");
     cudaSetDevice(h->device);
+    h->peer_maps.clear();  // the mappings of an earlier connect
     h->rank = rank;
     h->world = world;
     h->total_ctas = 0;
@@ -1766,30 +1755,26 @@ int krotov_comm_connect(krotov_handle h, int rank, int world, const void *descs)
     }
     for (int r = 0; r < world; ++r) {
         if (r == rank) {
-            for (int par = 0; par < 2; ++par) h->peer_mbox[par][r] = (double *)h->d_mbox[par].p;
+            for (int par = 0; par < 2; ++par) h->peer_mbox[par][r] = h->d_mbox[par].get<double>();
             continue;
         }
         CommDesc cd;
         memcpy(&cd, (const char *)descs + (size_t)r * KROTOV_COMM_DESC_BYTES, sizeof(cd));
         for (int par = 0; par < 2; ++par) {
-            void *ptr = nullptr;
-            KR_CUDA(h, cudaIpcOpenMemHandle(&ptr, cd.mh[par], cudaIpcMemLazyEnablePeerAccess));
-            h->peer_mbox[par][r] = (double *)ptr;
+            KR_CUDA(h, h->peer_maps.emplace_back().open(cd.mh[par]));
+            h->peer_mbox[par][r] = h->peer_maps.back().get<double>();
         }
-        h->peer_opened[r] = true;
     }
     h->iter_count = 0;
     if (h->rf) {  // the peers' chi trajectories (both parities in one allocation) and their rank-barrier flags
         for (int r = 0; r < world; ++r) {
             if (r == rank) {
-                h->peer_Xbase[r] = (double2 *)h->d_X.p;
+                h->peer_Xbase[r] = h->d_X.get<double2>();
             } else {
                 CommDesc cd;
                 memcpy(&cd, (const char *)descs + (size_t)r * KROTOV_COMM_DESC_BYTES, sizeof(cd));
-                void *ptr = nullptr;
-                KR_CUDA(h, cudaIpcOpenMemHandle(&ptr, cd.xh, cudaIpcMemLazyEnablePeerAccess));
-                h->peer_Xbase[r] = (double2 *)ptr;
-                h->peer_x_opened[r] = true;
+                KR_CUDA(h, h->peer_maps.emplace_back().open(cd.xh));
+                h->peer_Xbase[r] = h->peer_maps.back().get<double2>();
             }
             h->peer_flag[r] = (unsigned long long *)((char *)h->peer_mbox[0][r] + h->mail_bytes + h->xacc_bytes);
         }

@@ -55,8 +55,15 @@ def _worker(rank, world, port, kind, n_samples, n_grid, iters, q, env=None):
         comm = Comm(device=rank)
         w = _make(kind, n_samples, n_grid)
         hist = {"J_T": [], "shard": None}
+        live = K._lib.lib().krotov_live_device_objects
+        hist["live"] = [live()]
 
         def cb(wrk, it, eps_new, eps_old):
+            if it == 0 and (env or {}).get("TEST_RECONNECT"):
+                # connecting again drops the peer mappings of the first connect before it maps the peers anew
+                hist["live"].append(live())
+                comm.connect(wrk.engine)
+                hist["live"].append(live())
             hist["fallback"] = hist.get("fallback", 0) + wrk.engine.info()["fallback_steps"]
             hist["J_T"].append(wrk.result.J_T)
             hist["pulses"] = np.array([np.array(e) for e in eps_new])
@@ -70,8 +77,9 @@ def _worker(rank, world, port, kind, n_samples, n_grid, iters, q, env=None):
             extra["force_path"] = 3
         extra["multi_gpu"] = (env or {}).get("TEST_MULTI_GPU", "shard")
         res = K.optimize(to_problem(w, iter_stop=iters, callback=cb, device=rank, **extra), method=K.Krotov, comm=comm)
+        hist["live"].append(live())
         q.put((rank, hist["J_T"], hist["pulses"], hist["shard"], res.message, np.array(res.states), hist["ga"],
-               hist["fallback"]))
+               hist["fallback"], hist["live"]))
     finally:
         dist.destroy_process_group()
 
@@ -84,7 +92,7 @@ def _worker(rank, world, port, kind, n_samples, n_grid, iters, q, env=None):
     ("sm", 20, 21, {}), ("ss", 9, 21, {}), ("sm", 20, 21, {"KROTOV_NO_SWEEP_RANKS": "1"}),
     ("chain", 40, 21, {}), ("chain", 40, 21, {"KROTOV_NO_SWEEP_RANKS": "1"}),
     ("c4", 8, 201, {"TEST_MULTI_GPU": "replicate"}), ("c4", 64, 101, {"TEST_MULTI_GPU": "replicate"}),
-    ("c4", 3, 101, {"TEST_MULTI_GPU": "auto"})])
+    ("c4", 3, 101, {"TEST_MULTI_GPU": "auto"}), ("c4", 8, 201, {"TEST_MULTI_GPU": "replicate", "TEST_RECONNECT": "1"})])
 def test_two_ranks_match_single_gpu(kind, n_samples, n_grid, env):
     """kind c4: warp path (in-kernel exchange of the comm warps); kinds sm/ss: dense generators (d = 64: the cluster
     sweep, rank sums through the mailboxes from inside the sweep; with KROTOV_NO_SWEEP_RANKS the DMMA stream with the
@@ -108,7 +116,11 @@ def test_two_ranks_match_single_gpu(kind, n_samples, n_grid, env):
     for p in procs:
         p.join(timeout=60)
         assert p.exitcode == 0
-    (r0, J0, P0, s0, m0, st0, ga0, fb0), (r1, J1, P1, s1, m1, st1, ga1, fb1) = out
+    (r0, J0, P0, s0, m0, st0, ga0, fb0, live0), (r1, J1, P1, s1, m1, st1, ga1, fb1, live1) = out
+    for live in (live0, live1):  # every rank gives back all it allocated and mapped
+        assert live[-1] == live[0]
+        if env.get("TEST_RECONNECT"):
+            assert live[1] == live[2] > live[0]
     assert m0 == m1 == "Reached maximum number of iterations"
     n_traj = 4 * n_samples if kind == "c4" else n_samples
     replicated = env.get("TEST_MULTI_GPU") in ("replicate", "auto")
