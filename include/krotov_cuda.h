@@ -177,6 +177,13 @@ int krotov_set_cheby(krotov_handle h, int direction, int n_dt_class, const int32
  * krotov_set_cheby from the amplitudes' range. */
 int krotov_set_amplitudes(krotov_handle h, int degree, const double *poly, const double *shape);
 
+/* Saturating (bounded) control amplitudes: pulse parametrizations such as QuantumControl's TanhParametrization.
+ * s: [L] or NULL.  s[l] > 0: control l enters as shape[l][n] * poly_l(tanh(s[l] * eps)); s[l] == 0: as today.
+ * NULL restores s = 0 for all controls.  Non-finite or negative s -> KROTOV_ERR_ARG.  A control with s[l] > 0 makes
+ * the problem non-linear even when krotov_set_amplitudes left poly and shape NULL (poly_l(x) = x then).  Independent of
+ * krotov_set_amplitudes (either may be called first); takes effect with the next krotov_forward / krotov_iterate. */
+int krotov_set_amplitude_saturation(krotov_handle h, const double *s);
+
 /* ---- the hot path ----------------------------------------------------------------------
  * krotov_forward: forward propagation of every trajectory under `pulses` without update.
  * Replaces the loop over krotov_initial_fw_prop! (src/optimize.jl:182-184, 247-265).  Leaves

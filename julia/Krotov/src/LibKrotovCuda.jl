@@ -118,6 +118,12 @@ function set_amplitudes(h, poly::Union{Nothing,Matrix{Float64}}, shape::Union{No
                    poly === nothing ? C_NULL : pointer(poly), shape === nothing ? C_NULL : pointer(shape)))
 end
 
+# s[l] > 0: control l enters as shape[l][n] * poly_l(tanh(s[l] * eps)) (bounded amplitudes); `nothing` restores s = 0
+function set_amplitude_saturation(h, s::Union{Nothing,Vector{Float64}})
+    check(h, ccall((:krotov_set_amplitude_saturation, lib), Cint, (Ptr{Cvoid}, Ptr{Float64}), h.ptr,
+                   s === nothing ? C_NULL : pointer(s)))
+end
+
 # pulses: Matrix{Float64}(N_T, L), column-major == [L][N_T] row-major on the wire
 forward(h, pulses::Matrix{Float64}) =
     check(h, ccall((:krotov_forward, lib), Cint, (Ptr{Cvoid}, Ptr{Float64}), h.ptr, pulses))

@@ -12,7 +12,9 @@ interface; all propagation runs in ``libkrotov_cuda.so`` (``csrc/``), with no CP
 from .controls import discretize, discretize_on_midpoints, get_control_derivs, get_controls
 from .errors import ArgumentError, ErrorException
 from .functionals import J_T_re, J_T_sm, J_T_ss, chi_re, chi_sm, chi_ss, make_chi, taus
-from .generators import Generator, PolynomialAmplitude, ShapedAmplitude, hamiltonian
+from .generators import (Generator, LogisticParametrization, LogisticSqParametrization, ParametrizedAmplitude,
+                         PolynomialAmplitude, ShapedAmplitude, SquareParametrization, TanhParametrization,
+                         TanhSqParametrization, hamiltonian)
 from .optimize import (Cheby, Krotov, finalize_result, krotov_initial_fw_prop, krotov_iteration,
                        make_krotov_print_iters, make_print_iters, optimize, optimize_krotov, update_result,
                        update_sigma)

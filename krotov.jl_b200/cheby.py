@@ -131,7 +131,7 @@ class ChebyDirection:
         self.H0, self.Hc = H0, Hc
         # `device_envelope(corners) -> (e_min, e_max)`: the engine's solver for the generators it holds (ensembles)
         self._device_envelope = device_envelope
-        # non-linear amplitudes: `amplitude(l, eps)` = coefficient of H_l for the control value eps (range corners)
+        # non-linear amplitudes: `amplitude(l, lo, hi)` = coefficients of H_l at the two sides of the control range
         self._amplitude = amplitude
         # spectral envelopes by control ranges.  The two directions of a Hermitian problem propagate with the
         # same matrices and meet the same ranges one iteration apart (the forward check sees the pulse
@@ -174,8 +174,9 @@ class ChebyDirection:
         lo = [r[0] for r in self.control_ranges]
         hi = [r[1] for r in self.control_ranges]
         if self._amplitude is not None:  # the generator at the range corners carries a_l(corner), not the corner itself
-            lo = [self._amplitude(l, v) for l, v in enumerate(lo)]
-            hi = [self._amplitude(l, v) for l, v in enumerate(hi)]
+            corners = [self._amplitude(l, a, b) for l, (a, b) in enumerate(zip(lo, hi))]
+            lo = [c[0] for c in corners]
+            hi = [c[1] for c in corners]
         key = tuple(self.control_ranges)
         if self.manual is not None:
             e_min = np.full(n_gen, self.manual[0])

@@ -10,9 +10,9 @@ __all__ = ["discretize", "discretize_on_midpoints", "get_controls", "get_control
 
 def control_of(amplitude):
     """The control object behind an amplitude (the amplitude itself for a plain control function / vector)."""
-    from .generators import PolynomialAmplitude
+    from .generators import ControlAmplitude
 
-    return amplitude.control if isinstance(amplitude, PolynomialAmplitude) else amplitude
+    return amplitude.control if isinstance(amplitude, ControlAmplitude) else amplitude
 
 
 def _as_grid(tlist):
@@ -111,14 +111,14 @@ def get_control_derivs(generator, controls):
 def get_amplitudes(generator, controls):
     """``[amplitude object of control c or None]``: the non-linear / shaped amplitude through which each control enters
     ``generator`` (None = the control itself multiplies its operator).  One amplitude per control and generator."""
-    from .generators import Generator, PolynomialAmplitude
+    from .generators import ControlAmplitude, Generator
 
     out = []
     for c in controls:
         found = None
         if isinstance(generator, Generator):
             for a in generator.amplitudes:
-                if control_of(a) is c and isinstance(a, PolynomialAmplitude):
+                if control_of(a) is c and isinstance(a, ControlAmplitude):
                     if found is not None and found is not a:
                         raise ValueError("a control enters one generator through two different amplitudes: unsupported")
                     found = a

@@ -374,8 +374,15 @@ __global__ void build_G_kernel(double2 *G, const double2 *H, int dp, int L, doub
     }
 }
 
+// x = tanh(s_l e) for a saturating control (bounded amplitudes), else e.  Out of line: the persistent sweeps that
+// inline amp_apply keep their register allocation whether or not saturation is in use.
+static __device__ __noinline__ double amp_saturate(const double *sat, const int l, const double e) {
+    return sat[l] != 0.0 ? tanh(sat[l] * e) : e;
+}
+
 // coefficient of H_l in the generator for the control value e (non-linear amplitudes, src/optimize.jl:268-272)
-__device__ __forceinline__ double amp_apply(const AmpDev &am, const int l, const int N_T, const int n, const double e) {
+__device__ __forceinline__ double amp_apply(const AmpDev &am, const int l, const int N_T, const int n, double e) {
+    if (am.sat != nullptr) e = amp_saturate(am.sat, l, e);
     double c = e;
     if (am.poly != nullptr) {
         const double *q = am.poly + l * (kAmpDeg + 1);
@@ -1560,7 +1567,10 @@ void dense_set_comm(DenseEngine *e, const DenseComm &c) { e->comm = c; }
 
 void dense_destroy(DenseEngine *e) { delete e; }
 
-void dense_set_amp(DenseEngine *e, const AmpDev &a) { e->amp = a; }
+void dense_set_amp(DenseEngine *e, const AmpDev &a) {
+    e->amp = a;
+    e->cheb_version++;  // the amplitude pointers travel by value in the launch parameters: a captured iteration is stale now
+}
 
 void dense_info(DenseEngine *e, krotov_info *out) {
     out->grid_blocks = e->sparse ? (e->sweep_launches ? e->sw_grid : e->dp / SP_ROWS) : (e->streamk ? e->sm_count : e->dp / BM);

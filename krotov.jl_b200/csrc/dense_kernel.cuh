@@ -17,13 +17,15 @@ struct DenseComm {  // per-iteration view of the rank mailboxes (see krotov_comm
     long long timeout_cycles = 0;
 };
 void dense_set_comm(DenseEngine *e, const DenseComm &c);
-// Non-linear control amplitudes on the device (krotov_set_amplitudes); every pointer null = linear controls.
+// Non-linear control amplitudes on the device (krotov_set_amplitudes, krotov_set_amplitude_saturation); every pointer
+// null = linear controls.
 constexpr int kAmpDeg = 4;
 struct AmpDev {
     const double *amp_old = nullptr;  // [L][N_T] a_l(eps_old): coefficients of the generator under the known pulses
     const double *dfac = nullptr;     // [L][N_T] a_l'(eps_old): factor of mu_l (src/optimize.jl:337-346)
     const double *poly = nullptr;     // [L][kAmpDeg+1] polynomial coefficients, ascending powers
     const double *shape = nullptr;    // [L][N_T] per-interval factor
+    const double *sat = nullptr;      // [L] s_l > 0: the polynomial is evaluated at tanh(s_l eps) (bounded amplitudes)
     double *amp_new = nullptr;        // [L][N_T] a_l(eps_new), written by the pulse update (launch-per-term stream)
 };
 void dense_set_amp(DenseEngine *e, const AmpDev &a);

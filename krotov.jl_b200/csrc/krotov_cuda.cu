@@ -130,11 +130,14 @@ struct krotov_handle_s : HandleStream {
     double2 *peer_Xbase[kr::kMaxRanks] = {};      // chi trajectories of every rank (parity p at + p * x_slab)
     unsigned long long *peer_flag[kr::kMaxRanks] = {};
     int xchg_last = 0;   // cross-rank protocol of the last launch: 0 none, 1 hier, 2 onehop, 3 mailboxes
-    // non-linear control amplitudes (krotov_set_amplitudes)
-    bool amp_set = false;
+    // non-linear control amplitudes (krotov_set_amplitudes, krotov_set_amplitude_saturation)
+    bool amp_set = false;           // poly, shape or saturation present
     std::vector<double> amp_poly;   // [L][kAmpMaxDeg+1], ascending powers (empty = a(eps) = eps)
     std::vector<double> amp_shape;  // [L][N_T] (empty = 1)
-    DevBuf d_amp_poly, d_amp_shape, d_amp_old, d_amp_dfac, d_amp_new;
+    std::vector<double> amp_sat;    // [L] s_l: the polynomial is evaluated at tanh(s_l eps) where s_l > 0 (empty = none)
+    std::vector<double> amp_rows;   // [L][kAmpRow]: the warp kernels' table, amp_poly rows (a(eps) = eps if empty) then s_l
+    std::vector<double> amp_old_host, amp_dfac_host;  // a(eps_old), a'(eps_old): sources of the stream-ordered uploads
+    DevBuf d_amp_poly, d_amp_shape, d_amp_sat, d_amp_rows, d_amp_old, d_amp_dfac, d_amp_new;
     DevBuf d_emul;       // krotov_group_iterate: per-rank parameter blocks of the emulated multi-rank launch
     long long iter_count = 0;
     // the peers' mailboxes and chi trajectories mapped by krotov_comm_connect (peer_mbox / peer_Xbase point into them)
@@ -196,6 +199,18 @@ int upload(krotov_handle h, DevBuf &b, const std::vector<T> &v) {
     int rc = dev_alloc(h, b, v.size() * sizeof(T));
     if (rc) return rc;
     if (!v.empty()) KR_CUDA(h, cudaMemcpy(b.get<void>(), v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice));
+    return KROTOV_OK;
+}
+
+// the same, ordered on the handle's stream: the sweeps that read the table run on that (non-blocking) stream, and a
+// blocking copy on the legacy stream from pageable memory may return before its DMA lands.  `v` must outlive the copy,
+// so callers pass vectors the handle owns.
+template <typename T>
+int upload_async(krotov_handle h, DevBuf &b, const std::vector<T> &v) {
+    int rc = dev_alloc(h, b, v.size() * sizeof(T));
+    if (rc) return rc;
+    if (!v.empty())
+        KR_CUDA(h, cudaMemcpyAsync(b.get<void>(), v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice, h->stream));
     return KROTOV_OK;
 }
 
@@ -669,7 +684,7 @@ void fill_warp_params(krotov_handle h, int mode, kr::WarpParams &p) {
     p.eps_old = h->d_eps_old.get<const double>(); p.eps_new = h->d_eps_new.get<double>();
     p.amp_old = h->amp_set ? h->d_amp_old.get<const double>() : p.eps_old;
     p.amp_dfac = h->amp_set ? h->d_amp_dfac.get<const double>() : nullptr;
-    p.amp_poly = (h->amp_set && !h->amp_poly.empty()) ? h->d_amp_poly.get<const double>() : nullptr;
+    p.amp_poly = (h->amp_set && !h->amp_rows.empty()) ? h->d_amp_rows.get<const double>() : nullptr;
     p.amp_shape = (h->amp_set && !h->amp_shape.empty()) ? h->d_amp_shape.get<const double>() : nullptr;
     p.g_a_int = h->d_ga.get<double>();
     p.X = h->d_X.get<double2>(); p.Phi = h->d_Phi.get<double2>();
@@ -1248,12 +1263,26 @@ int krotov_set_cheby(krotov_handle h, int direction, int n_dt_class, const int32
 static int prepare_amplitudes(krotov_handle h, const double *pulses) {
     if (!h->amp_set) return KROTOV_OK;
     const int L = h->L, N_T = h->N_T, D = kr::kAmpMaxDeg;
-    std::vector<double> a((size_t)L * N_T), da((size_t)L * N_T);
-    for (int l = 0; l < L; ++l)
+    std::vector<double> &a = h->amp_old_host, &da = h->amp_dfac_host;
+    a.resize((size_t)L * N_T);
+    da.resize((size_t)L * N_T);
+    for (int l = 0; l < L; ++l) {
+        const double s = h->amp_sat.empty() ? 0.0 : h->amp_sat[l];
         for (int n = 0; n < N_T; ++n) {
             const double e = pulses[(size_t)l * N_T + n];
             double v = e, dv = 1.0;
-            if (!h->amp_poly.empty()) {
+            if (s > 0.0) {  // saturating: x = tanh(s e), a = shape P(x), a' = shape P'(x) s (1 - x)(1 + x)
+                const double x = std::tanh(s * e);
+                v = x;
+                if (!h->amp_poly.empty()) {
+                    const double *q = &h->amp_poly[(size_t)l * (D + 1)];
+                    v = q[D];
+                    for (int p = D - 1; p >= 0; --p) v = std::fma(v, x, q[p]);  // same Horner form as the kernels
+                    dv = 0.0;
+                    for (int p = D; p >= 1; --p) dv = dv * x + p * q[p];
+                }
+                dv = dv * s * ((1.0 - x) * (1.0 + x));
+            } else if (!h->amp_poly.empty()) {
                 const double *q = &h->amp_poly[(size_t)l * (D + 1)];
                 v = q[D];
                 for (int p = D - 1; p >= 0; --p) v = std::fma(v, e, q[p]);  // same Horner form as the kernels
@@ -1268,9 +1297,10 @@ static int prepare_amplitudes(krotov_handle h, const double *pulses) {
             a[(size_t)l * N_T + n] = v;
             da[(size_t)l * N_T + n] = dv;
         }
+    }
     int rc;
-    if ((rc = upload(h, h->d_amp_old, a))) return rc;
-    if ((rc = upload(h, h->d_amp_dfac, da))) return rc;
+    if ((rc = upload_async(h, h->d_amp_old, a))) return rc;
+    if ((rc = upload_async(h, h->d_amp_dfac, da))) return rc;
     return KROTOV_OK;
 }
 
@@ -1568,6 +1598,8 @@ int krotov_group_iterate(krotov_handle *hs, int world, const double *guess_pulse
     return KROTOV_OK;
 }
 
+static int amp_commit(krotov_handle h);
+
 int krotov_set_amplitudes(krotov_handle h, int degree, const double *poly, const double *shape) {
     if (!h) return KROTOV_ERR_ARG;
     if (poly && (degree < 1 || degree > kr::kAmpMaxDeg))
@@ -1586,10 +1618,44 @@ int krotov_set_amplitudes(krotov_handle h, int degree, const double *poly, const
             }
     }
     if (shape) h->amp_shape.assign(shape, shape + (size_t)L * N_T);
-    h->amp_set = poly != nullptr || shape != nullptr;
     int rc;
-    if (!h->amp_poly.empty() && (rc = upload(h, h->d_amp_poly, h->amp_poly))) return rc;
-    if (!h->amp_shape.empty() && (rc = upload(h, h->d_amp_shape, h->amp_shape))) return rc;
+    if (!h->amp_poly.empty() && (rc = upload_async(h, h->d_amp_poly, h->amp_poly))) return rc;
+    if (!h->amp_shape.empty() && (rc = upload_async(h, h->d_amp_shape, h->amp_shape))) return rc;
+    return amp_commit(h);
+}
+
+int krotov_set_amplitude_saturation(krotov_handle h, const double *s) {
+    if (!h) return KROTOV_ERR_ARG;
+    cudaSetDevice(h->device);
+    const int L = h->L;
+    if (s)
+        for (int l = 0; l < L; ++l)
+            if (!std::isfinite(s[l]) || s[l] < 0.0)
+                return fail(h, KROTOV_ERR_ARG, "amplitude saturation s[l] must be finite and >= 0");
+    h->amp_sat.clear();
+    if (s && std::any_of(s, s + L, [](double v) { return v > 0.0; })) h->amp_sat.assign(s, s + L);
+    int rc;
+    if (!h->amp_sat.empty() && (rc = upload_async(h, h->d_amp_sat, h->amp_sat))) return rc;
+    return amp_commit(h);
+}
+
+// after either amplitude entry point: the non-linear flag, the per-sweep tables and the block paths' view of them
+static int amp_commit(krotov_handle h) {
+    const int L = h->L, N_T = h->N_T;
+    h->amp_set = !h->amp_poly.empty() || !h->amp_shape.empty() || !h->amp_sat.empty();
+    int rc;
+    // the warp kernels' table: one row per control, the polynomial (identity where only saturation is set) then s_l
+    h->amp_rows.clear();
+    if (!h->amp_poly.empty() || !h->amp_sat.empty()) {
+        const int D = kr::kAmpMaxDeg, R = kr::kAmpRow;
+        h->amp_rows.assign((size_t)L * R, 0.0);
+        for (int l = 0; l < L; ++l) {
+            for (int p = 0; p <= D; ++p)
+                h->amp_rows[(size_t)l * R + p] = h->amp_poly.empty() ? (p == 1 ? 1.0 : 0.0) : h->amp_poly[(size_t)l * (D + 1) + p];
+            h->amp_rows[(size_t)l * R + D + 1] = h->amp_sat.empty() ? 0.0 : h->amp_sat[l];
+        }
+        if ((rc = upload_async(h, h->d_amp_rows, h->amp_rows))) return rc;
+    }
     if (h->amp_set) {
         if ((rc = dev_alloc(h, h->d_amp_old, (size_t)L * N_T * 8))) return rc;
         if ((rc = dev_alloc(h, h->d_amp_dfac, (size_t)L * N_T * 8))) return rc;
@@ -1602,6 +1668,7 @@ int krotov_set_amplitudes(krotov_handle h, int degree, const double *poly, const
             a.dfac = h->d_amp_dfac.get<const double>();
             a.poly = h->amp_poly.empty() ? nullptr : h->d_amp_poly.get<const double>();
             a.shape = h->amp_shape.empty() ? nullptr : h->d_amp_shape.get<const double>();
+            a.sat = h->amp_sat.empty() ? nullptr : h->d_amp_sat.get<const double>();
             a.amp_new = h->d_amp_new.get<double>();
         }
         kr::dense_set_amp(h->dense, a);

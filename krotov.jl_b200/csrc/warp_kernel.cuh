@@ -40,6 +40,7 @@ namespace kr {
 constexpr int kMaxRanks = 8;
 constexpr int kMaxCtrl = 8;
 constexpr int kAmpMaxDeg = 4;
+constexpr int kAmpRow = kAmpMaxDeg + 2;  // a row of WarpParams::amp_poly: kAmpMaxDeg+1 coefficients, then s_l
 constexpr unsigned long long kSentinel = 0xFFFFFFFFFFFFFFFFull;
 
 struct WarpParams {
@@ -69,7 +70,7 @@ struct WarpParams {
     // the forward step gets a(eps_new) from the comm warp.  All null / aliased for linear controls.
     const double *amp_old;     // [L][N_T]
     const double *amp_dfac;    // [L][N_T] or nullptr
-    const double *amp_poly;    // [L][kAmpMaxDeg+1] or nullptr
+    const double *amp_poly;    // [L][kAmpRow] (coefficients, then s_l: see amp_eval_cold) or nullptr
     const double *amp_shape;   // [L][N_T] or nullptr
     double *g_a_int;           // [L]
     double2 *X;                // [N][N_T+1][32]  chi trajectory, trajectory-major
@@ -803,14 +804,18 @@ static __device__ __noinline__ void exchange_gather(const WarpParams *pp, const 
     for (int l = 0; l < kMaxCtrl; ++l) tot_io[l] = tot[l];
 }
 
-// a_l(e, n) = shape * sum_p poly[l][p] e^p  (non-linear amplitudes only; kept out of the comm warp's loop body)
+// a_l(e, n) = shape * sum_p poly[l][p] x^p, x = tanh(s_l e) where s_l > 0 (saturating amplitudes), else x = e
+// (non-linear amplitudes only; kept out of the comm warp's loop body).  s_l travels in the polynomial's row rather than
+// in a parameter field of its own: the function reads the same two fields as without saturation, and the comm warp's
+// loop around its call site compiles to the same code.
 static __device__ __noinline__ double amp_eval_cold(const WarpParams *pp, const int l, const double e, const double shp) {
     double c = e;
     if (pp->amp_poly != nullptr) {
-        const double *q = pp->amp_poly + l * (kAmpMaxDeg + 1);
+        const double *q = pp->amp_poly + l * kAmpRow;
+        const double x = q[kAmpMaxDeg + 1] != 0.0 ? tanh(q[kAmpMaxDeg + 1] * e) : e;
         c = q[kAmpMaxDeg];
 #pragma unroll
-        for (int d = kAmpMaxDeg - 1; d >= 0; --d) c = fma(c, e, q[d]);
+        for (int d = kAmpMaxDeg - 1; d >= 0; --d) c = fma(c, x, q[d]);
     }
     if (pp->amp_shape != nullptr) c = __dmul_rn(shp, c);
     return c;

@@ -144,6 +144,13 @@ class KrotovCuda:
             shape = np.ascontiguousarray(shape, np.float64).reshape(self.L, self.N_T)
         self._check(self._lib.krotov_set_amplitudes(self._h, int(deg), _ptr(poly), _ptr(shape)))
 
+    def set_amplitude_saturation(self, s=None):
+        """Saturating amplitudes (``krotov_set_amplitude_saturation``): ``s``: (L,) or None.  Where ``s[l] > 0`` the
+        amplitude polynomial of control l is evaluated at ``tanh(s[l] * eps)``; None restores s = 0 everywhere."""
+        if s is not None:
+            s = np.ascontiguousarray(s, np.float64).reshape(self.L)
+        self._check(self._lib.krotov_set_amplitude_saturation(self._h, _ptr(s)))
+
     # -- hot path -------------------------------------------------------------------------
     def forward(self, pulses):
         p = np.ascontiguousarray(pulses, np.float64).reshape(self.L, self.N_T)
@@ -256,6 +263,10 @@ class KrotovCudaGroup:
     def set_amplitudes(self, poly=None, shape=None):
         for e in self.engines:
             e.set_amplitudes(poly, shape)
+
+    def set_amplitude_saturation(self, s=None):
+        for e in self.engines:
+            e.set_amplitude_saturation(s)
 
     def forward(self, pulses):
         for e in self.engines:  # no cross-rank dependency in a plain forward sweep

@@ -30,7 +30,26 @@ from .second_order import sigma_value
 
 log = logging.getLogger("krotov_jl_b200")
 
-__all__ = ["KrotovWrk", "IdDict"]
+__all__ = ["KrotovWrk", "IdDict", "saturated_corners"]
+
+
+def saturated_corners(poly, s, lo, hi, shape_max=None):
+    """Range of ``shape_max * P(tanh(s eps))`` over eps in [lo, hi] for a polynomial P of degree <= 2 (ascending
+    ``poly``): ``(P(x_lo), P(x_hi))`` when P is monotone on [x_lo, x_hi], else ``(min, max)`` including the vertex."""
+    c = [float(v) for v in poly] + [0.0] * 3
+    if any(v != 0.0 for v in c[3:]):
+        raise ArgumentError("a saturating amplitude takes a polynomial of degree <= 2")
+    P = lambda x: (c[2] * x + c[1]) * x + c[0]  # noqa: E731
+    x_lo, x_hi = float(np.tanh(s * lo)), float(np.tanh(s * hi))
+    v_lo, v_hi = P(x_lo), P(x_hi)
+    if c[2] != 0.0:
+        x_v = -c[1] / (2.0 * c[2])
+        if x_lo < x_v < x_hi:
+            vals = (v_lo, v_hi, P(x_v))
+            v_lo, v_hi = min(vals), max(vals)
+    if shape_max is not None:
+        v_lo, v_hi = shape_max * v_lo, shape_max * v_hi
+    return v_lo, v_hi
 
 
 class IdDict:
@@ -208,7 +227,7 @@ class KrotovWrk:
             raise ErrorException("no controls in trajectories: cannot optimize")
         self.control_derivs = [get_control_derivs(t.generator, self.controls) for t in self.trajectories]
         tlist = np.asarray(problem.tlist, np.float64)
-        self._amp_poly, self._amp_shape = self._collect_amplitudes(tlist)
+        self._amp_poly, self._amp_shape, self._amp_sat = self._collect_amplitudes(tlist)
         kwargs = dict(kwargs_in)  # shallow copy; ok to modify
         default_shape = kwargs_in.get("update_shape", lambda t: 1.0)
         default_lambda = float(kwargs_in.get("lambda_a", 1.0))
@@ -306,9 +325,10 @@ class KrotovWrk:
 
     # -------------------------------------------------------------------------------------
     def _collect_amplitudes(self, tlist):
-        """Non-linear / shaped amplitudes (``src/optimize.jl:268-272``): per control the polynomial and the per-interval
-        shape through which it enters the generators -- the same for every generator that depends on the control (the
-        batched device propagator evaluates one amplitude per control).  ``(None, None)`` for linear controls."""
+        """Non-linear / shaped amplitudes (``src/optimize.jl:268-272``): per control the polynomial, the per-interval
+        shape and the saturation ``s`` (a parametrization's ``tanh(s u)``, 0 = none) through which it enters the
+        generators -- the same for every generator that depends on the control (the batched device propagator evaluates
+        one amplitude per control).  ``(None, None, None)`` for linear controls."""
         L = len(self.controls)
         chosen = [None] * L
         seen = set()
@@ -322,14 +342,14 @@ class KrotovWrk:
                 if derivs[l] is None:
                     continue
                 a = amps[l]
-                key = None if a is None else (tuple(a.coeffs), id(a.shape) if a.shape is not None else None)
+                key = None if a is None else (a.key(), id(a.shape) if a.shape is not None else None)
                 if chosen[l] is None:
                     chosen[l] = (key, a)
                 elif chosen[l][0] != key:
                     raise ArgumentError("a control must enter all generators through the same amplitude")
         amps = [c[1] if c is not None else None for c in chosen]
         if all(a is None for a in amps):
-            return None, None
+            return None, None, None
         deg = max(len(a.coeffs) - 1 for a in amps if a is not None)
         poly = np.zeros((L, deg + 1))
         shape = None
@@ -344,7 +364,8 @@ class KrotovWrk:
                 shape[l] = discretize_on_midpoints(a.shape, tlist)
         if all(np.array_equal(poly[l], np.eye(deg + 1)[1]) for l in range(L)):
             poly = None  # only shapes: a(eps, n) = shape[n] * eps
-        return poly, shape
+        sat = np.array([0.0 if a is None else a.saturation for a in amps])
+        return poly, shape, (sat if np.any(sat > 0) else None)
 
     def _amp_envelope(self, l, eps):
         """Coefficient of H_l at a corner ``eps`` of the control range, for the spectral envelope: the polynomial at
@@ -357,6 +378,18 @@ class KrotovWrk:
         if self._amp_shape is not None:
             v = float(np.max(np.abs(self._amp_shape[l]))) * v
         return v
+
+    def _amp_envelope_corners(self, l, lo, hi):
+        """Coefficients of H_l for the spectral envelope over the control range [lo, hi]: ``(value at the lo side,
+        value at the hi side)``.  A saturating control (s_l > 0) takes the range of its polynomial P (degree <= 2) over
+        [tanh(s lo), tanh(s hi)] -- the end values, plus P at its vertex when the vertex lies inside, in which case the
+        pair is (min, max): tanh**2 over a range that straddles 0 must include the amplitude 0.  Every other control keeps
+        the corners of ``_amp_envelope``."""
+        s = 0.0 if self._amp_sat is None else float(self._amp_sat[l])
+        if s == 0.0:
+            return self._amp_envelope(l, lo), self._amp_envelope(l, hi)
+        return saturated_corners(self._amp_poly[l] if self._amp_poly is not None else [0.0, 1.0], s, lo, hi,
+                                 None if self._amp_shape is None else float(np.max(np.abs(self._amp_shape[l]))))
 
     def _build_device_side(self, tlist, comm):
         trajs = self.trajectories
@@ -447,9 +480,11 @@ class KrotovWrk:
             self._Hc = [Hc[g] for g in local_gens]
         if comm is not None and world > 1:
             comm.connect(self.engine)
-        nonlinear = self._amp_poly is not None or self._amp_shape is not None
+        nonlinear = self._amp_poly is not None or self._amp_shape is not None or self._amp_sat is not None
         if nonlinear:
             self.engine.set_amplitudes(self._amp_poly, self._amp_shape)
+        if self._amp_sat is not None:
+            self.engine.set_amplitude_saturation(self._amp_sat)
         # ---- Chebyshev settings of both directions (init_prop: un-widened ranges of the guess pulses)
         adj = lambda m: m.conj().T.tocsr() if hasattr(m, "tocsr") else m.conj().T  # noqa: E731
         same = lambda a, b: (abs(a - b).max() == 0) if hasattr(a, "tocsr") else np.array_equal(a, b)  # noqa: E731
@@ -476,7 +511,7 @@ class KrotovWrk:
                 limit=pk.get("cheby_coeffs_limit", 1e-12), specrange_buffer=pk.get("specrange_buffer", 0.01),
                 specrange_method=pk.get("specrange_method", "auto"), E_min=pk.get("E_min"), E_max=pk.get("E_max"),
                 envelope_cache=shared if self._shared_envelope_ok(pk) else None,
-                amplitude=self._amp_envelope if nonlinear else None, device_envelope=device_envelope)
+                amplitude=self._amp_envelope_corners if nonlinear else None, device_envelope=device_envelope)
 
         self.fw_settings = settings(self.fw_prop_kwargs[0], False)
         self.bw_settings = settings(self.bw_prop_kwargs[0], True)
