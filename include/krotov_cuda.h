@@ -66,6 +66,18 @@ enum krotov_path { /* which kernel family serves the handle (krotov_info.path) *
     KROTOV_PATH_SPARSE = 3 /* larger d, sparse generators: ELL SpMM over the state block per Chebyshev term      */
 };
 
+enum krotov_kernel { /* which kernel served the last forward/iterate call (krotov_info.kernel); 0 before the first */
+    KROTOV_KERNEL_TINY = 1,          /* WARP: d <= 4, one thread per trajectory, everything in registers        */
+    KROTOV_KERNEL_PREG = 2,          /* WARP: one trajectory per thread group, term rows held in registers      */
+    KROTOV_KERNEL_SEQ_PREG = 3,      /* WARP: several trajectories of one generator per warp, one after another */
+    KROTOV_KERNEL_PAIR = 4,          /* WARP: two trajectories of one generator per warp, interleaved           */
+    KROTOV_KERNEL_RELOAD = 5,        /* WARP: term rows re-read from memory for every use                       */
+    KROTOV_KERNEL_DMMA_STREAM = 6,   /* DENSE: one DMMA GEMM launch per Chebyshev term                          */
+    KROTOV_KERNEL_DENSE_SWEEP = 7,   /* DENSE: persistent cluster sweep                                         */
+    KROTOV_KERNEL_SPARSE_SWEEP = 8,  /* SPARSE: persistent sweep                                                */
+    KROTOV_KERNEL_SPARSE_STREAM = 9  /* SPARSE: one ELL SpMM launch per Chebyshev term                          */
+};
+
 /*
  * The control problem, reduced to arrays.  Replaces what KrotovWrk's constructor collects
  * (src/workspace.jl:65-131): trajectories (initial/target state, generator), tlist, update
@@ -130,7 +142,10 @@ typedef struct {
     int64_t graph_replays;   /* block paths: iterations served by replaying the captured CUDA graph since creation */
     double ms_rank_wait;     /* replicated forward sweep: time CTA 0 of this rank spent at the rank barrier behind the backward
                                 sweep in the last krotov_iterate (launch skew between the ranks + the slowest backward shard) */
-    int64_t reserved[3];
+    int32_t kernel;          /* enum krotov_kernel of the last forward/iterate call, 0 before the first */
+    int32_t lanes_per_traj;  /* WARP path: threads per trajectory of that kernel (32, 64 or 128; 1 for the tiny kernel);
+                                0 on the block paths */
+    int64_t reserved[2];
 } krotov_info;
 
 /* ---- lifetime ------------------------------------------------------------------------ */

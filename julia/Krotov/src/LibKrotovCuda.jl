@@ -11,6 +11,8 @@ const KROTOV_GEN_DENSE_COLMAJOR, KROTOV_GEN_CSR = Cint(0), Cint(1)
 const KROTOV_FORWARD, KROTOV_BACKWARD = Cint(0), Cint(1)
 const KROTOV_CHI_HOST, KROTOV_CHI_SM, KROTOV_CHI_SS, KROTOV_CHI_RE = Cint(0), Cint(1), Cint(2), Cint(3)
 const KROTOV_PATH_WARP, KROTOV_PATH_DENSE, KROTOV_PATH_SPARSE = Cint(1), Cint(2), Cint(3)
+const KROTOV_KERNEL_TINY, KROTOV_KERNEL_PREG, KROTOV_KERNEL_SEQ_PREG, KROTOV_KERNEL_PAIR, KROTOV_KERNEL_RELOAD = Cint(1), Cint(2), Cint(3), Cint(4), Cint(5)
+const KROTOV_KERNEL_DMMA_STREAM, KROTOV_KERNEL_DENSE_SWEEP, KROTOV_KERNEL_SPARSE_SWEEP, KROTOV_KERNEL_SPARSE_STREAM = Cint(6), Cint(7), Cint(8), Cint(9)
 const COMM_DESC_BYTES = 256
 
 # mirrors `krotov_problem` field by field
@@ -63,7 +65,9 @@ struct Info
     fallback_steps::Int64
     graph_replays::Int64
     ms_rank_wait::Float64
-    reserved::NTuple{3,Int64}
+    kernel::Int32
+    lanes_per_traj::Int32
+    reserved::NTuple{2,Int64}
 end
 
 mutable struct Handle

@@ -19,6 +19,9 @@ GEN_DENSE_COLMAJOR, GEN_CSR = 0, 1
 FORWARD, BACKWARD = 0, 1
 CHI_HOST, CHI_SM, CHI_SS, CHI_RE = 0, 1, 2, 3
 PATH_WARP, PATH_DENSE, PATH_SPARSE = 1, 2, 3
+# enum krotov_kernel (Info.kernel)
+(KERNEL_TINY, KERNEL_PREG, KERNEL_SEQ_PREG, KERNEL_PAIR, KERNEL_RELOAD, KERNEL_DMMA_STREAM, KERNEL_DENSE_SWEEP,
+ KERNEL_SPARSE_SWEEP, KERNEL_SPARSE_STREAM) = range(1, 10)
 COMM_DESC_BYTES = 256
 
 # every symbol include/krotov_cuda.h declares that returns a status code or a string (tests check the .so exports all
@@ -58,7 +61,8 @@ class Info(C.Structure):
         ("sm_count", C.c_int32), ("exchange", C.c_int32),
         ("launches_total", C.c_int64), ("launches_last", C.c_int64), ("ms_last", C.c_double),
         ("ms_last_backward", C.c_double), ("hbm_bytes_state", C.c_int64), ("fallback_steps", C.c_int64),
-        ("graph_replays", C.c_int64), ("ms_rank_wait", C.c_double), ("reserved", C.c_int64 * 3),
+        ("graph_replays", C.c_int64), ("ms_rank_wait", C.c_double), ("kernel", C.c_int32), ("lanes_per_traj", C.c_int32),
+        ("reserved", C.c_int64 * 2),
     ]
 
 

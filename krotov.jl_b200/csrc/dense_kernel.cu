@@ -1035,6 +1035,7 @@ struct DenseEngine {
     DevBuf sw_partial, sw_coef[2], sw_Emin[2], sw_Delta[2];  // double
     DevBuf sw_phase[2];                                      // double2
     long long sweep_launches = 0;
+    int kernel_last = 0;  // enum krotov_kernel of the last forward/iterate call
     // persistent cluster sweep for moderate dense generators (dense_sweep.cuh)
     bool dsweep = false;
     int ds_units = 0, ds_R = 0, ds_gpad = 0;
@@ -1290,6 +1291,11 @@ bool sweep_usable(const DenseEngine *e, int mode) {
     // KROTOV_NO_SWEEP_RANKS=1 keeps the launch-per-term stream there)
     if (e->comm.world > 1 && getenv("KROTOV_NO_SWEEP_RANKS")) return false;
     return (e->sweep || e->dsweep) && e->ch[0].set && (mode == 0 || e->ch[1].set) && !getenv("KROTOV_NO_SWEEP");
+}
+
+int kernel_kind(const DenseEngine *e, int mode) {
+    if (sweep_usable(e, mode)) return e->dsweep ? KROTOV_KERNEL_DENSE_SWEEP : KROTOV_KERNEL_SPARSE_SWEEP;
+    return e->sparse ? KROTOV_KERNEL_SPARSE_STREAM : KROTOV_KERNEL_DMMA_STREAM;
 }
 
 template <typename T>
@@ -1580,6 +1586,8 @@ void dense_info(DenseEngine *e, krotov_info *out) {
         out->grid_blocks = e->ds_units * kDsCluster;
         out->block_threads = kDsThreads;
     }
+    out->kernel = e->kernel_last;
+    out->lanes_per_traj = 0;
     out->nnz_union = e->sparse ? e->nnz_union : e->d * e->d;
     out->ell_width = e->sparse ? e->W : 0;
     out->hbm_bytes_state = (int64_t)(e->slab * (size_t)(e->N_T + 1) * 16);
@@ -1633,6 +1641,7 @@ bool dense_seed(DenseEngine *e, double2 *d_tau, std::string &err) {
 
 bool dense_forward(DenseEngine *e, const double *d_eps, double2 *d_tau, long long &launches, std::string &err) {
     e->launches = 0;
+    e->kernel_last = kernel_kind(e, 0);
     DK_CHECK(cudaMemcpyAsync(e->PSI.get<double2>(), e->PSI0.get<double2>(), e->slab * 16, cudaMemcpyDeviceToDevice, e->stream));
     if (sweep_usable(e, 0)) {
         if (!launch_sweep(e, 0, d_eps, nullptr, nullptr, nullptr, nullptr, err) || !finish_sweep(e, d_tau, err)) return false;
@@ -1670,6 +1679,7 @@ bool dense_iterate(DenseEngine *e, const double *d_eps_old, double *d_eps_new, c
                    std::string &err) {
     DenseEngine::GraphKey key;
     key.cheb_version = e->cheb_version;
+    e->kernel_last = kernel_kind(e, 1);
     const void *ptrs[8] = {d_eps_old, d_eps_new, d_alpha, d_dt, d_ga, d_chi_coef, d_tau, e->amp.amp_old};
     memcpy(key.ptr, ptrs, sizeof(ptrs));
     const bool graph_ok = e->comm.world <= 1 && !getenv("KROTOV_NO_GRAPH") && !sweep_usable(e, 1);  // (the sweep is 3 launches)

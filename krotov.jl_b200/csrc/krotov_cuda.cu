@@ -130,6 +130,7 @@ struct krotov_handle_s : HandleStream {
     double2 *peer_Xbase[kr::kMaxRanks] = {};      // chi trajectories of every rank (parity p at + p * x_slab)
     unsigned long long *peer_flag[kr::kMaxRanks] = {};
     int xchg_last = 0;   // cross-rank protocol of the last launch: 0 none, 1 hier, 2 onehop, 3 mailboxes
+    int kernel_last = 0, lanes_last = 0;  // enum krotov_kernel and threads per trajectory of the last warp-path launch
     // non-linear control amplitudes (krotov_set_amplitudes, krotov_set_amplitude_saturation)
     bool amp_set = false;           // poly, shape or saturation present
     std::vector<double> amp_poly;   // [L][kAmpMaxDeg+1], ascending powers (empty = a(eps) = eps)
@@ -761,6 +762,13 @@ void fill_warp_params(krotov_handle h, int mode, kr::WarpParams &p) {
     if (const char *e = getenv("KROTOV_TIMEOUT_CYCLES")) p.timeout_cycles = atoll(e);
 }
 
+// enum krotov_kernel of the persistent warp kernel choose_launch selected (the tiny kernel aside)
+int warp_kernel_kind(const krotov_handle h) {
+    if (h->pair) return KROTOV_KERNEL_PAIR;
+    if (h->preg) return h->tpw > 1 ? KROTOV_KERNEL_SEQ_PREG : KROTOV_KERNEL_PREG;
+    return KROTOV_KERNEL_RELOAD;
+}
+
 int launch_warp(krotov_handle h, int mode) {
     kr::WarpParams p;
     fill_warp_params(h, mode, p);
@@ -779,6 +787,8 @@ int launch_warp(krotov_handle h, int mode) {
         void *args[] = {(void *)&tp};
         KR_CUDA(h, cudaLaunchKernel((const void *)fn, dim3(1), dim3(32), args, smem, h->stream));
         h->launches_last += 1;
+        h->kernel_last = KROTOV_KERNEL_TINY;
+        h->lanes_last = 1;
         return KROTOV_OK;
     }
     KernelKey key{h->Wt, h->preg ? h->L : 0, h->pair ? 32 : h->lpt};
@@ -808,6 +818,8 @@ int launch_warp(krotov_handle h, int mode) {
         KR_CUDA(h, cudaLaunchKernel((const void *)fn, grid, block, args, smem, h->stream));
     }
     h->launches_last += 1;
+    h->kernel_last = warp_kernel_kind(h);
+    h->lanes_last = h->lpt;
     return KROTOV_OK;
 }
 
@@ -1161,6 +1173,8 @@ int krotov_get_info(krotov_handle h, krotov_info *out) {
     out->hbm_bytes_state = (int64_t)h->d_X.bytes();
     out->fallback_steps = h->fallback_steps;
     out->ms_rank_wait = h->ms_rank_wait;
+    out->kernel = h->kernel_last;
+    out->lanes_per_traj = h->lanes_last;
     if (h->dense) kr::dense_info(h->dense, out);
     return KROTOV_OK;
 }
@@ -1593,6 +1607,10 @@ int krotov_group_iterate(krotov_handle *hs, int world, const double *guess_pulse
     KR_CUDA(h0, cudaLaunchCooperativeKernel((const void *)it->second, grid, block, args, smem, h0->stream));
     KR_CUDA(h0, cudaStreamSynchronize(h0->stream));
     h0->launches_last += 1;
+    for (int r = 0; r < world; ++r) {
+        hs[r]->kernel_last = warp_kernel_kind(hs[r]);
+        hs[r]->lanes_last = hs[r]->lpt;
+    }
     for (int r = 0; r < world; ++r)
         if ((rc = iterate_finish(hs[r], new_pulses + (size_t)r * pn, g_a_int + (size_t)r * h0->L))) return rc;
     return KROTOV_OK;

@@ -1,0 +1,451 @@
+"""Every kernel family against the EXACT dynamics, on the features where kernels go wrong.
+
+The other GPU tests compare a kernel with the NumPy or C Chebyshev oracle, which shares the kernel's Chebyshev inputs
+(Bessel coefficients, dt classes, spectral window, phase): an error in those shared inputs passes them.  Here every cell
+also meets the oracle run with the exact propagator of every interval (``prop_method="expm"``), which uses none of
+them.  The problems combine, in few runs:
+
+- grids with several dt classes (three segments where dt returns to an earlier value and a last step that differs), a
+  jittered grid where every step has its own dt (a large coefficient table), N_T = 1 and 2;
+- ensembles of generators whose spectral radii are ~1.35x apart (different term counts), their trajectories sharing a
+  CTA or column block, one generator without a control term, trajectory weights, the three functionals;
+- variant A: linear controls and a weakly non-Hermitian generator; variant B: Hermitian, a polynomial amplitude times a
+  shape on one control and a TanhParametrization on another.
+
+Each cell selects its kernel with the knobs the library reads and asserts, through ``info()``, which kernel served it.
+The exact bound of every problem (BOUND) is 10x the CPU Chebyshev-oracle-vs-exact gap rounded up to a power of ten; the
+CPU tests at the bottom check that the oracle meets BOUND / 10, so a GPU miss is the kernel's."""
+import functools
+
+import numpy as np
+import pytest
+from scipy.linalg import expm
+
+import krotov_jl_b200 as K
+import sat_reference as S
+import workloads as W
+from krotov_jl_b200 import _lib as B
+from oracle import krotov_oracle as O
+
+RTOL_JT, ATOL_JT, ATOL_PULSE = 1e-10, 2e-15, 1e-9  # BASELINE.json
+_JT = {"sm": K.J_T_sm, "ss": K.J_T_ss, "re": K.J_T_re}
+
+
+# ---- problems ----------------------------------------------------------------------------------------------------------
+def _segments(T, n):
+    """~n steps in three segments, dt -> 1.25 dt -> dt, and a last step of 0.6 dt."""
+    k = n // 3
+    steps = [1.0] * k + [1.25] * k + [1.0] * (n - 2 * k - 1) + [0.6]
+    t = np.concatenate([[0.0], np.cumsum(steps)])
+    return t * (T / t[-1])
+
+
+def _jittered(T, n, seed):
+    """n steps, every one its own dt: dt_n = dt (1 + 1e-3 u_n)."""
+    u = np.random.default_rng(seed).uniform(-1.0, 1.0, n)
+    t = np.concatenate([[0.0], np.cumsum(1.0 + 1e-3 * u)])
+    return t * (T / t[-1])
+
+
+def _ensemble(w, n_gen, gen_of_traj, drop_term=True):
+    """n_gen generators, spectral radii 1.35x apart; the last one does not depend on the last control."""
+    H0, Hc = w.H0[0], w.Hc[0]
+    w.H0 = [H0 * 1.35**g for g in range(n_gen)]
+    w.Hc = [list(Hc) for _ in range(n_gen)]
+    if drop_term and len(Hc) > 1 and n_gen > 1:
+        w.Hc[-1][-1] = None
+    w.gen_of_traj = np.asarray(gen_of_traj, int)
+    return w
+
+
+def _non_hermitian(w, seed):
+    """Variant A: weak decay on every drift, a non-Hermitian admixture to the first control (as the seeded sweep), kept
+    to that control's sparsity pattern so that the rows stay as narrow as the kernel family needs."""
+    rng = np.random.default_rng(seed)
+    d = w.d
+    decay = -0.02j * np.diag(rng.uniform(0, 1, d))
+    Bm = (rng.standard_normal((d, d)) + 1j * rng.standard_normal((d, d))) / np.sqrt(d)
+    w.H0 = [h + decay for h in w.H0]
+    w.Hc = [[row[0] + 0.05 * Bm * (row[0] != 0)] + list(row[1:]) for row in w.Hc]
+    return w
+
+
+def _amplitudes(w):
+    """Variant B: control 0 as shape(t) * (eps + 0.8 eps^2 - 0.3 eps^3), control 1 through TanhParametrization."""
+    T = float(w.tlist[-1])
+    L = len(w.controls)
+    w.amp_poly = [[0.0, 1.0, 0.8, -0.3]] + [None] * (L - 1)
+    w.amp_shape = [lambda t: 0.6 + 0.4 * W.flattop(t, T=T, t_rise=0.3 * T)] + [None] * (L - 1)
+    amax = max(abs(W.midpoint_samples(w.controls[1], w.tlist)).max(), 0.05) if L > 1 else 0.0
+    params = [None] * L
+    if L > 1:
+        params[1] = K.TanhParametrization(-1.5 * amax, 1.5 * amax)
+    return w, params
+
+
+class Case:
+    def __init__(self, w, params=None, weight=None):
+        self.w, self.weight = w, weight
+        self.params = params if params is not None else [None] * len(w.controls)
+
+    def oracle(self):
+        p = S.oracle_problem(self.w, self.params)
+        if self.weight is not None:
+            p.weight = np.asarray(self.weight, float)
+        return p
+
+    def problem(self, **kw):
+        """The same problem through the public API (Generator objects shared by the trajectories of one generator)."""
+        w = self.w
+        amps = []
+        for l, c in enumerate(w.controls):
+            poly = None if w.amp_poly is None else w.amp_poly[l]
+            shape = None if w.amp_shape is None else w.amp_shape[l]
+            if self.params[l] is not None:
+                amps.append(K.ParametrizedAmplitude(c, self.params[l], shape))
+            elif poly is not None:
+                amps.append(K.PolynomialAmplitude(c, poly, shape))
+            elif shape is not None:
+                amps.append(K.ShapedAmplitude(c, shape))
+            else:
+                amps.append(c)
+        gens = [K.hamiltonian(w.H0[g], *[(w.Hc[g][l], amps[l]) for l in range(w.L) if w.Hc[g][l] is not None])
+                for g in range(len(w.H0))]
+        trajs = [K.Trajectory(w.psi0[k], gens[int(w.gen_of_traj[k])], target_state=w.target[k]) for k in range(w.N)]
+        if self.weight is not None:
+            for t, x in zip(trajs, self.weight):
+                t.weight = float(x)
+        args = dict(prop_method=K.Cheby, J_T=_JT[w.functional], lambda_a=w.lambda_a, update_shape=w.update_shape,
+                    print_iters=False)
+        if w.specrange is not None:
+            args.update(prop_E_min=w.specrange[0], prop_E_max=w.specrange[1])
+        args.update(kw)
+        return K.ControlProblem(trajs, w.tlist, **args)
+
+
+def _dummy(d, n_traj, L, n_grid, seed, functional, tlist=None, flat_shape=False):
+    w = W.dummy_dense(d=d, n_traj=n_traj, n_controls=L, n_grid=n_grid, seed=seed, functional=functional)
+    if tlist is not None:
+        w.tlist = tlist
+    if flat_shape:  # (the flattop update shape vanishes on the ends of very short grids)
+        w.update_shape = lambda t: 1.0
+    return w
+
+
+def _weights(n, seed):
+    return np.random.default_rng(seed).uniform(0.4, 1.6, n)
+
+
+def _warp(L, variant, functional):
+    """d = 7 (six off-diagonal slots: register-row, pair and reloaded-row instances exist for L = 1, 2, 3), three
+    generators over 6 trajectories in one CTA."""
+    w = _ensemble(_dummy(7, 6, L, 0, 40 + L, functional, tlist=_segments(5.0, 36)), 3, [0, 1, 2, 2, 0, 1])
+    if variant == "A":
+        return Case(_non_hermitian(w, 50 + L), weight=_weights(6, L))
+    w, params = _amplitudes(w)
+    return Case(w, params, weight=_weights(6, L))
+
+
+def _pair(variant):
+    """Generator-sharing pairs: trajectories 2j, 2j+1 share a generator, three generators."""
+    w = _ensemble(_dummy(7, 8, 2, 0, 61, "sm", tlist=_segments(5.0, 30)), 3, [0, 0, 1, 1, 2, 2, 0, 0])
+    if variant == "A":
+        return Case(_non_hermitian(w, 62), weight=_weights(8, 3))
+    w, params = _amplitudes(w)
+    return Case(w, params, weight=_weights(8, 3))
+
+
+def _c4(n_samples, levels, n_grid, T):
+    w = W.c4_ensemble(n_samples=n_samples, n_grid=n_grid, levels=levels, T=T)
+    w.tlist = _segments(T, n_grid - 1)
+    a = 0.6 * abs(W.midpoint_samples(w.controls[0], w.tlist)).max()
+    w.controls = [w.controls[0], lambda t, a=a: a * W.flattop(t, T=T, t_rise=0.2 * T)]  # (C4's second guess is 0)
+    return w
+
+
+def _sparse(variant):
+    w = W.spin_chain(n_spins=6, n_traj=8, n_grid=2, functional="ss")
+    w.tlist = _segments(4.0, 24)
+    w = _ensemble(w, 2, [0, 1, 0, 1, 1, 0, 0, 1], drop_term=False)
+    if variant == "A":
+        w.H0 = [h - 0.02j * np.diag(np.linspace(0, 1, w.d)) for h in w.H0]  # decay: non-Hermitian
+        return Case(w, weight=_weights(8, 9))
+    w, params = _amplitudes(w)
+    return Case(w, params, weight=_weights(8, 9))
+
+
+PROBLEMS = {
+    # tiny kernel: d <= 4, N <= 32, L <= 2; a jittered grid of 40 own dt (the coefficient table leaves shared memory)
+    "tiny_jitter": lambda: Case(_non_hermitian(_ensemble(_dummy(4, 6, 2, 0, 11, "sm", tlist=_jittered(5.0, 40, 1)), 2,
+                                                         [0, 1, 1, 0, 1, 0]), 12), weight=_weights(6, 1)),
+    "tiny_nt2": lambda: Case(_dummy(3, 3, 1, 0, 13, "re", tlist=np.array([0.0, 0.3, 0.45]), flat_shape=True)),
+    "warp_nt1": lambda: Case(_dummy(7, 3, 2, 2, 14, "ss", flat_shape=True), weight=_weights(3, 2)),
+    "warp_L1_A": lambda: _warp(1, "A", "ss"),
+    "warp_L1_B": lambda: _warp(1, "B", "re"),
+    "warp_L2_A": lambda: _warp(2, "A", "re"),
+    "warp_L2_B": lambda: _warp(2, "B", "sm"),
+    "warp_L3_A": lambda: _warp(3, "A", "sm"),
+    "warp_L3_B": lambda: _warp(3, "B", "ss"),
+    "warp_L5_A": lambda: _warp(5, "A", "ss"),
+    "warp_L5_B": lambda: _warp(5, "B", "sm"),
+    "pair_A": lambda: _pair("A"),
+    "pair_B": lambda: _pair("B"),
+    # more than 7 x 148 trajectories in runs of two per generator: sequential register rows
+    "seq_B": lambda: Case(*_amplitudes(_ensemble(_dummy(5, 1040, 2, 0, 71, "ss", tlist=_segments(5.0, 12)), 3,
+                                                 (np.arange(1040) // 2) % 3))),
+    # transmon ensembles: short times, so that the Chebyshev truncation error of the exact comparison stays small
+    "wide64_A": lambda: Case(_non_hermitian(_c4(6, 7, 21, 4.0), 81), weight=_weights(24, 4)),
+    "wide64_B": lambda: Case(*_amplitudes(_c4(6, 7, 21, 4.0)), weight=_weights(24, 4)),
+    "wide128_B": lambda: Case(*_amplitudes(_c4(1, 10, 16, 3.0))),
+    "ranks_B": lambda: Case(*_amplitudes(_c4(8, 5, 21, 4.0)), weight=_weights(32, 5)),
+    "ranks_lin": lambda: Case(_c4(8, 5, 21, 4.0), weight=_weights(32, 5)),
+    "dense_A": lambda: Case(_non_hermitian(_ensemble(_dummy(40, 6, 2, 0, 91, "ss", tlist=_segments(5.0, 20)), 2,
+                                                     [0, 1, 1, 0, 0, 1]), 92), weight=_weights(6, 6)),
+    "dense_B": lambda: Case(*_amplitudes(_ensemble(_dummy(40, 6, 2, 0, 93, "re", tlist=_segments(5.0, 20)), 2,
+                                                   [0, 1, 1, 0, 0, 1])), weight=_weights(6, 7)),
+    "sparse_A": lambda: _sparse("A"),
+    "sparse_B": lambda: _sparse("B"),
+}
+
+
+def _graph_case():
+    w = _ensemble(_dummy(48, 6, 2, 0, 95, "sm", tlist=_segments(5.0, 20)), 2, [0, 1, 0, 1, 1, 0])
+    w.specrange = (-6.0, 6.0)  # a fixed window: the tables never change, so the settled iteration is captured
+    return Case(w, weight=_weights(6, 8))
+
+
+PROBLEMS["graph_A"] = _graph_case
+ITERS = {"graph_A": 5}
+
+# exact bound per problem: 10 x the CPU Chebyshev-oracle-vs-exact gap, rounded up to a power of ten, <= 1e-11
+BOUND = {
+    "tiny_jitter": 1e-12, "tiny_nt2": 1e-13, "warp_nt1": 1e-12, "warp_L1_A": 1e-12, "seq_B": 1e-12, "dense_A": 1e-12,
+    "dense_B": 1e-12, "sparse_B": 1e-12, "graph_A": 1e-12,
+    "warp_L1_B": 1e-11, "warp_L2_A": 1e-11, "warp_L2_B": 1e-11, "warp_L3_A": 1e-11, "warp_L3_B": 1e-11,
+    "warp_L5_A": 1e-11, "warp_L5_B": 1e-11, "pair_A": 1e-11, "pair_B": 1e-11, "wide64_A": 1e-11, "wide64_B": 1e-11,
+    "wide128_B": 1e-11, "ranks_B": 1e-11, "ranks_lin": 1e-11, "sparse_A": 1e-11,
+}
+
+
+@functools.lru_cache(maxsize=None)
+def case(name):
+    return PROBLEMS[name]()
+
+
+# ---- references ------------------------------------------------------------------------------------------------------
+class _SharedExp(O.ExpPropagator):
+    """The exact propagator of one interval, computed once per (generator, direction, interval, amplitudes) and shared
+    by the trajectories of that generator."""
+
+    def __init__(self, *args, cache):
+        super().__init__(*args)
+        self.cache = cache
+
+    def prop_step(self):
+        ni, dt = self._interval_and_dt()
+        ops, cf = self._ops_coeffs(ni)
+        key = tuple(cf)
+        hit = self.cache.get(ni)
+        if hit is None or hit[0] != key:
+            H = sum(c * op for op, c in zip(ops, cf))
+            hit = (key, expm(-1j * dt * (H.toarray() if hasattr(H, "toarray") else H)))
+            self.cache[ni] = hit
+        self.state = hit[1] @ self.state
+        self._advance()
+        return self.state
+
+
+def reference_run(p, iters, prop_method):
+    """The oracle's loop (``optimize_krotov``, first order, saturating amplitudes included) recording J_T, g_a_int and
+    tau of every iteration, the final pulses and states, and every slot of both storages after the last iteration."""
+    wrk = S.SatOracleWrk(p, prop_method=prop_method, store_fw=True)
+    if prop_method == "expm":
+        caches = {}
+        for k in range(p.N):
+            g = int(p.gen_of_traj[k])
+            for q, props in enumerate((wrk.fw_propagators, wrk.bw_propagators)):
+                old = props[k]
+                props[k] = _SharedExp(old.H0, old.Hc, old.tlist, old.parameters, old.backward, p,
+                                      cache=caches.setdefault((g, q), {}))
+    eps_i, eps_ip1 = wrk.pulses0, wrk.pulses1
+    for k in range(p.N):
+        O.krotov_initial_fw_prop(eps_i, p.psi0[k], k, wrk)
+    O.update_result(wrk)
+    out = dict(J_T=[wrk.J_T], g_a_int=[], tau=[wrk.tau_vals.copy()])
+    for _ in range(iters):
+        O.krotov_iteration(wrk, eps_i, eps_ip1)
+        states = O.update_result(wrk)
+        out["J_T"].append(wrk.J_T)
+        out["g_a_int"].append(wrk.g_a_int.copy())
+        out["tau"].append(wrk.tau_vals.copy())
+        eps_i, eps_ip1 = eps_ip1, eps_i
+    out["pulses"] = np.array(eps_i)
+    out["states"] = np.array(states)
+    out["X"] = np.array(wrk.bw_storage)
+    out["Phi"] = np.array(wrk.fw_storage)
+    return out
+
+
+@functools.lru_cache(maxsize=None)
+def exact(name):
+    return reference_run(case(name).oracle(), ITERS.get(name, 2), "expm")
+
+
+@functools.lru_cache(maxsize=None)
+def cheby(name):
+    return reference_run(case(name).oracle(), ITERS.get(name, 2), "cheby")
+
+
+def deviations(got, ref, storage=True):
+    """Largest absolute deviation per quantity."""
+    dev = dict(J_T=np.abs(np.asarray(got["J_T"]) - ref["J_T"]).max(),
+               pulses=np.abs(np.asarray(got["pulses"]) - ref["pulses"]).max(),
+               g_a_int=np.abs(np.asarray(got["g_a_int"]) - np.asarray(ref["g_a_int"])).max(),
+               tau=np.abs(np.asarray(got["tau"]) - np.asarray(ref["tau"])).max(),
+               states=np.abs(np.asarray(got["states"]) - ref["states"]).max())
+    if storage:
+        dev["X"] = np.abs(np.asarray(got["X"]) - ref["X"]).max()
+        dev["Phi"] = np.abs(np.asarray(got["Phi"]) - ref["Phi"]).max()
+    return dev
+
+
+# ---- cells ---------------------------------------------------------------------------------------------------------------
+# name -> (problem, environment, optimize keywords, kernel, lanes per trajectory, exchange)
+_PREG, _SEQ, _PAIR, _RELOAD = B.KERNEL_PREG, B.KERNEL_SEQ_PREG, B.KERNEL_PAIR, B.KERNEL_RELOAD
+CELLS = {
+    "tiny_jitter": ("tiny_jitter", {}, {}, B.KERNEL_TINY, 1, 0),
+    "tiny_nt2": ("tiny_nt2", {}, {}, B.KERNEL_TINY, 1, 0),
+    "preg_nt1": ("warp_nt1", {}, {}, _PREG, 32, 0),
+    "preg_L1_A": ("warp_L1_A", {}, {}, _PREG, 32, 0),
+    "preg_L1_B": ("warp_L1_B", {}, {}, _PREG, 32, 0),
+    "preg_L2_A": ("warp_L2_A", {}, {}, _PREG, 32, 0),
+    "preg_L2_B": ("warp_L2_B", {}, {}, _PREG, 32, 0),
+    "preg_L3_A": ("warp_L3_A", {}, {}, _PREG, 32, 0),
+    "preg_L3_B": ("warp_L3_B", {}, {}, _PREG, 32, 0),
+    "reload_L5_A": ("warp_L5_A", {"KROTOV_NO_PREG": "1"}, {}, _RELOAD, 32, 0),
+    "reload_L5_B": ("warp_L5_B", {"KROTOV_NO_PREG": "1"}, {}, _RELOAD, 32, 0),
+    "pair_A": ("pair_A", {"KROTOV_FORCE_PAIR": "1"}, {}, _PAIR, 32, 0),
+    "pair_B": ("pair_B", {"KROTOV_FORCE_PAIR": "1"}, {}, _PAIR, 32, 0),
+    "seq_B": ("seq_B", {"KROTOV_SEQ_PREG": "1"}, {}, _SEQ, 32, 0),
+    "wide64_A": ("wide64_A", {}, {}, _PREG, 64, 0),
+    "wide64_B": ("wide64_B", {}, {}, _PREG, 64, 0),
+    "wide128_B": ("wide128_B", {}, {}, _PREG, 128, 0),
+    "ranks_hier_B": ("ranks_B", {"KROTOV_XCHG": "hier"}, dict(emulate_ranks=2, multi_gpu="shard"), _PREG, 32, 1),
+    "ranks_mbox": ("ranks_lin", {"KROTOV_XCHG": "mbox"}, dict(emulate_ranks=3, multi_gpu="shard"), _PREG, 32, 3),
+    "ranks_rf_B": ("ranks_B", {}, dict(emulate_ranks=2, multi_gpu="replicate"), _PREG, 32, 5),
+    "dmma_A": ("dense_A", {"KROTOV_NO_DSWEEP": "1"}, {}, B.KERNEL_DMMA_STREAM, 0, 0),
+    "dmma_B": ("dense_B", {"KROTOV_NO_DSWEEP": "1"}, {}, B.KERNEL_DMMA_STREAM, 0, 0),
+    "dsweep_A": ("dense_A", {}, {}, B.KERNEL_DENSE_SWEEP, 0, 0),
+    "dsweep_B": ("dense_B", {}, {}, B.KERNEL_DENSE_SWEEP, 0, 0),
+    "sparse_sweep_A": ("sparse_A", {}, dict(force_path=3), B.KERNEL_SPARSE_SWEEP, 0, 0),
+    "sparse_sweep_B": ("sparse_B", {}, dict(force_path=3), B.KERNEL_SPARSE_SWEEP, 0, 0),
+    "sparse_stream_A": ("sparse_A", {"KROTOV_NO_SWEEP": "1"}, dict(force_path=3), B.KERNEL_SPARSE_STREAM, 0, 0),
+    "sparse_stream_B": ("sparse_B", {"KROTOV_NO_SWEEP": "1"}, dict(force_path=3), B.KERNEL_SPARSE_STREAM, 0, 0),
+    "graph_A": ("graph_A", {"KROTOV_NO_DSWEEP": "1"}, {}, B.KERNEL_DMMA_STREAM, 0, 0),
+}
+
+
+def run_cell(c, iters, storage, **kw):
+    """Optimise through the public API; J_T, g_a_int, tau of every iteration, the final pulses and states, every slot of
+    both storages after the last iteration (one-rank runs) and ``info()`` of the last iteration."""
+    hist = dict(J_T=[], g_a_int=[], tau=[])
+
+    def record(wrk, it, eps_new, eps_old):
+        hist["J_T"].append(wrk.result.J_T)
+        hist["tau"].append(np.array(wrk.result.tau_vals))
+        if it > 0:
+            hist["g_a_int"].append(np.array(wrk.g_a_int))
+        hist["pulses"] = np.array([np.array(e) for e in eps_new])
+        hist["info"] = wrk.engine.info()
+        if it == iters and storage:
+            hist["X"] = np.array([np.array(wrk.bw_storage[k]) for k in range(c.w.N)])
+            hist["Phi"] = np.array([np.array(wrk.fw_storage[k]) for k in range(c.w.N)])
+
+    res = K.optimize(c.problem(iter_stop=iters, callback=record, store_fw_states=storage, **kw), method=K.Krotov)
+    hist["states"] = np.array(res.states)
+    return hist
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("cell", list(CELLS))
+def test_cell_against_exact_dynamics(cell, monkeypatch):
+    name, env, kw, kernel, lanes, exchange = CELLS[cell]
+    for k, v in env.items():
+        monkeypatch.setenv(k, v)
+    iters = ITERS.get(name, 2)
+    storage = "emulate_ranks" not in kw
+    got = run_cell(case(name), iters, storage, **kw)
+    info = got["info"]
+    assert (info["kernel"], info["lanes_per_traj"], info["exchange"]) == (kernel, lanes, exchange), info
+    if name.startswith("tiny_jitter"):  # the coefficient table is read from global memory (coef_in_smem = 0)
+        w = case(name).w
+        assert len(set(np.diff(w.tlist))) == w.N_T
+        assert (1 + w.L) * w.d**2 * 32 * 16 + w.N_T * (info["m_fw"] + info["m_bw"]) * 32 * 8 > 160 * 1024
+    if name == "graph_A":
+        assert info["graph_replays"] >= 1
+    ch = cheby(name)
+    dj = np.abs(np.asarray(got["J_T"]) - ch["J_T"])
+    assert np.all(dj <= RTOL_JT * np.abs(ch["J_T"]) + ATOL_JT), (got["J_T"], ch["J_T"])
+    assert np.abs(got["pulses"] - ch["pulses"]).max() <= ATOL_PULSE
+    assert np.abs(np.asarray(got["g_a_int"]) - np.asarray(ch["g_a_int"])).max() <= 1e-11
+    dev = deviations(got, exact(name), storage)
+    assert max(dev.values()) <= BOUND[name], dev
+
+
+# ---- CPU: the references and the bounds ----------------------------------------------------------------------------------
+@pytest.mark.parametrize("name", list(PROBLEMS))
+def test_chebyshev_oracle_meets_a_tenth_of_the_bound(name):
+    """The bound of every problem is sound: the Chebyshev oracle itself stays within BOUND / 10 of the exact run, for
+    every quantity the GPU cells compare (every storage slot included)."""
+    assert BOUND[name] <= 1e-11
+    dev = deviations(cheby(name), exact(name))
+    assert max(dev.values()) <= BOUND[name] / 10, dev
+
+
+def test_exact_reference_against_40_digit_arithmetic():
+    """The float64 expm reference (shared per-generator propagators) against mp_reference.krotov_exact_general."""
+    import mp_reference as M
+
+    name = "tiny_nt2"
+    p = case(name).oracle()
+    ref = M.krotov_exact_general(p, iters=2, dps=40)
+    ex = exact(name)
+    assert np.abs(np.array(ref["J_T"]) - ex["J_T"]).max() < 1e-15
+    assert np.abs(np.array(ref["pulses"]) - ex["pulses"]).max() < 1e-15
+    assert np.abs(np.array(ref["g_a_int"]) - np.array(ex["g_a_int"])).max() < 1e-15
+    assert np.abs(np.array(ref["tau"]) - ex["tau"][-1]).max() < 1e-15
+
+
+def _two_corner_problem():
+    """Two anti-correlated controls: lambda_max(H0 + a1 H1 + a2 H2) peaks at a MIXED corner of the control ranges."""
+    w = W.dummy_dense(d=4, n_traj=2, n_controls=2, n_grid=41, seed=5)
+    X = np.zeros((4, 4))
+    X[0, 1] = X[1, 0] = X[2, 3] = X[3, 2] = 0.3
+    H1 = np.diag([3.0, 0, 0, 0]).astype(complex) + X
+    H2 = np.diag([-3.0, 0, 0, 0]).astype(complex) + X / 2
+    w.H0, w.Hc = [np.diag([0.0, 0.5, 1.0, 1.5]).astype(complex)], [[H1, H2]]
+    p = W.to_oracle(w)
+    p.pulses[1] = p.pulses[1] - p.pulses[1].max()  # control 2 <= 0
+    return p, H1, H2
+
+
+def test_two_corner_spectral_envelope_misses_the_mixed_corner():
+    """The spectral envelope is taken at two corners (all controls at their minimum, all at their maximum), as upstream
+    does.  With anti-correlated controls the extreme eigenvalue sits at a mixed corner: the window is too narrow and the
+    Chebyshev run leaves the exact dynamics by more than 1e-12; a window over all four corners brings it back."""
+    p, H1, H2 = _two_corner_problem()
+    ex = reference_run(p, 2, "expm")
+    two = reference_run(p, 2, "cheby")
+    gap = max(np.abs(np.array(two["J_T"]) - ex["J_T"]).max(), np.abs(two["states"] - ex["states"]).max())
+    assert gap > 1e-12
+    H0 = p.H0[0]
+    lo, hi = [5 * x.min() for x in p.pulses], [5 * x.max() for x in p.pulses]  # the oracle's widened ranges
+    ev = [np.linalg.eigvalsh(H0 + a * H1 + b * H2) for a in (lo[0], hi[0]) for b in (lo[1], hi[1])]
+    E_lo, E_hi = min(e[0] for e in ev), max(e[-1] for e in ev)
+    two_lo = min(np.linalg.eigvalsh(H0 + lo[0] * H1 + lo[1] * H2)[0], np.linalg.eigvalsh(H0 + hi[0] * H1 + hi[1] * H2)[0])
+    assert E_lo < two_lo  # the mixed corner extends the window
+    p4, _, _ = _two_corner_problem()
+    p4.specrange = (E_lo - 0.05, E_hi + 0.05)
+    four = reference_run(p4, 2, "cheby")
+    gap4 = max(np.abs(np.array(four["J_T"]) - ex["J_T"]).max(), np.abs(four["states"] - ex["states"]).max())
+    assert gap4 < 1e-12
