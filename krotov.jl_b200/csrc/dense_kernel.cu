@@ -1165,8 +1165,7 @@ bool sweep_configure(DenseEngine *e) {
         e->sweep = false;
         return false;
     }
-    cudaMemcpy(e->sw_blk.get<int>(), blk.data(), blk.size() * 4, cudaMemcpyHostToDevice);
-    return true;
+    return copy_to_device(e->sw_blk.get<int>(), blk.data(), blk.size() * 4, e->stream, true) == cudaSuccess;
 }
 
 inline const double *gen_coeffs_old(const DenseEngine *e, const double *d_eps);
@@ -1219,7 +1218,7 @@ bool dsweep_configure(DenseEngine *e) {
     if (!dalloc<int>(e->ds_units_dev, units.size(), err) ||
         !dalloc<double>(e->sw_partial, (size_t)kMaxL * n_units * kDsCluster, err) || !dalloc<unsigned>(e->sw_bar, 1, err))
         return false;
-    cudaMemcpy(e->ds_units_dev.get<int>(), units.data(), units.size() * 4, cudaMemcpyHostToDevice);
+    if (copy_to_device(e->ds_units_dev.get<int>(), units.data(), units.size() * 4, e->stream, true) != cudaSuccess) return false;
     e->ds_units = n_units;
     e->dsweep = true;
     return true;
@@ -1299,9 +1298,9 @@ int kernel_kind(const DenseEngine *e, int mode) {
 }
 
 template <typename T>
-bool sweep_upload(DevBuf &dst, const std::vector<T> &src, std::string &err) {
+bool sweep_upload(DenseEngine *e, DevBuf &dst, const std::vector<T> &src, std::string &err) {
     if (!dalloc<T>(dst, src.size(), err)) return false;  // (frees the previous table first)
-    DK_CHECK(cudaMemcpy(dst.get<void>(), src.data(), src.size() * sizeof(T), cudaMemcpyHostToDevice));
+    DK_CHECK(copy_to_device(dst.get<void>(), src.data(), src.size() * sizeof(T), e->stream, true));
     return true;
 }
 
@@ -1503,7 +1502,7 @@ DenseEngine *dense_create(int d, int N, int L, int N_T, int n_gen, const std::ve
         if (ok && e->streamk) {
             ok = dalloc<double2>(e->sk_ws, (size_t)R * kSkParts * BM * 64, err) &&
                  dalloc<unsigned>(e->sk_flags, (size_t)R * kSkParts * 4, err);
-            if (ok) cudaMemset(e->sk_flags.get<unsigned>(), 0, (size_t)R * kSkParts * 4 * sizeof(unsigned));
+            if (ok) cudaMemsetAsync(e->sk_flags.get<unsigned>(), 0, (size_t)R * kSkParts * 4 * sizeof(unsigned), e->stream);
         }
     }
     if (ok && e->sparse)
@@ -1517,7 +1516,7 @@ DenseEngine *dense_create(int d, int N, int L, int N_T, int n_gen, const std::ve
         for (size_t i = 0; i < (size_t)e->dp; ++i)
             for (int sl = 0; sl < e->W; ++sl)
                 cols[i * e->W + sl] = (i < (size_t)d) ? (*sp->cols)[i * e->W + sl] : (int)i;
-        cudaMemcpy(e->ell_cols.get<int>(), cols.data(), nslots * 4, cudaMemcpyHostToDevice);
+        copy_to_device(e->ell_cols.get<int>(), cols.data(), nslots * 4, e->stream, true);
         std::vector<cplx> vbuf(nslots);
         for (int dir = 0; dir < (e->hermitian ? 1 : 2); ++dir) {
             const std::vector<cplx> &src = dir == 0 ? *sp->vals_f : *sp->vals_b;
@@ -1525,7 +1524,7 @@ DenseEngine *dense_create(int d, int N, int L, int N_T, int n_gen, const std::ve
             for (int q = 0; q < n_gen * (1 + L); ++q) {
                 std::fill(vbuf.begin(), vbuf.end(), cplx(0, 0));
                 memcpy(vbuf.data(), &src[(size_t)q * d * e->W], sizeof(cplx) * (size_t)d * e->W);
-                cudaMemcpy(dst + (size_t)q * nslots, vbuf.data(), nslots * 16, cudaMemcpyHostToDevice);
+                copy_to_device(dst + (size_t)q * nslots, vbuf.data(), nslots * 16, e->stream, true);
             }
         }
     }
@@ -1539,12 +1538,12 @@ DenseEngine *dense_create(int d, int N, int L, int N_T, int n_gen, const std::ve
         const cplx *M = &Hdense[(size_t)q * d * d];
         std::fill(buf.begin(), buf.end(), cplx(0, 0));
         for (int i = 0; i < d; ++i) memcpy(&buf[(size_t)i * e->dp], &M[(size_t)i * d], sizeof(cplx) * d);
-        cudaMemcpy(e->Hf.get<double2>() + (size_t)q * mat, buf.data(), mat * 16, cudaMemcpyHostToDevice);
+        copy_to_device(e->Hf.get<double2>() + (size_t)q * mat, buf.data(), mat * 16, e->stream, true);
         if (!e->hermitian) {
             std::fill(buf.begin(), buf.end(), cplx(0, 0));
             for (int i = 0; i < d; ++i)
                 for (int j = 0; j < d; ++j) buf[(size_t)i * e->dp + j] = std::conj(M[(size_t)j * d + i]);
-            cudaMemcpy(e->Hb.get<double2>() + (size_t)q * mat, buf.data(), mat * 16, cudaMemcpyHostToDevice);
+            copy_to_device(e->Hb.get<double2>() + (size_t)q * mat, buf.data(), mat * 16, e->stream, true);
         }
     }
     auto to_block = [&](const double *src, double2 *dst) {
@@ -1554,14 +1553,14 @@ DenseEngine *dense_create(int d, int N, int L, int N_T, int n_gen, const std::ve
             for (int k = 0; k < N; ++k)
                 for (int i = 0; i < d; ++i) blk[(size_t)i * e->ld + e->col_of_traj[k]] = s[(size_t)k * d + i];
         }
-        cudaMemcpy(dst, blk.data(), e->slab * 16, cudaMemcpyHostToDevice);
+        copy_to_device(dst, blk.data(), e->slab * 16, e->stream, true);
     };
     to_block(psi0, e->PSI0.get<double2>());
     to_block(target, e->TGT.get<double2>());
-    cudaMemset(e->CHI.get<double2>(), 0, e->slab * 16);
-    cudaMemset(e->PSI.get<double2>(), 0, e->slab * 16);
-    cudaMemcpy(e->d_col_of_traj.get<int>(), e->col_of_traj.data(), (size_t)N * 4, cudaMemcpyHostToDevice);
-    cudaMemcpy(e->d_traj_of_col.get<int>(), e->traj_of_col.data(), (size_t)e->ld * 4, cudaMemcpyHostToDevice);
+    cudaMemsetAsync(e->CHI.get<double2>(), 0, e->slab * 16, e->stream);
+    cudaMemsetAsync(e->PSI.get<double2>(), 0, e->slab * 16, e->stream);
+    copy_to_device(e->d_col_of_traj.get<int>(), e->col_of_traj.data(), (size_t)N * 4, e->stream, false);
+    copy_to_device(e->d_traj_of_col.get<int>(), e->traj_of_col.data(), (size_t)e->ld * 4, e->stream, false);
     if (cudaGetLastError() != cudaSuccess) {
         err = "dense_create: upload failed";
         return nullptr;
@@ -1611,9 +1610,9 @@ bool dense_set_cheby(DenseEngine *e, int direction, int ndtc, const std::vector<
         std::vector<double2> ph(phase.size());
         for (size_t i = 0; i < phase.size(); ++i) ph[i] = make_double2(phase[i].real(), phase[i].imag());
         cudaStreamSynchronize(e->stream);
-        if (!sweep_upload(e->sw_coef[direction], coef, err) || !sweep_upload(e->sw_m[direction], m, err) ||
-            !sweep_upload(e->sw_phase[direction], ph, err) || !sweep_upload(e->sw_dtc[direction], dtc_of_step, err) ||
-            !sweep_upload(e->sw_Emin[direction], E_min, err) || !sweep_upload(e->sw_Delta[direction], Delta, err))
+        if (!sweep_upload(e, e->sw_coef[direction], coef, err) || !sweep_upload(e, e->sw_m[direction], m, err) ||
+            !sweep_upload(e, e->sw_phase[direction], ph, err) || !sweep_upload(e, e->sw_dtc[direction], dtc_of_step, err) ||
+            !sweep_upload(e, e->sw_Emin[direction], E_min, err) || !sweep_upload(e, e->sw_Delta[direction], Delta, err))
             return false;
     }
     for (int v : m)
@@ -1790,7 +1789,7 @@ bool dense_set_chi(DenseEngine *e, const double *chi_host, std::string &err) {
     const cplx *s = reinterpret_cast<const cplx *>(chi_host);
     for (int k = 0; k < e->N; ++k)
         for (int i = 0; i < e->d; ++i) blk[(size_t)i * e->ld + e->col_of_traj[k]] = s[(size_t)k * e->d + i];
-    DK_CHECK(cudaMemcpy(e->CHI.get<double2>(), blk.data(), e->slab * 16, cudaMemcpyHostToDevice));
+    DK_CHECK(copy_to_device(e->CHI.get<double2>(), blk.data(), e->slab * 16, e->stream, true));
     e->chi_from_host = true;
     return true;
 }

@@ -1,6 +1,6 @@
 // Owners of the library's device memory: one cudaMalloc allocation (DevBuf) and one CUDA IPC mapping of a peer's
 // allocation (IpcMapping).  Both are move-only and give back what they hold in their destructors; this header is the
-// only place that frees device memory or closes a mapping.
+// only place that frees device memory or closes a mapping.  copy_to_device is how host data reaches that memory.
 #pragma once
 #include <cuda_runtime.h>
 
@@ -101,5 +101,15 @@ class IpcMapping {
   private:
     void *p_ = nullptr;
 };
+
+// Copies `bytes` from host memory to device memory on `stream`, the stream of the handle that owns `dst`.  Every write
+// to the library's device memory is ordered on that stream: the sweeps run there, it is non-blocking, so nothing orders
+// it after work on the legacy stream, and a blocking cudaMemcpy from pageable memory may return before its DMA lands.
+// The copy may read `src` after this returns: `wait` waits for it, so that the caller may then free or rewrite `src`.
+inline cudaError_t copy_to_device(void *dst, const void *src, size_t bytes, cudaStream_t stream, bool wait) {
+    cudaError_t e = cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, stream);
+    if (e == cudaSuccess && wait) e = cudaStreamSynchronize(stream);
+    return e;
+}
 
 }  // namespace kr

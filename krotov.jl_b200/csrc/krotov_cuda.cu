@@ -195,23 +195,13 @@ int dev_alloc(krotov_handle h, DevBuf &b, size_t bytes) {
     return KROTOV_OK;
 }
 
+// v into b (grown as needed), ordered on the handle's stream (kr::copy_to_device).  wait = false only for a vector the
+// handle owns and does not rewrite before its stream is next synchronised; locals wait.
 template <typename T>
-int upload(krotov_handle h, DevBuf &b, const std::vector<T> &v) {
+int upload(krotov_handle h, DevBuf &b, const std::vector<T> &v, bool wait) {
     int rc = dev_alloc(h, b, v.size() * sizeof(T));
     if (rc) return rc;
-    if (!v.empty()) KR_CUDA(h, cudaMemcpy(b.get<void>(), v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice));
-    return KROTOV_OK;
-}
-
-// the same, ordered on the handle's stream: the sweeps that read the table run on that (non-blocking) stream, and a
-// blocking copy on the legacy stream from pageable memory may return before its DMA lands.  `v` must outlive the copy,
-// so callers pass vectors the handle owns.
-template <typename T>
-int upload_async(krotov_handle h, DevBuf &b, const std::vector<T> &v) {
-    int rc = dev_alloc(h, b, v.size() * sizeof(T));
-    if (rc) return rc;
-    if (!v.empty())
-        KR_CUDA(h, cudaMemcpyAsync(b.get<void>(), v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice, h->stream));
+    if (!v.empty()) KR_CUDA(h, kr::copy_to_device(b.get<void>(), v.data(), v.size() * sizeof(T), h->stream, wait));
     return KROTOV_OK;
 }
 
@@ -832,9 +822,9 @@ int check_err_flag(krotov_handle h) {
     long long wait_cycles;
     memcpy(&wait_cycles, flags + 2, 8);
     h->ms_rank_wait = h->rf ? (double)wait_cycles / (double)h->sm_clock_khz : 0.0;
-    if (flags[1]) cudaMemset(h->d_err.get<int>() + 1, 0, sizeof(int));
+    if (flags[1]) KR_CUDA(h, cudaMemsetAsync(h->d_err.get<int>() + 1, 0, sizeof(int), h->stream));
     if (flag) {
-        cudaMemset(h->d_err.get<void>(), 0, sizeof(int));
+        KR_CUDA(h, cudaMemsetAsync(h->d_err.get<void>(), 0, sizeof(int), h->stream));
         return fail(h, KROTOV_ERR_TIMEOUT, "in-kernel exchange timed out waiting for a partial sum");
     }
     return KROTOV_OK;
@@ -1012,27 +1002,28 @@ static int create_handle(krotov_handle h, const krotov_problem *pb) {
         if (!(pb->lambda_a[l] != 0.0)) return fail(h, KROTOV_ERR_ARG, "lambda_a must be non-zero");
         for (int n = 0; n < N_T; ++n) alpha[(size_t)l * N_T + n] = pb->update_shape[(size_t)l * N_T + n] / pb->lambda_a[l];
     }
-    if ((rc = upload(h, h->d_alpha, alpha))) return rc;
-    if ((rc = upload(h, h->d_dt, h->dt))) return rc;
-    if ((rc = upload(h, h->d_gen, h->gen_of_traj))) return rc;
-    if ((rc = upload(h, h->d_weight, h->weight))) return rc;
+    if ((rc = upload(h, h->d_alpha, alpha, true))) return rc;
+    if ((rc = upload(h, h->d_dt, h->dt, false))) return rc;
+    if ((rc = upload(h, h->d_gen, h->gen_of_traj, false))) return rc;
+    if ((rc = upload(h, h->d_weight, h->weight, false))) return rc;
     if ((rc = dev_alloc(h, h->d_eps_old, (size_t)L * N_T * 8))) return rc;
     if ((rc = dev_alloc(h, h->d_eps_new, (size_t)L * N_T * 8))) return rc;
     if ((rc = dev_alloc(h, h->d_ga, kr::kMaxCtrl * 8))) return rc;
     if ((rc = dev_alloc(h, h->d_tau, (size_t)N * 16))) return rc;
     if ((rc = dev_alloc(h, h->d_chicoef, (size_t)N * 16))) return rc;
     if ((rc = dev_alloc(h, h->d_err, 16))) return rc;
-    cudaMemset(h->d_err.get<void>(), 0, 16);
-    cudaMemset(h->d_tau.get<void>(), 0, (size_t)N * 16);
+    KR_CUDA(h, cudaMemsetAsync(h->d_err.get<void>(), 0, 16, h->stream));
+    KR_CUDA(h, cudaMemsetAsync(h->d_tau.get<void>(), 0, (size_t)N * 16, h->stream));
     // peer mailboxes for the per-time-step exchange between ranks: [N_T][L][rank], one per iteration parity
     // behind them (warp path): the accumulators of the one-hop cross-rank sum, word stride up to one 128-byte line
     h->mail_bytes = (size_t)N_T * kr::kMaxRanks * L * 8;
     h->xacc_bytes = (path == KROTOV_PATH_WARP && L * kr::kXLimbs <= 32) ? (size_t)N_T * L * kr::kXLimbs * kXaccMaxStride * 8 : 0;
     for (int par = 0; par < 2; ++par) {
         if ((rc = dev_alloc(h, h->d_mbox[par], h->mail_bytes + h->xacc_bytes + 256))) return rc;
-        cudaMemset(h->d_mbox[par].get<char>() + h->mail_bytes + h->xacc_bytes, 0, 256);  // rank-barrier flags (parity 0 only)
-        cudaMemset(h->d_mbox[par].get<void>(), 0xFF, h->mail_bytes);
-        if (h->xacc_bytes) cudaMemset(h->d_mbox[par].get<char>() + h->mail_bytes, 0, h->xacc_bytes);
+        // rank-barrier flags (parity 0 only)
+        KR_CUDA(h, cudaMemsetAsync(h->d_mbox[par].get<char>() + h->mail_bytes + h->xacc_bytes, 0, 256, h->stream));
+        KR_CUDA(h, cudaMemsetAsync(h->d_mbox[par].get<void>(), 0xFF, h->mail_bytes, h->stream));
+        if (h->xacc_bytes) KR_CUDA(h, cudaMemsetAsync(h->d_mbox[par].get<char>() + h->mail_bytes, 0, h->xacc_bytes, h->stream));
         h->peer_mbox[par][0] = h->d_mbox[par].get<double>();
     }
 
@@ -1048,13 +1039,13 @@ static int create_handle(krotov_handle h, const krotov_problem *pb) {
                     }
     if (path == KROTOV_PATH_WARP) {
         if (!pattern_built && (rc = build_pattern(h))) return rc;
-        if ((rc = upload(h, h->d_cols, h->cols))) return rc;
+        if ((rc = upload(h, h->d_cols, h->cols, false))) return rc;
         {
             std::vector<cplx> raw;
             build_raw_rows(h, KROTOV_FORWARD, raw);
-            if ((rc = upload(h, h->d_rawf, raw))) return rc;
+            if ((rc = upload(h, h->d_rawf, raw, true))) return rc;
             build_raw_rows(h, KROTOV_BACKWARD, raw);
-            if ((rc = upload(h, h->d_rawb, raw))) return rc;
+            if ((rc = upload(h, h->d_rawb, raw, true))) return rc;
         }
         choose_launch(h);
         h->tiny = d >= 2 && d <= 4 && N <= 32 && tiny_kernel_for(d, L) != nullptr && !getenv("KROTOV_NO_TINY");
@@ -1067,10 +1058,10 @@ static int create_handle(krotov_handle h, const krotov_problem *pb) {
         };
         std::vector<cplx> tmp;
         pad_states(pb->psi0, tmp);
-        if ((rc = upload(h, h->d_psi0, tmp))) return rc;
+        if ((rc = upload(h, h->d_psi0, tmp, true))) return rc;
         if (h->has_target) {
             pad_states(pb->target, tmp);
-            if ((rc = upload(h, h->d_target, tmp))) return rc;
+            if ((rc = upload(h, h->d_target, tmp, true))) return rc;
         }
         const size_t slab = (size_t)N * (N_T + 1) * h->lpt * 16;
         h->x_slab = slab / 16;
@@ -1082,7 +1073,8 @@ static int create_handle(krotov_handle h, const krotov_problem *pb) {
         if ((rc = dev_alloc(h, h->d_psif, (size_t)N * h->lpt * 16))) return rc;
         // Freshly initialised propagators hold the initial states: that is what `skip_initial_forward_propagation`
         // (src/optimize.jl:171-181) leaves for the first chi(T) (:297) and update_result! (:378-381)
-        cudaMemcpy(h->d_psif.get<void>(), h->d_psi0.get<void>(), (size_t)N * h->lpt * 16, cudaMemcpyDeviceToDevice);
+        KR_CUDA(h, cudaMemcpyAsync(h->d_psif.get<void>(), h->d_psi0.get<void>(), (size_t)N * h->lpt * 16, cudaMemcpyDeviceToDevice,
+                                   h->stream));
         if (h->has_target) {
             std::vector<cplx> tau0(N);
             const cplx *s0 = reinterpret_cast<const cplx *>(pb->psi0), *tg = reinterpret_cast<const cplx *>(pb->target);
@@ -1091,14 +1083,14 @@ static int create_handle(krotov_handle h, const krotov_problem *pb) {
                 for (int i = 0; i < d; ++i) a += std::conj(tg[(size_t)k * d + i]) * s0[(size_t)k * d + i];
                 tau0[k] = a;
             }
-            cudaMemcpy(h->d_tau.get<void>(), tau0.data(), (size_t)N * 16, cudaMemcpyHostToDevice);
+            if ((rc = upload(h, h->d_tau, tau0, true))) return rc;
         }
         h->swept = true;
         if ((rc = dev_alloc(h, h->d_R, ((size_t)N_T * h->nCTA * L + (size_t)N_T * L) * 8))) return rc;
         if ((rc = dev_alloc(h, h->d_acc, (size_t)N_T * L * kr::kFixLimbs * 8))) return rc;
         if (getenv("KROTOV_PROF")) {
             if ((rc = dev_alloc(h, h->d_prof, (size_t)h->nCTA * 8 * 8))) return rc;
-            cudaMemset(h->d_prof.get<void>(), 0, h->d_prof.bytes());
+            KR_CUDA(h, cudaMemsetAsync(h->d_prof.get<void>(), 0, h->d_prof.bytes(), h->stream));
         }
     } else {
         kr::SparseDesc sd;
@@ -1219,10 +1211,10 @@ int krotov_set_cheby(krotov_handle h, int direction, int n_dt_class, const int32
     }
     ct.dtc_of_step.assign(dt_class_of_step, dt_class_of_step + h->N_T);
     int rc;
-    if ((rc = upload(h, ct.dtc, ct.dtc_of_step))) return rc;
-    if ((rc = upload(h, ct.coef, ct.coef_host))) return rc;
-    if ((rc = upload(h, ct.m, ct.m_host))) return rc;
-    if ((rc = upload(h, ct.phase, ct.phase_host))) return rc;
+    if ((rc = upload(h, ct.dtc, ct.dtc_of_step, false))) return rc;
+    if ((rc = upload(h, ct.coef, ct.coef_host, false))) return rc;
+    if ((rc = upload(h, ct.m, ct.m_host, false))) return rc;
+    if ((rc = upload(h, ct.phase, ct.phase_host, true))) return rc;  // (waits for all four: the next call rewrites ct)
     ct.set = true;
     tr.lap("tables uploaded");
     if (h->path == KROTOV_PATH_WARP) {
@@ -1237,31 +1229,30 @@ int krotov_set_cheby(krotov_handle h, int direction, int n_dt_class, const int32
                 fb[2 * g] = direction == KROTOV_FORWARD ? -sc : sc;
                 fb[2 * g + 1] = Delta[g] / 2 + E_min[g];
             }
-            if ((rc = dev_alloc(h, h->d_rowscale, fb.size() * 8))) return rc;
-            KR_CUDA(h, cudaMemcpyAsync(h->d_rowscale.get<void>(), fb.data(), fb.size() * 8, cudaMemcpyHostToDevice, h->stream));
+            if ((rc = upload(h, h->d_rowscale, fb, true))) return rc;
             const size_t total = (size_t)h->n_gen * (1 + h->L) * (h->Wt + 1) * h->lpt;
             if ((rc = dev_alloc(h, dP, total * 16))) return rc;
             scale_rows_kernel<<<(unsigned)((total + 255) / 256), 256, 0, h->stream>>>(
                 raw.get<const double2>(), h->d_rowscale.get<const double2>(), dP.get<double2>(), 1 + h->L, h->Wt, h->lpt, h->d, total);
-            KR_CUDA(h, cudaStreamSynchronize(h->stream));  // fb is a local; the next call may rewrite d_rowscale
+            KR_CUDA(h, cudaStreamSynchronize(h->stream));  // the next call may rewrite d_rowscale
             h->launches_total += 1;
             tr.lap("rows scaled on the device");
         } else {
             build_rows(h, direction, rows);
             tr.lap("rows built");
-            if ((rc = upload(h, dP, rows))) return rc;
+            if ((rc = upload(h, dP, rows, true))) return rc;
         }
         if (direction == KROTOV_FORWARD) {
             std::vector<double> inv_s(h->n_gen);
             for (int g = 0; g < h->n_gen; ++g) inv_s[g] = Delta[g] / 4.0;
-            if ((rc = upload(h, h->d_inv_s, inv_s))) return rc;
+            if ((rc = upload(h, h->d_inv_s, inv_s, true))) return rc;
         }
         if (h->tiny) {
             build_dense_terms(h, direction, rows);
             bool imag = !getenv("KROTOV_NO_TINY_IMAG");
             for (const cplx &v : rows) imag = imag && (v.real() == 0.0);
             h->tiny_imag[direction] = imag;
-            if ((rc = upload(h, direction == KROTOV_FORWARD ? h->d_Tf : h->d_Tb, rows))) return rc;
+            if ((rc = upload(h, direction == KROTOV_FORWARD ? h->d_Tf : h->d_Tb, rows, true))) return rc;
         }
         tr.lap("rows uploaded");
     } else {
@@ -1313,8 +1304,8 @@ static int prepare_amplitudes(krotov_handle h, const double *pulses) {
         }
     }
     int rc;
-    if ((rc = upload_async(h, h->d_amp_old, a))) return rc;
-    if ((rc = upload_async(h, h->d_amp_dfac, da))) return rc;
+    if ((rc = upload(h, h->d_amp_old, a, false))) return rc;
+    if ((rc = upload(h, h->d_amp_dfac, da, false))) return rc;
     return KROTOV_OK;
 }
 
@@ -1365,7 +1356,8 @@ int krotov_set_chi(krotov_handle h, const double *chi) {
         const cplx *s = reinterpret_cast<const cplx *>(chi);
         for (int k = 0; k < N; ++k)
             for (int i = 0; i < d; ++i) tmp[(size_t)k * h->lpt + i] = s[(size_t)k * d + i];
-        KR_CUDA(h, cudaMemcpy(h->d_chiT.get<void>(), tmp.data(), tmp.size() * 16, cudaMemcpyHostToDevice));
+        int rc;
+        if ((rc = upload(h, h->d_chiT, tmp, true))) return rc;
     } else {
         std::string e;
         if (!kr::dense_set_chi(h->dense, chi, e)) return fail(h, KROTOV_ERR_CUDA, e);
@@ -1378,7 +1370,9 @@ int krotov_set_chi_coeffs(krotov_handle h, const double *coef) {
     if (!h || !coef) return KROTOV_ERR_ARG;
     if (!h->has_target) return fail(h, KROTOV_ERR_STATE, "krotov_set_chi_coeffs needs target states");
     cudaSetDevice(h->device);
-    KR_CUDA(h, cudaMemcpy(h->d_chicoef.get<void>(), coef, (size_t)h->N * 16, cudaMemcpyHostToDevice));
+    const cplx *c = reinterpret_cast<const cplx *>(coef);
+    int rc;
+    if ((rc = upload(h, h->d_chicoef, std::vector<cplx>(c, c + h->N), true))) return rc;
     h->chicoef_valid = true;
     h->chiT_valid = false;
     return KROTOV_OK;
@@ -1579,7 +1573,7 @@ int krotov_group_iterate(krotov_handle *hs, int world, const double *guess_pulse
             pv[world + r].rf_world = 0;
         }
     }
-    if ((rc = upload(h0, h0->d_emul, pv))) return rc;
+    if ((rc = upload(h0, h0->d_emul, pv, true))) return rc;
     kr::WarpParams p0;
     memset(&p0, 0, sizeof(p0));
     p0.emul = h0->d_emul.get<const kr::WarpParams>();
@@ -1637,8 +1631,8 @@ int krotov_set_amplitudes(krotov_handle h, int degree, const double *poly, const
     }
     if (shape) h->amp_shape.assign(shape, shape + (size_t)L * N_T);
     int rc;
-    if (!h->amp_poly.empty() && (rc = upload_async(h, h->d_amp_poly, h->amp_poly))) return rc;
-    if (!h->amp_shape.empty() && (rc = upload_async(h, h->d_amp_shape, h->amp_shape))) return rc;
+    if (!h->amp_poly.empty() && (rc = upload(h, h->d_amp_poly, h->amp_poly, false))) return rc;
+    if (!h->amp_shape.empty() && (rc = upload(h, h->d_amp_shape, h->amp_shape, false))) return rc;
     return amp_commit(h);
 }
 
@@ -1653,7 +1647,7 @@ int krotov_set_amplitude_saturation(krotov_handle h, const double *s) {
     h->amp_sat.clear();
     if (s && std::any_of(s, s + L, [](double v) { return v > 0.0; })) h->amp_sat.assign(s, s + L);
     int rc;
-    if (!h->amp_sat.empty() && (rc = upload_async(h, h->d_amp_sat, h->amp_sat))) return rc;
+    if (!h->amp_sat.empty() && (rc = upload(h, h->d_amp_sat, h->amp_sat, false))) return rc;
     return amp_commit(h);
 }
 
@@ -1672,7 +1666,7 @@ static int amp_commit(krotov_handle h) {
                 h->amp_rows[(size_t)l * R + p] = h->amp_poly.empty() ? (p == 1 ? 1.0 : 0.0) : h->amp_poly[(size_t)l * (D + 1) + p];
             h->amp_rows[(size_t)l * R + D + 1] = h->amp_sat.empty() ? 0.0 : h->amp_sat[l];
         }
-        if ((rc = upload_async(h, h->d_amp_rows, h->amp_rows))) return rc;
+        if ((rc = upload(h, h->d_amp_rows, h->amp_rows, false))) return rc;
     }
     if (h->amp_set) {
         if ((rc = dev_alloc(h, h->d_amp_old, (size_t)L * N_T * 8))) return rc;

@@ -136,7 +136,7 @@ def tls_krotov_exact(iters=5, n_grid=501, dps=50, float_grid=True, amp_poly=None
     return dict(J_T=[float(x) for x in J], J_T_mp=J, g_a_int=[float(x) for x in ga_hist], pulses=[float(x) for x in eps])
 
 
-def krotov_exact_general(p, iters=2, dps=40, sigma=None):
+def krotov_exact_general(p, iters=2, dps=40, sigma=None, chi=None, J_T=None):
     """The Krotov loop of ``src/optimize.jl:279-371`` for ANY small problem in `dps`-digit arithmetic with the exact
     propagator of every interval (``mpmath.expm``): several trajectories and generators, several controls, complex /
     missing control operators, weights, non-uniform grids, non-Hermitian generators (the backward sweep uses the adjoint
@@ -145,7 +145,11 @@ def krotov_exact_general(p, iters=2, dps=40, sigma=None):
     used.  Returns J_T per iteration, the running costs and the final pulses as floats.
 
     sigma: None | one number per time interval -- second-order update, the overlap of interval n gains
-    (sigma_n / 2) <psi_new(t_n) - psi_old(t_n)| mu |psi_new(t_n)> (any generator, any sigma(t): the general formula)."""
+    (sigma_n / 2) <psi_new(t_n) - psi_old(t_n)| mu |psi_new(t_n)> (any generator, any sigma(t): the general formula).
+
+    chi, J_T: None (the built-in functional of ``p.functional``) or callables of the final-time states (`dps`-digit
+    column vectors, one per trajectory) returning chi(T) (one column vector per trajectory) and J_T: a general
+    boundary condition.  tau stays the overlap with the targets."""
     mp.mp.dps = dps
     N, d, L, N_T = p.psi0.shape[0], p.psi0.shape[1], len(p.pulses), len(p.tlist) - 1
     c = lambda z: mp.mpc(float(z.real), float(z.imag))  # noqa: E731
@@ -215,12 +219,12 @@ def krotov_exact_general(p, iters=2, dps=40, sigma=None):
     for k in range(N):
         old[k][N_T] = states[k]
     tau = taus(states)
-    J, ga_hist = [J_of(tau)], []
+    J, ga_hist = [J_of(tau) if J_T is None else J_T(states)], []
     for _ in range(iters):
-        chi = chi_of(tau)
+        chi_T = chi_of(tau) if chi is None else chi(states)
         X = [[None] * (N_T + 1) for _ in range(N)]
         for k in range(N):
-            X[k][N_T] = chi[k]
+            X[k][N_T] = chi_T[k]
         for n in range(N_T - 1, -1, -1):  # backward with the adjoint generator under the GUESS pulses
             Ub = {g: mp.expm(j * dts[n] * H(g, [amp(l, n, eps[l][n]) for l in range(L)]).H) for g in gens}
             for k in range(N):
@@ -249,7 +253,7 @@ def krotov_exact_general(p, iters=2, dps=40, sigma=None):
             old[k][N_T] = states[k]
         eps = new
         tau = taus(states)
-        J.append(J_of(tau))
+        J.append(J_of(tau) if J_T is None else J_T(states))
         ga_hist.append(ga)
     return dict(J_T=[float(x) for x in J], g_a_int=[[float(x) for x in g] for g in ga_hist],
                 pulses=[[float(x) for x in row] for row in eps],

@@ -60,6 +60,36 @@ def test_destroy_functions_name_no_buffer():
     assert not re.search(r"\b(double2|double|int|unsigned|long long)\s*\*\s*\w+\s*=\s*nullptr", engine)
 
 
+def _calls(src, name):
+    """The argument text of every call of `name` (balanced parentheses, across lines)."""
+    out = []
+    for m in re.finditer(r"\b" + name + r"\(", src):
+        depth, i = 1, m.end()
+        while depth:
+            depth += {"(": 1, ")": -1}.get(src[i], 0)
+            i += 1
+        out.append(src[m.end():i - 1])
+    return out
+
+
+def test_every_device_write_is_ordered_on_the_handle_stream():
+    """The sweeps run on the handle's non-blocking stream, which nothing orders after work on the legacy stream: every
+    copy or memset that writes device memory is queued on the handle's stream (copy_to_device, cudaMemcpyAsync,
+    cudaMemsetAsync).  Blocking cudaMemcpy stays only for device-to-host reads."""
+    sources = sorted(f for f in os.listdir(CSRC) if f.endswith((".cu", ".cuh")))
+    assert {"krotov_cuda.cu", "dense_kernel.cu"} <= set(sources)
+    for f in sources:
+        src = _code(os.path.join(CSRC, f))
+        assert not _calls(src, "cudaMemset"), f
+        for args in _calls(src, "cudaMemcpy") + _calls(src, "cudaMemcpy2D"):
+            assert "cudaMemcpyDeviceToHost" in args, (f, args)
+        for args in _calls(src, "cudaMemcpyAsync") + _calls(src, "cudaMemsetAsync") + _calls(src, "copy_to_device"):
+            if "cudaStream_t" not in args:  # (not the definition of copy_to_device)
+                assert re.search(r",\s*(\w+->)?stream\s*(,|$)", args), (f, args)
+    copies = _calls(_code(os.path.join(CSRC, "device_buffer.cuh")), "cudaMemcpyAsync")
+    assert copies == ["dst, src, bytes, cudaMemcpyHostToDevice, stream"]
+
+
 # ---- on the GPU ----------------------------------------------------------------------------------------------------
 def _live():
     return K._lib.lib().krotov_live_device_objects()

@@ -12,10 +12,16 @@ them.  The problems combine, in few runs:
 - variant A: linear controls and a weakly non-Hermitian generator; variant B: Hermitian, a polynomial amplitude times a
   shape on one control and a TanhParametrization on another.
 
+Every cell also runs with chi(T) from the host (``krotov_set_chi``, a separate code path in every kernel family): a
+general observable functional, second order (sigma folded into chi(T)) and a trajectory without a target.  A sequence
+test switches one handle between chi(T) from tau, ``krotov_set_chi`` and ``krotov_set_chi_coeffs``.
+
 Each cell selects its kernel with the knobs the library reads and asserts, through ``info()``, which kernel served it.
-The exact bound of every problem (BOUND) is 10x the CPU Chebyshev-oracle-vs-exact gap rounded up to a power of ten; the
-CPU tests at the bottom check that the oracle meets BOUND / 10, so a GPU miss is the kernel's."""
+The exact bound of every (problem, boundary condition) (BOUND) is 10x the CPU Chebyshev-oracle-vs-exact gap rounded up
+to a power of ten; the CPU tests at the bottom check that the oracle meets BOUND / 10, so a GPU miss is the kernel's,
+and that every host boundary condition moves the exact pulses by >= 1e4 x BOUND."""
 import functools
+import zlib
 
 import numpy as np
 import pytest
@@ -217,7 +223,91 @@ def _graph_case():
 PROBLEMS["graph_A"] = _graph_case
 ITERS = {"graph_A": 5}
 
-# exact bound per problem: 10 x the CPU Chebyshev-oracle-vs-exact gap, rounded up to a power of ten, <= 1e-11
+
+@functools.lru_cache(maxsize=None)
+def case(name):
+    return PROBLEMS[name]()
+
+
+# ---- boundary conditions ---------------------------------------------------------------------------------------------
+# Where chi(T) comes from.  builtin: c_k |target_k>, formed on the device from tau (chi_coef_kernel); user_chi: the
+# Observable functional below, chi(T) from the host (krotov_set_chi) every iteration; sigma: second order with a constant
+# sigma, folded into chi(T) on the host (second_order.py); no_target: the Observable functional with no target for
+# trajectory 0 (tau_0 = 0).
+BOUNDARIES = ("builtin", "user_chi", "sigma", "no_target")
+
+
+class Observable:
+    """J_T = 1 - (1/N) sum_k w_k Re<Psi_k|O_k|Psi_k>, chi_k = -dJ_T/d<Psi_k| = (w_k / N) O_k Psi_k, with
+    O_k = |tgt_k><tgt_k| + coupling R_k and R_k a seeded random Hermitian matrix of its own for every trajectory:
+    trajectories that share a CTA, a pair or a column block get different chi(T), and every component of chi(T) is
+    non-zero."""
+
+    def __init__(self, target, weight, seed, coupling):
+        N, d = target.shape
+        g = np.random.default_rng(seed).standard_normal((2, N, d, d))
+        A = g[0] + 1j * g[1]
+        R =(A + A.conj().transpose(0, 2, 1)) / (2 * np.sqrt(d))
+        self.O = np.einsum("ki,kj->kij", target, target.conj()) + coupling * R
+        self.w = np.ones(N) if weight is None else np.asarray(weight, float)
+
+    @staticmethod
+    def _psi(states):
+        return np.array([np.asarray(s) for s in states], complex)
+
+    def chi(self, states, trajectories=None):
+        return list((self.w / len(self.w))[:, None] * np.einsum("kij,kj->ki", self.O, self._psi(states)))
+
+    def J_T(self, states, trajectories=None):
+        psi = self._psi(states)
+        return 1.0 - float(np.sum(self.w * np.einsum("ki,kij,kj->k", psi.conj(), self.O, psi).real)) / len(self.w)
+
+    def mp_hooks(self):
+        """(J_T, chi) of mp_reference.krotov_exact_general: the same functional on mpmath column vectors."""
+        import mpmath as mp
+
+        N, d = self.O.shape[:2]
+        O = [mp.matrix([[mp.mpc(complex(self.O[k, i, j])) for j in range(d)] for i in range(d)]) for k in range(N)]
+        w = [mp.mpf(float(x)) for x in self.w]
+
+        def J_T(states):
+            return 1 - sum(w[k] * mp.re((states[k].H * (O[k] * states[k]))[0, 0]) for k in range(N)) / N
+
+        def chi(states):
+            return [(w[k] / N) * (O[k] * states[k]) for k in range(N)]
+
+        return J_T, chi
+
+
+# constant sigma per Hermitian problem: moves the pulses by >= 1e-4 against first order (test_boundaries_move_the_pulses).
+# Not warp_nt1: with one time interval the second-order term is <Psi^(i+1)(0) - Psi^(i)(0)|...> = 0.  The sigma term
+# is summed over the trajectories without the 1/N of chi: seq_B's 1040 trajectories take a sigma ~1/200 of the others'.
+SIGMA = {
+    "tiny_nt2": -4.0, "warp_L1_B": -4.0, "warp_L2_B": -4.0, "warp_L3_B": -4.0, "warp_L5_B": -4.0, "pair_B": -4.0,
+    "seq_B": -0.02, "wide64_B": -4.0, "wide128_B": -8.0, "ranks_B": -4.0, "ranks_lin": -4.0, "dense_B": -4.0,
+    "sparse_B": -1.0, "graph_A": -4.0,
+}
+# problems of the no_target cells: tiny, register rows, pair, dense sweep, sparse sweep
+NO_TARGET = ("tiny_nt2", "warp_L2_B", "pair_B", "dense_B", "sparse_B")
+
+
+def applies(name, boundary):
+    return (boundary in ("builtin", "user_chi") or (boundary == "sigma" and name in SIGMA) or
+            (boundary == "no_target" and name in NO_TARGET))
+
+
+@functools.lru_cache(maxsize=None)
+def observable(name, boundary):
+    w, c = case(name).w, case(name)
+    target = np.array(w.target, complex).reshape(w.N, w.d)
+    if boundary == "no_target":
+        target[0] = 0.0
+    # (warp_nt1: its one interval spans the whole time; with 0.3 the updated pulse widens the spectral window so far that
+    # the Chebyshev oracle itself leaves the exact run by 1.7e-12)
+    return Observable(target, c.weight, seed=zlib.crc32(name.encode()), coupling=0.1 if name == "warp_nt1" else 0.3)
+
+
+# exact bound per (problem, boundary): 10 x the CPU Chebyshev-oracle-vs-exact gap, rounded up to a power of ten, <= 1e-11
 BOUND = {
     "tiny_jitter": 1e-12, "tiny_nt2": 1e-13, "warp_nt1": 1e-12, "warp_L1_A": 1e-12, "seq_B": 1e-12, "dense_A": 1e-12,
     "dense_B": 1e-12, "sparse_B": 1e-12, "graph_A": 1e-12,
@@ -225,11 +315,18 @@ BOUND = {
     "warp_L5_A": 1e-11, "warp_L5_B": 1e-11, "pair_A": 1e-11, "pair_B": 1e-11, "wide64_A": 1e-11, "wide64_B": 1e-11,
     "wide128_B": 1e-11, "ranks_B": 1e-11, "ranks_lin": 1e-11, "sparse_A": 1e-11,
 }
-
-
-@functools.lru_cache(maxsize=None)
-def case(name):
-    return PROBLEMS[name]()
+BOUND = {(name, "builtin"): b for name, b in BOUND.items()}
+BOUND.update({(name, "user_chi"): 1e-11 for name in PROBLEMS})
+BOUND.update({(name, "user_chi"): 1e-12 for name in ("tiny_jitter", "warp_nt1", "warp_L1_A", "seq_B", "dense_A",
+                                                     "dense_B", "sparse_B", "graph_A")})
+BOUND["tiny_nt2", "user_chi"] = 1e-13
+BOUND.update({(name, "sigma"): 1e-11 for name in SIGMA})
+BOUND.update({(name, "sigma"): 1e-12 for name in ("seq_B", "dense_B", "sparse_B", "graph_A")})
+BOUND["tiny_nt2", "sigma"] = 1e-13
+BOUND.update({("tiny_nt2", "no_target"): 1e-12, ("warp_L2_B", "no_target"): 1e-11, ("pair_B", "no_target"): 1e-11,
+              ("dense_B", "no_target"): 1e-12, ("sparse_B", "no_target"): 1e-12})
+BOUND.update({("tiny_jitter", "sequence"): 1e-12, ("warp_L2_A", "sequence"): 1e-11, ("pair_B", "sequence"): 1e-11,
+              ("graph_A", "sequence"): 1e-12, ("dense_A", "sequence"): 1e-12, ("sparse_B", "sequence"): 1e-12})
 
 
 # ---- references ------------------------------------------------------------------------------------------------------
@@ -255,10 +352,19 @@ class _SharedExp(O.ExpPropagator):
         return self.state
 
 
-def reference_run(p, iters, prop_method):
-    """The oracle's loop (``optimize_krotov``, first order, saturating amplitudes included) recording J_T, g_a_int and
-    tau of every iteration, the final pulses and states, and every slot of both storages after the last iteration."""
+def reference_run(p, iters, prop_method, chi=None, J_T=None, sigma=None):
+    """The oracle's loop (``optimize_krotov``, saturating amplitudes included) recording J_T, g_a_int and tau of every
+    iteration, the final pulses and states, and every slot of both storages after the last iteration.
+
+    chi: None (the built-in chi(T) of ``p.functional``), a callable Psi(T) -> chi(T) for every iteration, or
+    {iteration: callable} for the iterations (1-based) that take chi(T) from it.  J_T: a callable Psi(T) -> J_T in place
+    of the built-in functional.  sigma: a constant second-order sigma, through the oracle's general formula from the
+    stored previous trajectory.  With sigma there is no X: the device stores the backward-propagated boundary condition
+    chi(T) - sigma/2 Psi^(i)(T) (second_order.py), whose distance from the exact one is sigma/2 times the propagation
+    error of Psi^(i) -- the pulses, g_a_int and J_T test the fold."""
     wrk = S.SatOracleWrk(p, prop_method=prop_method, store_fw=True)
+    if sigma is not None:
+        wrk.enable_second_order()
     if prop_method == "expm":
         caches = {}
         for k in range(p.N):
@@ -270,30 +376,55 @@ def reference_run(p, iters, prop_method):
     eps_i, eps_ip1 = wrk.pulses0, wrk.pulses1
     for k in range(p.N):
         O.krotov_initial_fw_prop(eps_i, p.psi0[k], k, wrk)
-    O.update_result(wrk)
-    out = dict(J_T=[wrk.J_T], g_a_int=[], tau=[wrk.tau_vals.copy()])
-    for _ in range(iters):
-        O.krotov_iteration(wrk, eps_i, eps_ip1)
+
+    def result():
         states = O.update_result(wrk)
+        if J_T is not None:
+            wrk.J_T = J_T(states)
+        return states
+
+    result()
+    out = dict(J_T=[wrk.J_T], g_a_int=[], tau=[wrk.tau_vals.copy()])
+    sv = None if sigma is None else np.full(p.N_T, float(sigma))
+    for i in range(1, iters + 1):
+        O.krotov_iteration(wrk, eps_i, eps_ip1, chi=chi.get(i) if isinstance(chi, dict) else chi, sigma_vals=sv)
+        states = result()
         out["J_T"].append(wrk.J_T)
         out["g_a_int"].append(wrk.g_a_int.copy())
         out["tau"].append(wrk.tau_vals.copy())
         eps_i, eps_ip1 = eps_ip1, eps_i
     out["pulses"] = np.array(eps_i)
     out["states"] = np.array(states)
-    out["X"] = np.array(wrk.bw_storage)
+    out["X"] = np.array(wrk.bw_storage) if sigma is None else None
     out["Phi"] = np.array(wrk.fw_storage)
     return out
 
 
-@functools.lru_cache(maxsize=None)
-def exact(name):
-    return reference_run(case(name).oracle(), ITERS.get(name, 2), "expm")
+def boundary_problem(name, boundary):
+    """The oracle problem of `case(name)` and the keywords of reference_run for the boundary condition."""
+    p = case(name).oracle()
+    kw = {}
+    if boundary in ("user_chi", "no_target"):
+        obs = observable(name, boundary)
+        kw = dict(chi=obs.chi, J_T=obs.J_T)
+        if boundary == "no_target":
+            p.target = np.array(p.target)
+            p.target[0] = 0.0
+    elif boundary == "sigma":
+        kw = dict(sigma=SIGMA[name])
+    return p, kw
 
 
 @functools.lru_cache(maxsize=None)
-def cheby(name):
-    return reference_run(case(name).oracle(), ITERS.get(name, 2), "cheby")
+def exact(name, boundary="builtin"):
+    p, kw = boundary_problem(name, boundary)
+    return reference_run(p, ITERS.get(name, 2), "expm", **kw)
+
+
+@functools.lru_cache(maxsize=None)
+def cheby(name, boundary="builtin"):
+    p, kw = boundary_problem(name, boundary)
+    return reference_run(p, ITERS.get(name, 2), "cheby", **kw)
 
 
 def deviations(got, ref, storage=True):
@@ -303,9 +434,9 @@ def deviations(got, ref, storage=True):
                g_a_int=np.abs(np.asarray(got["g_a_int"]) - np.asarray(ref["g_a_int"])).max(),
                tau=np.abs(np.asarray(got["tau"]) - np.asarray(ref["tau"])).max(),
                states=np.abs(np.asarray(got["states"]) - ref["states"]).max())
-    if storage:
-        dev["X"] = np.abs(np.asarray(got["X"]) - ref["X"]).max()
-        dev["Phi"] = np.abs(np.asarray(got["Phi"]) - ref["Phi"]).max()
+    for key in ("X", "Phi") if storage else ():
+        if ref[key] is not None:
+            dev[key] = np.abs(np.asarray(got[key]) - ref[key]).max()
     return dev
 
 
@@ -345,36 +476,69 @@ CELLS = {
 }
 
 
-def run_cell(c, iters, storage, **kw):
+def run_cell(c, iters, storage, no_target=False, on_iteration=None, **kw):
     """Optimise through the public API; J_T, g_a_int, tau of every iteration, the final pulses and states, every slot of
-    both storages after the last iteration (one-rank runs) and ``info()`` of the last iteration."""
-    hist = dict(J_T=[], g_a_int=[], tau=[])
+    both storages after the last iteration (one-rank runs), ``info()`` of the last iteration, ``graph_replays`` after
+    every iteration and the number of ``set_chi`` calls.  no_target: trajectory 0 has no target state.
+    on_iteration(wrk, it): called at the end of the callback of iteration `it`."""
+    hist = dict(J_T=[], g_a_int=[], tau=[], replays=[], set_chi=0)
 
     def record(wrk, it, eps_new, eps_old):
+        if it == 0:
+            set_chi = wrk.engine.set_chi
+
+            def counted(chi):
+                hist["set_chi"] += 1
+                set_chi(chi)
+
+            wrk.engine.set_chi = counted
         hist["J_T"].append(wrk.result.J_T)
         hist["tau"].append(np.array(wrk.result.tau_vals))
         if it > 0:
             hist["g_a_int"].append(np.array(wrk.g_a_int))
         hist["pulses"] = np.array([np.array(e) for e in eps_new])
         hist["info"] = wrk.engine.info()
+        hist["replays"].append(hist["info"]["graph_replays"])
         if it == iters and storage:
             hist["X"] = np.array([np.array(wrk.bw_storage[k]) for k in range(c.w.N)])
             hist["Phi"] = np.array([np.array(wrk.fw_storage[k]) for k in range(c.w.N)])
+        if on_iteration is not None:
+            on_iteration(wrk, it)
 
-    res = K.optimize(c.problem(iter_stop=iters, callback=record, store_fw_states=storage, **kw), method=K.Krotov)
+    problem = c.problem(iter_stop=iters, callback=record, store_fw_states=storage, **kw)
+    if no_target:
+        problem.trajectories[0].target_state = None
+    res = K.optimize(problem, method=K.Krotov)
     hist["states"] = np.array(res.states)
     return hist
 
 
+def _boundary_keywords(name, boundary):
+    """The keywords of ``optimize`` for the boundary condition."""
+    if boundary in ("user_chi", "no_target"):
+        obs = observable(name, boundary)
+        return dict(J_T=obs.J_T, chi=obs.chi)
+    if boundary == "sigma":
+        return dict(sigma=SIGMA[name])
+    return {}
+
+
+def _cell_params():
+    """(cell, boundary) for every boundary that applies to the cell's problem; the built-in cells keep their ids."""
+    return [pytest.param(cell, b, id=cell if b == "builtin" else f"{cell}-{b}")
+            for b in BOUNDARIES for cell in CELLS if applies(CELLS[cell][0], b)]
+
+
 @pytest.mark.gpu
-@pytest.mark.parametrize("cell", list(CELLS))
-def test_cell_against_exact_dynamics(cell, monkeypatch):
+@pytest.mark.parametrize("cell,boundary", _cell_params())
+def test_cell_against_exact_dynamics(cell, boundary, monkeypatch):
     name, env, kw, kernel, lanes, exchange = CELLS[cell]
     for k, v in env.items():
         monkeypatch.setenv(k, v)
     iters = ITERS.get(name, 2)
     storage = "emulate_ranks" not in kw
-    got = run_cell(case(name), iters, storage, **kw)
+    got = run_cell(case(name), iters, storage, no_target=boundary == "no_target", **kw,
+                   **_boundary_keywords(name, boundary))
     info = got["info"]
     assert (info["kernel"], info["lanes_per_traj"], info["exchange"]) == (kernel, lanes, exchange), info
     if name.startswith("tiny_jitter"):  # the coefficient table is read from global memory (coef_in_smem = 0)
@@ -383,33 +547,130 @@ def test_cell_against_exact_dynamics(cell, monkeypatch):
         assert (1 + w.L) * w.d**2 * 32 * 16 + w.N_T * (info["m_fw"] + info["m_bw"]) * 32 * 8 > 160 * 1024
     if name == "graph_A":
         assert info["graph_replays"] >= 1
-    ch = cheby(name)
+    # chi(T) from the host once per iteration, and never for a built-in functional
+    assert got["set_chi"] == (0 if boundary == "builtin" else iters)
+    if boundary == "no_target":
+        assert all(t[0] == 0 for t in got["tau"])  # krotov_get_tau: exactly 0 without a target
+    ch = cheby(name, boundary)
     dj = np.abs(np.asarray(got["J_T"]) - ch["J_T"])
     assert np.all(dj <= RTOL_JT * np.abs(ch["J_T"]) + ATOL_JT), (got["J_T"], ch["J_T"])
     assert np.abs(got["pulses"] - ch["pulses"]).max() <= ATOL_PULSE
     assert np.abs(np.asarray(got["g_a_int"]) - np.asarray(ch["g_a_int"])).max() <= 1e-11
-    dev = deviations(got, exact(name), storage)
-    assert max(dev.values()) <= BOUND[name], dev
+    dev = deviations(got, exact(name, boundary), storage)
+    assert max(dev.values()) <= BOUND[name, boundary], dev
+
+
+# ---- one handle, chi(T) from three sources in turn ----------------------------------------------------------------------
+# "No krotov_set_chi* since the last sweep -> chi(T) from tau" (include/krotov_cuda.h): a built-in functional, and before
+# iteration 5 krotov_set_chi (the Observable chi), before iteration 7 krotov_set_chi_coeffs; every other iteration must
+# form chi(T) from tau again.
+SEQ_CELLS = ("tiny_jitter", "preg_L2_A", "pair_B", "graph_A", "dsweep_A", "sparse_sweep_B", "sparse_stream_B")
+SEQ_ITERS = 8
+
+
+def _seq_coeffs(name):
+    c = case(name).w
+    g = np.random.default_rng(zlib.crc32(name.encode()) + 1).standard_normal((2, c.N))
+    return (g[0] + 1j * g[1]) / c.N
+
+
+def _seq_sources(name):
+    """{iteration: chi(T) callable} of the sequence, for the reference."""
+    target = np.array(case(name).w.target, complex).reshape(case(name).w.N, -1)
+    coef = _seq_coeffs(name)
+    return {5: observable(name, "user_chi").chi, 7: lambda states: list(coef[:, None] * target)}
+
+
+@functools.lru_cache(maxsize=None)
+def sequence_reference(name, prop_method):
+    return reference_run(case(name).oracle(), SEQ_ITERS, prop_method, chi=_seq_sources(name))
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("cell", SEQ_CELLS)
+def test_chi_source_sequence_on_one_handle(cell, monkeypatch):
+    name, env, kw, kernel, lanes, exchange = CELLS[cell]
+    for k, v in env.items():
+        monkeypatch.setenv(k, v)
+    sources = _seq_sources(name)
+
+    def switch(wrk, it):
+        if it == 4:
+            wrk.engine.set_chi(np.array(sources[5](wrk.result.states)))
+        if it == 6:
+            wrk.engine.set_chi_coeffs(_seq_coeffs(name))
+
+    got = run_cell(case(name), SEQ_ITERS, True, on_iteration=switch, **kw)
+    info = got["info"]
+    assert (info["kernel"], info["lanes_per_traj"], info["exchange"]) == (kernel, lanes, exchange), info
+    assert got["set_chi"] == 1
+    if name == "graph_A":  # iteration 4 replays the graph captured in iteration 3; iteration 5 (host chi) does not
+        assert got["replays"][3:6] == [0, 1, 1], got["replays"]
+    ref = sequence_reference(name, "expm")
+    dev = deviations(got, ref)
+    assert max(dev.values()) <= BOUND[name, "sequence"], dev
+    # every iteration: J_T, tau and g_a_int are per iteration
+    assert np.abs(np.asarray(got["J_T"]) - ref["J_T"]).max() <= BOUND[name, "sequence"]
 
 
 # ---- CPU: the references and the bounds ----------------------------------------------------------------------------------
-@pytest.mark.parametrize("name", list(PROBLEMS))
-def test_chebyshev_oracle_meets_a_tenth_of_the_bound(name):
-    """The bound of every problem is sound: the Chebyshev oracle itself stays within BOUND / 10 of the exact run, for
-    every quantity the GPU cells compare (every storage slot included)."""
-    assert BOUND[name] <= 1e-11
-    dev = deviations(cheby(name), exact(name))
-    assert max(dev.values()) <= BOUND[name] / 10, dev
+def _bound_params():
+    return [pytest.param(name, b, id=name if b == "builtin" else f"{name}-{b}")
+            for b in BOUNDARIES for name in PROBLEMS if applies(name, b)]
+
+
+@pytest.mark.parametrize("name,boundary", _bound_params())
+def test_chebyshev_oracle_meets_a_tenth_of_the_bound(name, boundary):
+    """The bound of every (problem, boundary) is sound: the Chebyshev oracle itself stays within BOUND / 10 of the exact
+    run, for every quantity the GPU cells compare (every storage slot included)."""
+    assert BOUND[name, boundary] <= 1e-11
+    dev = deviations(cheby(name, boundary), exact(name, boundary))
+    assert max(dev.values()) <= BOUND[name, boundary] / 10, dev
+
+
+@pytest.mark.parametrize("name", sorted({CELLS[c][0] for c in SEQ_CELLS}))
+def test_chebyshev_oracle_meets_a_tenth_of_the_sequence_bound(name):
+    assert BOUND[name, "sequence"] <= 1e-11
+    dev = deviations(sequence_reference(name, "cheby"), sequence_reference(name, "expm"))
+    assert max(dev.values()) <= BOUND[name, "sequence"] / 10, dev
+
+
+@pytest.mark.parametrize("name,boundary", [p for p in _bound_params() if p.values[1] != "builtin"])
+def test_boundaries_move_the_pulses(name, boundary):
+    """Every boundary condition moves the exact pulses by >= 1e4 x BOUND against the built-in one (and sigma by >= 1e-4
+    against first order): a kernel that ignored a host chi(T), or read it with the wrong stride, trajectory or pair slot,
+    cannot meet the bound."""
+    move = np.abs(exact(name, boundary)["pulses"] - exact(name)["pulses"]).max()
+    assert move >= 1e4 * BOUND[name, boundary]
+    if boundary == "sigma":
+        assert move >= 1e-4
+
+
+@pytest.mark.parametrize("name", sorted({CELLS[c][0] for c in SEQ_CELLS}))
+def test_sequence_sources_move_the_pulses(name):
+    """The host sources of the sequence change the exact pulses by >= 1e4 x BOUND against the built-in run."""
+    builtin = reference_run(case(name).oracle(), SEQ_ITERS, "expm")["pulses"]
+    assert np.abs(sequence_reference(name, "expm")["pulses"] - builtin).max() >= 1e4 * BOUND[name, "sequence"]
 
 
 def test_exact_reference_against_40_digit_arithmetic():
     """The float64 expm reference (shared per-generator propagators) against mp_reference.krotov_exact_general."""
+    _against_40_digit_arithmetic("builtin")
+
+
+def test_exact_reference_with_user_chi_against_40_digit_arithmetic():
+    """The same with the Observable functional (chi(T) and J_T through the hooks of krotov_exact_general)."""
+    _against_40_digit_arithmetic("user_chi")
+
+
+def _against_40_digit_arithmetic(boundary):
     import mp_reference as M
 
     name = "tiny_nt2"
     p = case(name).oracle()
-    ref = M.krotov_exact_general(p, iters=2, dps=40)
-    ex = exact(name)
+    hooks = {} if boundary == "builtin" else dict(zip(("J_T", "chi"), observable(name, boundary).mp_hooks()))
+    ref = M.krotov_exact_general(p, iters=2, dps=40, **hooks)
+    ex = exact(name, boundary)
     assert np.abs(np.array(ref["J_T"]) - ex["J_T"]).max() < 1e-15
     assert np.abs(np.array(ref["pulses"]) - ex["pulses"]).max() < 1e-15
     assert np.abs(np.array(ref["g_a_int"]) - np.array(ex["g_a_int"])).max() < 1e-15
