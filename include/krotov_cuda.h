@@ -81,15 +81,16 @@ enum krotov_kernel { /* which kernel served the last forward/iterate call (kroto
 /*
  * The control problem, reduced to arrays.  Replaces what KrotovWrk's constructor collects
  * (src/workspace.jl:65-131): trajectories (initial/target state, generator), tlist, update
- * shapes S_l, lambda_a, control derivatives.  Linear controls only: mu_kl = dH_k/d eps_l is the
- * static term l of generator k (src/optimize.jl:275-276); a term flagged absent is the
- * reference's `nothing` (src/optimize.jl:344).
+ * shapes S_l, lambda_a, control derivatives.  Term l of generator k is a static operator H_kl (term 0 the drift); a term
+ * flagged absent is the reference's `nothing` (src/optimize.jl:344).  By default term l is control l and enters linearly,
+ * mu_kl = dH_k/d eps_l = H_kl (src/optimize.jl:275-276); krotov_set_amplitudes / krotov_set_amplitude_saturation give a
+ * term a non-linear amplitude and krotov_set_control_terms ties several terms to one control.
  */
 typedef struct {
     int32_t struct_size; /* = sizeof(krotov_problem), for ABI evolution */
     int32_t d;           /* Hilbert-space dimension                     */
     int32_t n_traj;      /* N: trajectories held by THIS handle (this rank's shard) */
-    int32_t n_ctrl;      /* L                                            */
+    int32_t n_ctrl;      /* L: control terms (= controls unless krotov_set_control_terms ties terms) */
     int32_t n_steps;     /* N_T = length(tlist) - 1                      */
     int32_t n_gen;       /* distinct generators (ensemble members sharing a Hamiltonian share one) */
     int32_t gen_format;  /* enum krotov_gen_format                       */
@@ -198,6 +199,22 @@ int krotov_set_amplitudes(krotov_handle h, int degree, const double *poly, const
  * the problem non-linear even when krotov_set_amplitudes left poly and shape NULL (poly_l(x) = x then).  Independent of
  * krotov_set_amplitudes (either may be called first); takes effect with the next krotov_forward / krotov_iterate. */
 int krotov_set_amplitude_saturation(krotov_handle h, const double *s);
+
+/* Control terms: one control that enters the generators through several (operator, amplitude) pairs, e.g. a drive in a
+ * rotating frame, cos(Dt) eps X + sin(Dt) eps Y, or a drive together with its quadratic ac-Stark shift.  The handle's
+ * n_ctrl counts TERMS: gen_values, term_present, update_shape, lambda_a, the amplitude polynomial, shape and saturation
+ * are per term.  control_of_term[n_ctrl] says which control each term belongs to (ids 0..C-1, numbered in order of first
+ * appearance); NULL = every term is its own control (the default; the identity map is the same state).  The overlap
+ * sums stay per term, S_t(n) = sum_k Im<chi_k| H_t |psi_k>; the update ties them (src/optimize.jl:351-358 with
+ * mu = sum_t a_t' H_t, as QuantumPropagators' get_control_deriv returns it):
+ *     du_c(n) = sum over the terms t of control c, ascending t, of a_t'(eps_c^(i)[n], n) S_t(n)
+ *     eps_c^(i+1)[n] = eps_c^(i)[n] + alpha_c[n] du_c(n),    H_t enters the forward step as a_t(eps_c^(i+1)[n], n) H_t.
+ * Pulses stay [n_ctrl][N_T], one row per term: the guess rows of tied terms must be bitwise equal (else krotov_forward /
+ * krotov_iterate return KROTOV_ERR_ARG), and the rows of one control in new_pulses are.  g_a_int[t] holds the control's
+ * integral at the control's first term and 0 at its other terms, so that sum_t g_a_int[t] = sum_c g_a_c.
+ * KROTOV_ERR_ARG: an id out of range or out of first-appearance order, or tied terms with different update_shape rows or
+ * lambda_a.  Takes effect with the next krotov_forward / krotov_iterate. */
+int krotov_set_control_terms(krotov_handle h, const int32_t *control_of_term);
 
 /* ---- the hot path ----------------------------------------------------------------------
  * krotov_forward: forward propagation of every trajectory under `pulses` without update.

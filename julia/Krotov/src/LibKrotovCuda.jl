@@ -128,6 +128,13 @@ function set_amplitude_saturation(h, s::Union{Nothing,Vector{Float64}})
                    s === nothing ? C_NULL : pointer(s)))
 end
 
+# control_of_term[t] (0-based control id of term t, numbered in order of first appearance) for a problem whose n_ctrl counts
+# (operator, amplitude) terms; `nothing` = every term is its own control
+function set_control_terms(h, control_of_term::Union{Nothing,Vector{Int32}})
+    check(h, ccall((:krotov_set_control_terms, lib), Cint, (Ptr{Cvoid}, Ptr{Int32}), h.ptr,
+                   control_of_term === nothing ? C_NULL : pointer(control_of_term)))
+end
+
 # pulses: Matrix{Float64}(N_T, L), column-major == [L][N_T] row-major on the wire
 forward(h, pulses::Matrix{Float64}) =
     check(h, ccall((:krotov_forward, lib), Cint, (Ptr{Cvoid}, Ptr{Float64}), h.ptr, pulses))

@@ -28,7 +28,7 @@ COMM_DESC_BYTES = 256
 # of them); krotov_live_device_objects returns a count and is bound below
 EXPORTS = [
     "krotov_abi_version", "krotov_create", "krotov_destroy", "krotov_last_error", "krotov_get_info",
-    "krotov_set_cheby", "krotov_set_amplitudes", "krotov_set_amplitude_saturation", "krotov_forward", "krotov_set_chi", "krotov_set_chi_coeffs", "krotov_iterate",
+    "krotov_set_cheby", "krotov_set_amplitudes", "krotov_set_amplitude_saturation", "krotov_set_control_terms", "krotov_forward", "krotov_set_chi", "krotov_set_chi_coeffs", "krotov_iterate",
     "krotov_get_states", "krotov_get_tau", "krotov_get_storage", "krotov_get_profile", "krotov_comm_export", "krotov_comm_connect",
     "krotov_group_connect", "krotov_group_iterate",
     "krotov_hermitian_extremes", "krotov_envelope_extremes", "krotov_envelope_extremes_device",
@@ -90,6 +90,7 @@ def lib():
     L.krotov_set_cheby.argtypes = [vp, i32, i32, vp, vp, vp, vp, vp, vp, i32]
     L.krotov_set_amplitudes.argtypes = [vp, i32, vp, vp]
     L.krotov_set_amplitude_saturation.argtypes = [vp, vp]
+    L.krotov_set_control_terms.argtypes = [vp, vp]
     L.krotov_forward.argtypes = [vp, vp]
     L.krotov_set_chi.argtypes = [vp, vp]
     L.krotov_set_chi_coeffs.argtypes = [vp, vp]

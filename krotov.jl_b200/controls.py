@@ -5,7 +5,8 @@ from __future__ import annotations
 
 import numpy as np
 
-__all__ = ["discretize", "discretize_on_midpoints", "get_controls", "get_control_derivs", "control_of", "get_amplitudes"]
+__all__ = ["discretize", "discretize_on_midpoints", "get_controls", "get_control_derivs", "control_of", "get_amplitudes",
+           "get_control_terms"]
 
 
 def control_of(amplitude):
@@ -126,3 +127,42 @@ def get_amplitudes(generator, controls):
                     raise ValueError("a control enters one generator both directly and through an amplitude: unsupported")
         out.append(found)
     return out
+
+
+def _amplitude_key(a):
+    """What makes two amplitudes of one control the same term: the same function of the control and the same shape
+    object.  None for the control itself."""
+    from .generators import ControlAmplitude
+
+    if not isinstance(a, ControlAmplitude):
+        return None
+    return (a.key(), id(a.shape) if a.shape is not None else None)
+
+
+def get_control_terms(generators, controls):
+    """The control terms of ``generators``: every (operator, amplitude) pair through which a control enters them.
+
+    Operators of one generator that depend on one control through the same amplitude (same ``key()`` and the same shape
+    object, or the control itself) are summed into one operator; different amplitudes make separate terms.  Term l is
+    control l for l < L (the control's first amplitude, in order of appearance); the further terms of controls that
+    enter through several amplitudes follow.  Returns ``(terms, ops)``: ``terms[t] = (l, amplitude or None)`` and
+    ``ops[g][t]`` the operator of term t in ``generators[g]`` (None where the generator lacks the term)."""
+    from .generators import ControlAmplitude, Generator
+
+    index = {id(c): l for l, c in enumerate(controls)}
+    seen = [[] for _ in controls]  # per control: (key, amplitude) in order of appearance
+    per_gen = []
+    for gen in generators:
+        ops = {}
+        if isinstance(gen, Generator):
+            for op, a in zip(gen.control_ops, gen.amplitudes):
+                l = index[id(control_of(a))]
+                k = _amplitude_key(a)
+                ops[(l, k)] = op if (l, k) not in ops else ops[(l, k)] + op
+                if all(k != kk for kk, _ in seen[l]):
+                    seen[l].append((k, a if isinstance(a, ControlAmplitude) else None))
+        per_gen.append(ops)
+    order = [(l, seen[l][0]) for l in range(len(controls)) if seen[l]]
+    order += [(l, ka) for l in range(len(controls)) for ka in seen[l][1:]]
+    terms = [(l, a) for l, (_, a) in order]
+    return terms, [[ops.get((l, k)) for l, (k, _) in order] for ops in per_gen]

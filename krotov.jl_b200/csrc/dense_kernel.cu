@@ -394,6 +394,47 @@ __device__ __forceinline__ double amp_apply(const AmpDev &am, const int l, const
     return c;
 }
 
+// Tied control terms (krotov_set_control_terms), one thread, once the overlap sums s[t] of every term are known over all
+// ranks: term t moves with du of its control, the sum over the control's terms in ascending t of a_t'(eps_old) s[t]
+// (src/optimize.jl:351-358 with mu = sum_t a_t' H_t).  On return s[t] = a_t(eps_new), the coefficient of H_t in the
+// forward step; eps_new and ga are written when `write`.  Out of line: the sweeps keep their code for untied problems.
+// P: the launch parameters (update_kernel's arguments, SweepParams or DSweepParams), read through a pointer to the
+// grid constant.
+template <class P>
+static __device__ __noinline__ void tie_update_cold(const P *pp, const int n, double *s, const bool write) {
+    const P &p = *pp;
+    const int L = p.L, N_T = p.N_T;
+    const double *ctrl = p.am.tie, *dfac = p.am.tie + L;
+    double du[kMaxL];
+    for (int t = 0; t < L; ++t) {
+        bool first = true;
+        for (int u = 0; u < L; ++u)
+            if (ctrl[u] == ctrl[t]) {
+                const double v = __dmul_rn(dfac[(size_t)u * N_T + n], s[u]);
+                du[t] = first ? v : __dadd_rn(du[t], v);
+                first = false;
+            }
+    }
+    for (int t = 0; t < L; ++t) {
+        const double a = p.alpha[(size_t)t * N_T + n];
+        const double e_new = __dadd_rn(p.eps_old[(size_t)t * N_T + n], __dmul_rn(a, du[t]));  // :355-356
+        s[t] = amp_apply(p.am, t, N_T, n, e_new);
+        if (write) {
+            p.eps_new[(size_t)t * N_T + n] = e_new;
+            const double prev = (n == 0) ? 0.0 : p.ga[t];
+            p.ga[t] = __dadd_rn(prev, __dmul_rn(__dmul_rn(a, __dmul_rn(fabs(du[t]), fabs(du[t]))), p.dt[n]));  // :357
+        }
+    }
+}
+
+// update_kernel's arguments in the shape tie_update_cold reads
+struct UpdateArgs {
+    int L, N_T;
+    const double *alpha, *eps_old, *dt;
+    double *eps_new, *ga;
+    AmpDev am;
+};
+
 // The rank's sum `s` of control l at time step n -> the sum over all ranks, the same bits on every rank: the rank sum is
 // pushed into slot [rank] of every rank's mailbox (system-scope stores over NVLink, by the caller flagged `push` only)
 // and the `world` slots of the own mailbox are polled and added in rank order.  Called by ONE lane; every CTA of the
@@ -423,12 +464,11 @@ __device__ __forceinline__ double rank_sum_lane(const DenseComm &cm, const int L
     return tot;
 }
 
-// fixed-order sum of the CTA partials of every control, rank exchange, pulse update (src/optimize.jl:351-358).
+// fixed-order sum of the CTA partials of control term l and the rank exchange; every lane returns the sum.
 // With several ranks the rank sum is pushed into every peer's mailbox (system-scope stores over NVLink) and
 // the `world` slots are summed in rank order -- the same protocol as the warp path's reducer.
-__global__ void update_kernel(const double *partial, int n_partial, int L, const double *alpha, const double *eps_old,
-                              double *eps_new, double *ga, const double *dt, int N_T, int n, DenseComm cm, AmpDev am) {
-    const int l = blockIdx.x, lane = threadIdx.x;
+__device__ __forceinline__ double term_sum(const double *partial, const int n_partial, const int L, const int l, const int n,
+                                           const DenseComm &cm, const int lane) {
     double s = 0.0;
     for (int c = lane; c < n_partial; c += 32) s += partial[(size_t)l * n_partial + c];
 #pragma unroll
@@ -453,6 +493,14 @@ __global__ void update_kernel(const double *partial, int n_partial, int L, const
         s = 0.0;
         for (int r = 0; r < cm.world; ++r) s += __shfl_sync(0xffffffffu, v, r);
     }
+    return s;
+}
+
+// pulse update (src/optimize.jl:351-358): block l updates term l
+__global__ void update_kernel(const double *partial, int n_partial, int L, const double *alpha, const double *eps_old,
+                              double *eps_new, double *ga, const double *dt, int N_T, int n, DenseComm cm, AmpDev am) {
+    const int l = blockIdx.x, lane = threadIdx.x;
+    double s = term_sum(partial, n_partial, L, l, n, cm, lane);
     if (lane == 0) {
         const double a = alpha[(size_t)l * N_T + n];
         if (am.dfac != nullptr) s = __dmul_rn(am.dfac[(size_t)l * N_T + n], s);  // mu_l = a_l'(eps^(i)) H_l
@@ -461,6 +509,22 @@ __global__ void update_kernel(const double *partial, int n_partial, int L, const
         if (am.amp_new != nullptr) am.amp_new[(size_t)l * N_T + n] = amp_apply(am, l, N_T, n, e_new);
         const double prev = (n == 0) ? 0.0 : ga[l];
         ga[l] = __dadd_rn(prev, __dmul_rn(__dmul_rn(a, __dmul_rn(fabs(s), fabs(s))), dt[n]));
+    }
+}
+
+// the same for tied control terms: ONE block sums every term, then ties them (tie_update_cold)
+__global__ void update_tied_kernel(const double *partial, int n_partial, int L, const double *alpha, const double *eps_old,
+                                   double *eps_new, double *ga, const double *dt, int N_T, int n, DenseComm cm, AmpDev am) {
+    __shared__ double s_sh[kMaxL];
+    const int lane = threadIdx.x;
+    for (int t = 0; t < L; ++t) {
+        const double s = term_sum(partial, n_partial, L, t, n, cm, lane);
+        if (lane == 0) s_sh[t] = s;
+    }
+    if (lane == 0) {
+        const UpdateArgs u{L, N_T, alpha, eps_old, dt, eps_new, ga, am};
+        tie_update_cold(&u, n, s_sh, true);
+        for (int t = 0; t < L; ++t) am.amp_new[(size_t)t * N_T + n] = s_sh[t];
     }
 }
 
@@ -938,16 +1002,22 @@ __global__ void __launch_bounds__(SP_WARPS * 32, 2) sparse_sweep_kernel(const __
                     if (lane == 0) {
                         const double a = p.alpha[(size_t)l * p.N_T + n];
                         sacc = rank_sum_lane(p.cm, p.L, n, l, sacc, blockIdx.x == 0);
-                        if (p.am.dfac != nullptr) sacc = __dmul_rn(p.am.dfac[(size_t)l * p.N_T + n], sacc);
-                        const double e_new = __dadd_rn(p.eps_old[(size_t)l * p.N_T + n], __dmul_rn(a, sacc));  // :355-356
-                        eps_sh[l] = amp_apply(p.am, l, p.N_T, n, e_new);
-                        if (blockIdx.x == 0) {
-                            p.eps_new[(size_t)l * p.N_T + n] = e_new;
-                            const double prev = (n == 0) ? 0.0 : p.ga[l];
-                            p.ga[l] = __dadd_rn(prev, __dmul_rn(__dmul_rn(a, __dmul_rn(fabs(sacc), fabs(sacc))), p.dt[n]));  // :357
+                        if (p.am.tie != nullptr) {
+                            eps_sh[l] = sacc;  // tied control terms: the update waits for the sums of all terms
+                        } else {
+                            if (p.am.dfac != nullptr) sacc = __dmul_rn(p.am.dfac[(size_t)l * p.N_T + n], sacc);
+                            const double e_new = __dadd_rn(p.eps_old[(size_t)l * p.N_T + n], __dmul_rn(a, sacc));  // :355-356
+                            eps_sh[l] = amp_apply(p.am, l, p.N_T, n, e_new);
+                            if (blockIdx.x == 0) {
+                                p.eps_new[(size_t)l * p.N_T + n] = e_new;
+                                const double prev = (n == 0) ? 0.0 : p.ga[l];
+                                p.ga[l] = __dadd_rn(prev, __dmul_rn(__dmul_rn(a, __dmul_rn(fabs(sacc), fabs(sacc))), p.dt[n]));  // :357
+                            }
                         }
                     }
                 }
+                if (p.am.tie != nullptr && lane == 0)
+                    tie_update_cold(&p, n, eps_sh, blockIdx.x == 0);
             }
             __syncthreads();
             for (int l = 0; l < p.L; ++l) eps[l] = eps_sh[l];
@@ -1773,8 +1843,12 @@ bool iterate_body(DenseEngine *e, const double *d_eps_old, double *d_eps_new, co
                 if (!launch_gemm(e, b, p, err)) return false;
             }
         }
-        update_kernel<<<e->L, 32, 0, e->stream>>>(e->partial.get<double>(), e->n_partial, e->L, d_alpha, d_eps_old, d_eps_new, d_ga,
-                                                 d_dt, N_T, n, e->comm, e->amp);
+        if (e->amp.tie != nullptr)
+            update_tied_kernel<<<1, 32, 0, e->stream>>>(e->partial.get<double>(), e->n_partial, e->L, d_alpha, d_eps_old, d_eps_new,
+                                                        d_ga, d_dt, N_T, n, e->comm, e->amp);
+        else
+            update_kernel<<<e->L, 32, 0, e->stream>>>(e->partial.get<double>(), e->n_partial, e->L, d_alpha, d_eps_old, d_eps_new, d_ga,
+                                                     d_dt, N_T, n, e->comm, e->amp);
         e->launches++;
         if (!step(e, KROTOV_FORWARD, n, gen_coeffs_new(e, d_eps_new),
                   e->store_fw ? e->PHI.get<double2>() + e->slab * (size_t)n : nullptr, err))

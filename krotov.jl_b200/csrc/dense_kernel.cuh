@@ -27,6 +27,9 @@ struct AmpDev {
     const double *shape = nullptr;    // [L][N_T] per-interval factor
     const double *sat = nullptr;      // [L] s_l > 0: the polynomial is evaluated at tanh(s_l eps) (bounded amplitudes)
     double *amp_new = nullptr;        // [L][N_T] a_l(eps_new), written by the pulse update (launch-per-term stream)
+    // Tied control terms (krotov_set_control_terms): [L] control of every term (as doubles), then [L][N_T] a_t'(eps_old).
+    // nullptr: every term is its own control.
+    const double *tie = nullptr;
 };
 void dense_set_amp(DenseEngine *e, const AmpDev &a);
 // Sparse generators (d > 32): ELL description with one shared pattern, slot 0 = diagonal.

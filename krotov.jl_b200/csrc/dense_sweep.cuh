@@ -378,16 +378,22 @@ __global__ void __launch_bounds__(kDsThreads, 1) dense_cluster_sweep_kernel(cons
                     if (lane == 0) {
                         const double al = p.alpha[(size_t)l * p.N_T + n];
                         sacc = rank_sum_lane(p.cm, p.L, n, l, sacc, blockIdx.x == 0);
-                        if (p.am.dfac != nullptr) sacc = __dmul_rn(p.am.dfac[(size_t)l * p.N_T + n], sacc);
-                        const double e_new = __dadd_rn(p.eps_old[(size_t)l * p.N_T + n], __dmul_rn(al, sacc));  // :355-356
-                        eps_sh[l] = amp_apply(p.am, l, p.N_T, n, e_new);
-                        if (blockIdx.x == 0) {
-                            p.eps_new[(size_t)l * p.N_T + n] = e_new;
-                            const double prev = (n == 0) ? 0.0 : p.ga[l];
-                            p.ga[l] = __dadd_rn(prev, __dmul_rn(__dmul_rn(al, __dmul_rn(fabs(sacc), fabs(sacc))), p.dt[n]));  // :357
+                        if (p.am.tie != nullptr) {
+                            eps_sh[l] = sacc;  // tied control terms: the update waits for the sums of all terms
+                        } else {
+                            if (p.am.dfac != nullptr) sacc = __dmul_rn(p.am.dfac[(size_t)l * p.N_T + n], sacc);
+                            const double e_new = __dadd_rn(p.eps_old[(size_t)l * p.N_T + n], __dmul_rn(al, sacc));  // :355-356
+                            eps_sh[l] = amp_apply(p.am, l, p.N_T, n, e_new);
+                            if (blockIdx.x == 0) {
+                                p.eps_new[(size_t)l * p.N_T + n] = e_new;
+                                const double prev = (n == 0) ? 0.0 : p.ga[l];
+                                p.ga[l] = __dadd_rn(prev, __dmul_rn(__dmul_rn(al, __dmul_rn(fabs(sacc), fabs(sacc))), p.dt[n]));  // :357
+                            }
                         }
                     }
                 }
+                if (p.am.tie != nullptr && lane == 0)
+                    tie_update_cold(&p, n, eps_sh, blockIdx.x == 0);
             }
             __syncthreads();
             for (int l = 0; l < p.L; ++l) cf[l] = eps_sh[l];

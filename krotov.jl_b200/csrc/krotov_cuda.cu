@@ -139,6 +139,12 @@ struct krotov_handle_s : HandleStream {
     std::vector<double> amp_rows;   // [L][kAmpRow]: the warp kernels' table, amp_poly rows (a(eps) = eps if empty) then s_l
     std::vector<double> amp_old_host, amp_dfac_host;  // a(eps_old), a'(eps_old): sources of the stream-ordered uploads
     DevBuf d_amp_poly, d_amp_shape, d_amp_sat, d_amp_rows, d_amp_old, d_amp_dfac, d_amp_new;
+    // tied control terms (krotov_set_control_terms)
+    std::vector<int> tie_ctrl;               // [L] control of every term; empty = every term is its own control
+    std::vector<int> tie_first;              // [L] 1 at the first term of its control
+    std::vector<double> tie_host;            // the tie table of the coming sweep: [L] tie_ctrl, then [L][N_T] a_t'(eps_old)
+    std::vector<double> update_shape_host, lambda_host;  // krotov_problem.update_shape / lambda_a (the setter's checks)
+    DevBuf d_tie;
     DevBuf d_emul;       // krotov_group_iterate: per-rank parameter blocks of the emulated multi-rank launch
     long long iter_count = 0;
     // the peers' mailboxes and chi trajectories mapped by krotov_comm_connect (peer_mbox / peer_Xbase point into them)
@@ -677,6 +683,7 @@ void fill_warp_params(krotov_handle h, int mode, kr::WarpParams &p) {
     p.amp_dfac = h->amp_set ? h->d_amp_dfac.get<const double>() : nullptr;
     p.amp_poly = (h->amp_set && !h->amp_rows.empty()) ? h->d_amp_rows.get<const double>() : nullptr;
     p.amp_shape = (h->amp_set && !h->amp_shape.empty()) ? h->d_amp_shape.get<const double>() : nullptr;
+    p.tie = h->tie_ctrl.empty() ? nullptr : h->d_tie.get<const double>();
     p.g_a_int = h->d_ga.get<double>();
     p.X = h->d_X.get<double2>(); p.Phi = h->d_Phi.get<double2>();
     p.psi0 = h->d_psi0.get<const double2>();
@@ -1003,6 +1010,8 @@ static int create_handle(krotov_handle h, const krotov_problem *pb) {
         for (int n = 0; n < N_T; ++n) alpha[(size_t)l * N_T + n] = pb->update_shape[(size_t)l * N_T + n] / pb->lambda_a[l];
     }
     if ((rc = upload(h, h->d_alpha, alpha, true))) return rc;
+    h->update_shape_host.assign(pb->update_shape, pb->update_shape + (size_t)L * N_T);
+    h->lambda_host.assign(pb->lambda_a, pb->lambda_a + L);
     if ((rc = upload(h, h->d_dt, h->dt, false))) return rc;
     if ((rc = upload(h, h->d_gen, h->gen_of_traj, false))) return rc;
     if ((rc = upload(h, h->d_weight, h->weight, false))) return rc;
@@ -1268,6 +1277,12 @@ int krotov_set_cheby(krotov_handle h, int direction, int n_dt_class, const int32
 static int prepare_amplitudes(krotov_handle h, const double *pulses) {
     if (!h->amp_set) return KROTOV_OK;
     const int L = h->L, N_T = h->N_T, D = kr::kAmpMaxDeg;
+    for (int t = 0; t < (int)h->tie_ctrl.size(); ++t) {  // tied terms carry their control's pulse: one row per term
+        const int t0 = (int)(std::find(h->tie_ctrl.begin(), h->tie_ctrl.end(), h->tie_ctrl[t]) - h->tie_ctrl.begin());
+        if (t0 != t && memcmp(pulses + (size_t)t * N_T, pulses + (size_t)t0 * N_T, (size_t)N_T * 8) != 0)
+            return fail(h, KROTOV_ERR_ARG, "pulse rows of tied control terms " + std::to_string(t0) + " and " +
+                                               std::to_string(t) + " differ");
+    }
     std::vector<double> &a = h->amp_old_host, &da = h->amp_dfac_host;
     a.resize((size_t)L * N_T);
     da.resize((size_t)L * N_T);
@@ -1304,6 +1319,13 @@ static int prepare_amplitudes(krotov_handle h, const double *pulses) {
         }
     }
     int rc;
+    if (!h->tie_ctrl.empty()) {
+        // tied control terms: a' goes into the tie table, the kernels' per-term factor becomes 1 (WarpParams::tie)
+        h->tie_host.assign(h->tie_ctrl.begin(), h->tie_ctrl.end());
+        h->tie_host.insert(h->tie_host.end(), da.begin(), da.end());
+        std::fill(da.begin(), da.end(), 1.0);
+        if ((rc = upload(h, h->d_tie, h->tie_host, false))) return rc;
+    }
     if ((rc = upload(h, h->d_amp_old, a, false))) return rc;
     if ((rc = upload(h, h->d_amp_dfac, da, false))) return rc;
     return KROTOV_OK;
@@ -1423,6 +1445,8 @@ static int iterate_finish(krotov_handle h, double *new_pulses, double *g_a_int) 
     if ((rc = check_err_flag(h))) return rc;
     KR_CUDA(h, cudaMemcpy(new_pulses, h->d_eps_new.get<void>(), (size_t)h->L * h->N_T * 8, cudaMemcpyDeviceToHost));
     KR_CUDA(h, cudaMemcpy(g_a_int, h->d_ga.get<void>(), (size_t)h->L * 8, cudaMemcpyDeviceToHost));
+    for (int t = 0; t < (int)h->tie_first.size(); ++t)  // tied terms: the control's integral sits at its first term
+        if (!h->tie_first[t]) g_a_int[t] = 0.0;
     h->chiT_valid = false;
     h->chicoef_valid = false;
     h->swept = true;
@@ -1654,7 +1678,8 @@ int krotov_set_amplitude_saturation(krotov_handle h, const double *s) {
 // after either amplitude entry point: the non-linear flag, the per-sweep tables and the block paths' view of them
 static int amp_commit(krotov_handle h) {
     const int L = h->L, N_T = h->N_T;
-    h->amp_set = !h->amp_poly.empty() || !h->amp_shape.empty() || !h->amp_sat.empty();
+    // tied control terms run on the non-linear code path (with a(eps) = eps where no amplitude is set)
+    h->amp_set = !h->amp_poly.empty() || !h->amp_shape.empty() || !h->amp_sat.empty() || !h->tie_ctrl.empty();
     int rc;
     // the warp kernels' table: one row per control, the polynomial (identity where only saturation is set) then s_l
     h->amp_rows.clear();
@@ -1673,6 +1698,7 @@ static int amp_commit(krotov_handle h) {
         if ((rc = dev_alloc(h, h->d_amp_dfac, (size_t)L * N_T * 8))) return rc;
         if ((rc = dev_alloc(h, h->d_amp_new, (size_t)L * N_T * 8))) return rc;
     }
+    if (!h->tie_ctrl.empty() && (rc = dev_alloc(h, h->d_tie, ((size_t)L + (size_t)L * N_T) * 8))) return rc;
     if (h->dense) {
         kr::AmpDev a;
         if (h->amp_set) {
@@ -1682,10 +1708,44 @@ static int amp_commit(krotov_handle h) {
             a.shape = h->amp_shape.empty() ? nullptr : h->d_amp_shape.get<const double>();
             a.sat = h->amp_sat.empty() ? nullptr : h->d_amp_sat.get<const double>();
             a.amp_new = h->d_amp_new.get<double>();
+            a.tie = h->tie_ctrl.empty() ? nullptr : h->d_tie.get<const double>();
         }
         kr::dense_set_amp(h->dense, a);
     }
     return KROTOV_OK;
+}
+
+int krotov_set_control_terms(krotov_handle h, const int32_t *control_of_term) {
+    if (!h) return KROTOV_ERR_ARG;
+    cudaSetDevice(h->device);
+    const int L = h->L, N_T = h->N_T;
+    std::vector<int> ctrl, first(L, 0);
+    bool tied = false;
+    if (control_of_term) {
+        int next = 0;  // ids are numbered in order of first appearance: term t opens control `next` or joins an earlier one
+        for (int t = 0; t < L; ++t) {
+            const int c = control_of_term[t];
+            if (c < 0 || c > next)
+                return fail(h, KROTOV_ERR_ARG, "control_of_term[" + std::to_string(t) + "] = " + std::to_string(c) +
+                                                   ": ids must be 0..C-1 in order of first appearance");
+            if (c == next) {
+                first[t] = 1;
+                ++next;
+                continue;
+            }
+            tied = true;
+            const int t0 = (int)(std::find(control_of_term, control_of_term + t, c) - control_of_term);
+            if (h->lambda_host[t] != h->lambda_host[t0] ||
+                memcmp(&h->update_shape_host[(size_t)t * N_T], &h->update_shape_host[(size_t)t0 * N_T], (size_t)N_T * 8) != 0)
+                return fail(h, KROTOV_ERR_ARG, "tied control terms " + std::to_string(t0) + " and " + std::to_string(t) +
+                                                   " have different update_shape rows or lambda_a");
+        }
+        if (tied) ctrl.assign(control_of_term, control_of_term + L);
+    }
+    // the identity map (or NULL) is the untied state itself
+    h->tie_ctrl = ctrl;
+    if (tied) h->tie_first = first; else h->tie_first.clear();
+    return amp_commit(h);
 }
 
 int krotov_get_states(krotov_handle h, double *states) {

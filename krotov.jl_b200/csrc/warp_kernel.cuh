@@ -95,7 +95,10 @@ struct WarpParams {
     int *err_flag;
     long long timeout_cycles;
     long long *prof;           // optional [nCTA][8] cycle counters (KROTOV_PROF=1), see krotov_get_profile
-    long long pad_;            // (keeps sizeof a multiple of 8 whatever follows)
+    // Tied control terms (krotov_set_control_terms): [L] control of every term (as doubles), then [L][N_T] a_t'(eps_old);
+    // amp_dfac then holds ones, so that the comm warp's loop applies alpha_t to the control's du (see tie_sum_cold).
+    // nullptr: every term is its own control.
+    const double *tie;
     // several ranks emulated by ONE cooperative launch on one device (krotov_group_iterate: the multi-rank protocols
     // on a single-GPU box; ranks as separate launches on one GPU may never be co-resident): the launch parameter then
     // only carries `emul`, the per-rank parameter blocks in device memory, and CTA b serves the rank whose
@@ -821,6 +824,26 @@ static __device__ __noinline__ double amp_eval_cold(const WarpParams *pp, const 
     return c;
 }
 
+// Tied control terms: every lane of the comm warp passes the grid-wide overlap sum `s` of its term (lanes < L) and gets
+// back du of the term's control, the sum over the control's terms in ascending t of a_t'(eps_old) s_t (the same bits on
+// every lane of every CTA and rank: the inputs are).  Out of line, as amp_eval_cold.
+static __device__ __noinline__ double tie_sum_cold(const WarpParams *pp, const int lane, const int n, const int L, const double s) {
+    const double *ctrl = pp->tie, *dfac = pp->tie + L;
+    const double v = lane < L ? __dmul_rn(dfac[(size_t)lane * pp->N_T + n], s) : 0.0;
+    const double c = lane < L ? ctrl[lane] : -1.0;
+    double du = 0.0;
+    bool first = true;
+#pragma unroll
+    for (int t = 0; t < kMaxCtrl; ++t) {
+        const double vt = __shfl_sync(0xffffffffu, v, t);
+        if (t < L && ctrl[t] == c) {
+            du = first ? vt : __dadd_rn(du, vt);
+            first = false;
+        }
+    }
+    return du;
+}
+
 // The communication warp of a CTA (shared by both kernel variants): per time step it waits for the CTA's
 // per-lane partial overlaps (named barrier 1), reduces them in a fixed order, runs the grid / rank exchange,
 // applies the pulse update (src/optimize.jl:351-358) and releases the trajectory warps (named barrier 2).
@@ -840,6 +863,7 @@ __device__ __forceinline__ void comm_warp_run(const WarpParams &p, const int cta
     }
     double ga = 0.0;  // lane l accumulates g_a_int[l]  (CTA 0 writes it)
     const bool nonlin = p.amp_dfac != nullptr;  // non-linear control amplitudes (rare): handled out of line
+    const bool tied = p.tie != nullptr;         // tied control terms (rare, implies nonlin): handled out of line
     long long c_wait_a = 0, c_reduce = 0, c_gather = 0;
     for (int n = 0; n < N_T; ++n) {
         double a_ln = 0.0, e_old = 0.0, dtn = 0.0, dfac = 1.0, shp = 1.0, a_eff = 0.0;
@@ -901,6 +925,7 @@ __device__ __forceinline__ void comm_warp_run(const WarpParams &p, const int cta
 #pragma unroll
         for (int l = 0; l < kMaxCtrl; ++l)
             if (lane == l) mine = tot[l];
+        if (tied) mine = tie_sum_cold(p_sh, lane, n, L, mine);  // (amp_dfac holds ones: a_eff = alpha, du = mine)
         double e_new = 0.0;
         if (lane < L) {
             const double d_eps = __dmul_rn(a_eff, mine);     // src/optimize.jl:355 (a_eff = alpha, or alpha a_l' when non-linear)

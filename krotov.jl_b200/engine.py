@@ -151,6 +151,13 @@ class KrotovCuda:
             s = np.ascontiguousarray(s, np.float64).reshape(self.L)
         self._check(self._lib.krotov_set_amplitude_saturation(self._h, _ptr(s)))
 
+    def set_control_terms(self, control_of_term=None):
+        """Tie control terms to controls (``krotov_set_control_terms``): ``control_of_term``: (L,) control id of every
+        term, numbered in order of first appearance; None = every term is its own control."""
+        if control_of_term is not None:
+            control_of_term = np.ascontiguousarray(control_of_term, np.int32).reshape(self.L)
+        self._check(self._lib.krotov_set_control_terms(self._h, _ptr(control_of_term)))
+
     # -- hot path -------------------------------------------------------------------------
     def forward(self, pulses):
         p = np.ascontiguousarray(pulses, np.float64).reshape(self.L, self.N_T)
@@ -267,6 +274,10 @@ class KrotovCudaGroup:
     def set_amplitude_saturation(self, s=None):
         for e in self.engines:
             e.set_amplitude_saturation(s)
+
+    def set_control_terms(self, control_of_term=None):
+        for e in self.engines:
+            e.set_control_terms(control_of_term)
 
     def forward(self, pulses):
         for e in self.engines:  # no cross-rank dependency in a plain forward sweep

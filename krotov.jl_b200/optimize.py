@@ -55,9 +55,9 @@ def krotov_initial_fw_prop(eps0, wrk):
     ``src/optimize.jl:182-184``): range check of ``reinit_prop!`` (``:251``), then one device sweep."""
     for view in wrk.fw_propagators:
         view.parameters = eps0
-    if wrk.fw_settings.reinit(eps0, transform_control_ranges):
+    if wrk.fw_settings.reinit(wrk._term_rows(eps0), transform_control_ranges):
         wrk.fw_settings.push(wrk.engine, B.FORWARD)
-    wrk.engine.forward(_stack(eps0))
+    wrk.engine.forward(_stack(wrk._term_rows(eps0)))
     wrk._states.invalidate()
 
 
@@ -97,15 +97,17 @@ def krotov_iteration(wrk, eps_i, eps_ip1):
     # reinit_prop! of the backward propagators under the guess pulses (:305-306)
     for view in wrk.bw_propagators:
         view.parameters = eps_i
-    if wrk.bw_settings.reinit(eps_i, transform_control_ranges):
+    if wrk.bw_settings.reinit(wrk._term_rows(eps_i), transform_control_ranges):
         wrk.bw_settings.push(wrk.engine, B.BACKWARD)
     # reinit_prop! of the forward propagators (:321-325): the check sees the eps^(i+1) buffers as they
     # are NOW (stale content), exactly like the reference's aliased arrays
     for view in wrk.fw_propagators:
         view.parameters = eps_ip1
-    if wrk.fw_settings.reinit(eps_ip1, transform_control_ranges):
+    if wrk.fw_settings.reinit(wrk._term_rows(eps_ip1), transform_control_ranges):
         wrk.fw_settings.push(wrk.engine, B.FORWARD)
-    new, ga = wrk.engine.iterate(_stack(eps_i))
+    new, ga = wrk.engine.iterate(_stack(wrk._term_rows(eps_i)))
+    if wrk._term_ctrl is not None:  # control terms -> controls: term l < L is control l, g_a sits at a control's first term
+        ga = np.bincount(wrk._term_ctrl, weights=ga, minlength=len(eps_ip1))
     for l in range(len(eps_ip1)):
         eps_ip1[l][:] = new[l]  # in place: callbacks hold references to these arrays
     wrk.g_a_int[:] = ga

@@ -20,7 +20,7 @@ import numpy as np
 
 from . import _lib as B
 from .cheby import ChebyDirection
-from .controls import discretize_on_midpoints, get_amplitudes, get_control_derivs, get_controls
+from .controls import discretize_on_midpoints, get_control_derivs, get_control_terms, get_controls
 from .engine import KrotovCuda
 from .errors import ArgumentError, ErrorException
 from .functionals import make_chi
@@ -225,8 +225,18 @@ class KrotovWrk:
         self.controls = get_controls(self.trajectories)
         if len(self.controls) == 0:
             raise ErrorException("no controls in trajectories: cannot optimize")
+        # control_derivs[k][l]: the sum of the operators through which control l enters generator k (None: it does not),
+        # whatever their amplitudes -- for a control with several terms this is not mu = sum_t a_t' H_t; the device
+        # evaluates mu per term (see _terms)
         self.control_derivs = [get_control_derivs(t.generator, self.controls) for t in self.trajectories]
         tlist = np.asarray(problem.tlist, np.float64)
+        # control terms: (control, amplitude) pairs, term l = control l for l < L, further terms of controls that enter
+        # through several amplitudes after them; _term_ops[g][t] per distinct generator (by identity, first appearance)
+        gens = list({id(t.generator): t.generator for t in self.trajectories}.values())
+        self._terms, self._term_ops = get_control_terms(gens, self.controls)
+        self._term_ctrl = (None if len(self._terms) == len(self.controls) else
+                           np.array([l for l, _ in self._terms], np.int32))
+        self._check_term_functions()
         self._amp_poly, self._amp_shape, self._amp_sat = self._collect_amplitudes(tlist)
         kwargs = dict(kwargs_in)  # shallow copy; ok to modify
         default_shape = kwargs_in.get("update_shape", lambda t: 1.0)
@@ -325,33 +335,15 @@ class KrotovWrk:
 
     # -------------------------------------------------------------------------------------
     def _collect_amplitudes(self, tlist):
-        """Non-linear / shaped amplitudes (``src/optimize.jl:268-272``): per control the polynomial, the per-interval
+        """Non-linear / shaped amplitudes (``src/optimize.jl:268-272``): per control TERM the polynomial, the per-interval
         shape and the saturation ``s`` (a parametrization's ``tanh(s u)``, 0 = none) through which it enters the
-        generators -- the same for every generator that depends on the control (the batched device propagator evaluates
-        one amplitude per control).  ``(None, None, None)`` for linear controls."""
-        L = len(self.controls)
-        chosen = [None] * L
-        seen = set()
-        for t in self.trajectories:
-            if id(t.generator) in seen:
-                continue
-            seen.add(id(t.generator))
-            amps = get_amplitudes(t.generator, self.controls)
-            derivs = get_control_derivs(t.generator, self.controls)
-            for l in range(L):
-                if derivs[l] is None:
-                    continue
-                a = amps[l]
-                key = None if a is None else (a.key(), id(a.shape) if a.shape is not None else None)
-                if chosen[l] is None:
-                    chosen[l] = (key, a)
-                elif chosen[l][0] != key:
-                    raise ArgumentError("a control must enter all generators through the same amplitude")
-        amps = [c[1] if c is not None else None for c in chosen]
+        generators.  ``(None, None, None)`` when every term is its control itself."""
+        amps = [a for _, a in self._terms]
+        T = len(amps)
         if all(a is None for a in amps):
             return None, None, None
         deg = max(len(a.coeffs) - 1 for a in amps if a is not None)
-        poly = np.zeros((L, deg + 1))
+        poly = np.zeros((T, deg + 1))
         shape = None
         for l, a in enumerate(amps):
             if a is None:
@@ -360,12 +352,29 @@ class KrotovWrk:
             poly[l, : len(a.coeffs)] = a.coeffs
             if a.shape is not None:
                 if shape is None:
-                    shape = np.ones((L, len(tlist) - 1))
+                    shape = np.ones((T, len(tlist) - 1))
                 shape[l] = discretize_on_midpoints(a.shape, tlist)
-        if all(np.array_equal(poly[l], np.eye(deg + 1)[1]) for l in range(L)):
+        if all(np.array_equal(poly[l], np.eye(deg + 1)[1]) for l in range(T)):
             poly = None  # only shapes: a(eps, n) = shape[n] * eps
         sat = np.array([0.0 if a is None else a.saturation for a in amps])
         return poly, shape, (sat if np.any(sat > 0) else None)
+
+    def _check_term_functions(self):
+        """Every generator that depends on a control must see it through the same amplitude FUNCTIONS (``key()``): the
+        terms of a control may differ between generators in their shapes only (an ensemble member with its own
+        distortion of the pulse envelope), not in the polynomial or parametrization that maps the control value."""
+        fn = lambda a: None if a is None else a.key()  # noqa: E731
+        for l in range(len(self.controls)):
+            seen = {frozenset(fn(a) for (c, a), op in zip(self._terms, row) if c == l and op is not None)
+                    for row in self._term_ops}
+            seen.discard(frozenset())
+            if len(seen) > 1:
+                raise ArgumentError("a control must enter all generators through the same amplitudes (their shapes may "
+                                    "differ between generators)")
+
+    def _term_rows(self, rows):
+        """Per-control rows (pulses, update shapes, lambda) -> one row per control term: term t carries its control's."""
+        return rows if self._term_ctrl is None else [rows[l] for l in self._term_ctrl]
 
     def _amp_envelope(self, l, eps):
         """Coefficient of H_l at a corner ``eps`` of the control range, for the spectral envelope: the polynomial at
@@ -393,7 +402,7 @@ class KrotovWrk:
 
     def _build_device_side(self, tlist, comm):
         trajs = self.trajectories
-        N, L = self.N, len(self.controls)
+        N, L = self.N, len(self._terms)  # (the device counts control terms)
         d = trajs[0].initial_state.shape[0]
         # distinct generators by identity: ensemble members sharing a Hamiltonian share its storage
         gen_ids, gens, gen_of_traj = {}, [], np.zeros(N, np.int32)
@@ -401,7 +410,7 @@ class KrotovWrk:
             key = id(t.generator)
             if key not in gen_ids:
                 gen_ids[key] = len(gens)
-                gens.append((t.generator, self.control_derivs[k]))
+                gens.append((t.generator, self._term_ops[len(gens)]))
             gen_of_traj[k] = gen_ids[key]
         H0, Hc = [], []
         for gen, derivs in gens:
@@ -428,7 +437,8 @@ class KrotovWrk:
         rank, world = (comm.rank, comm.world) if comm is not None else (0, 1)
         from .distributed import shard_bounds
 
-        S = np.array(self.update_shapes, np.float64).reshape(L, -1)
+        S = np.array(self._term_rows(self.update_shapes), np.float64).reshape(L, -1)
+        lam = np.array(self._term_rows(self.lambda_vals), np.float64)
         pk = self.fw_prop_kwargs[0]
         device = int(self.kwargs.get("device", comm.device if comm is not None else 0))
 
@@ -453,7 +463,7 @@ class KrotovWrk:
                 tlist=tlist, H0=[H0[g] for g in local_gens], Hc=[Hc[g] for g in local_gens],
                 gen_of_traj=np.array([remap[int(g)] for g in gen_of_traj[lo:hi]], np.int32),
                 psi0=psi0[lo:hi], target=None if target is None else target[lo:hi], weight=weight[lo:hi],
-                update_shape=S, lambda_a=self.lambda_vals, functional=functional, n_traj_global=N,
+                update_shape=S, lambda_a=lam, functional=functional, n_traj_global=N,
                 store_fw=self.store_fw, device=device, force_path=int(self.kwargs.get("force_path", 0)),
                 csr=bool(self.kwargs.get("csr_generators", False)), replicated_forward=self._replicated)
             return eng, local_gens
@@ -480,6 +490,8 @@ class KrotovWrk:
             self._Hc = [Hc[g] for g in local_gens]
         if comm is not None and world > 1:
             comm.connect(self.engine)
+        if self._term_ctrl is not None:
+            self.engine.set_control_terms(self._term_ctrl)
         nonlinear = self._amp_poly is not None or self._amp_shape is not None or self._amp_sat is not None
         if nonlinear:
             self.engine.set_amplitudes(self._amp_poly, self._amp_shape)
@@ -507,7 +519,7 @@ class KrotovWrk:
             H0s = [adj(h) for h in self._H0] if backward else self._H0
             Hcs = [[None if h is None else adj(h) for h in row] for row in self._Hc] if backward else self._Hc
             return ChebyDirection(
-                H0s, Hcs, tlist, backward, self._init_pulses,
+                H0s, Hcs, tlist, backward, self._term_rows(self._init_pulses),
                 limit=pk.get("cheby_coeffs_limit", 1e-12), specrange_buffer=pk.get("specrange_buffer", 0.01),
                 specrange_method=pk.get("specrange_method", "auto"), E_min=pk.get("E_min"), E_max=pk.get("E_max"),
                 envelope_cache=shared if self._shared_envelope_ok(pk) else None,
