@@ -53,6 +53,14 @@ enum krotov_gen_format {
 
 enum krotov_direction { KROTOV_FORWARD = 0, KROTOV_BACKWARD = 1 };
 
+enum krotov_propagator { /* krotov_problem.propagator */
+    KROTOV_PROP_CHEBY = 0, /* Chebyshev series (krotov_set_cheby); the default of a zeroed problem              */
+    KROTOV_PROP_EXPMV = 1  /* truncated Taylor series with scaling (krotov_set_taylor): exact for non-Hermitian
+                              generators; persistent one-warp-per-trajectory kernel only (d <= 32, sharded ranks,
+                              at most one trajectory per warp of a co-resident grid: 13 x SMs with rows of <= 12
+                              entries, 7 x SMs with wider ones) */
+};
+
 enum krotov_functional { /* built-in chi = -dJ_T/d<psi| (QuantumControl.Functionals.make_chi analytic forms) */
     KROTOV_CHI_HOST = 0, /* caller supplies chi_k(T) every iteration via krotov_set_chi            */
     KROTOV_CHI_SM = 1,   /* J_T_sm : chi_k = w_k/N^2 (sum_j w_j tau_j) |tgt_k>                     */
@@ -75,7 +83,8 @@ enum krotov_kernel { /* which kernel served the last forward/iterate call (kroto
     KROTOV_KERNEL_DMMA_STREAM = 6,   /* DENSE: one DMMA GEMM launch per Chebyshev term                          */
     KROTOV_KERNEL_DENSE_SWEEP = 7,   /* DENSE: persistent cluster sweep                                         */
     KROTOV_KERNEL_SPARSE_SWEEP = 8,  /* SPARSE: persistent sweep                                                */
-    KROTOV_KERNEL_SPARSE_STREAM = 9  /* SPARSE: one ELL SpMM launch per Chebyshev term                          */
+    KROTOV_KERNEL_SPARSE_STREAM = 9, /* SPARSE: one ELL SpMM launch per Chebyshev term                          */
+    KROTOV_KERNEL_TAYLOR = 10        /* WARP: one trajectory per warp, truncated-Taylor step (KROTOV_PROP_EXPMV)  */
 };
 
 /*
@@ -115,7 +124,10 @@ typedef struct {
                                    is sharded and chi written to every rank over NVLink, the time-serial forward sweep
                                    runs on every rank (no per-step exchange).  Chosen at krotov_comm_connect when every
                                    rank asked for it and runs the persistent kernel with one trajectory per warp. */
-    int32_t reserved[6];
+    int32_t propagator;         /* enum krotov_propagator; 0 = Chebyshev.  KROTOV_PROP_EXPMV on a problem the persistent
+                                   one-warp-per-trajectory kernel does not serve (d > 32, block paths, replicated_forward)
+                                   -> KROTOV_ERR_UNSUPPORTED */
+    int32_t reserved[5];
 } krotov_problem;
 
 typedef struct {
@@ -126,6 +138,7 @@ typedef struct {
     int32_t grid_blocks;     /* CTAs of the persistent kernel                        */
     int32_t block_threads;
     int32_t m_fw;            /* Chebyshev coefficient counts currently loaded (max over generators): forward, */
+                             /* (KROTOV_PROP_EXPMV: the largest m * s, Taylor terms per step; (m - 1) s products) */
     int32_t m_bw;            /* backward */
     int32_t sm_count;
     int32_t exchange;        /* cross-rank protocol of the last launch: 0 none (one rank), 1 hierarchical sum (local
@@ -181,6 +194,23 @@ int64_t krotov_live_device_objects(void);
 int krotov_set_cheby(krotov_handle h, int direction, int n_dt_class, const int32_t *dt_class_of_step,
                      const double *dt_of_class, const double *E_min, const double *Delta, const int32_t *m,
                      const double *coeffs, int m_max);
+
+/* Truncated Taylor series with scaling (Al-Mohy & Higham, SIAM J. Sci. Comput. 33 (2011); the algorithm of
+ * scipy.sparse.linalg.expm_multiply) for handles created with propagator = KROTOV_PROP_EXPMV; the counterpart of
+ * krotov_set_cheby, with the same dt classes.  One interval of generator g and class c applies
+ *     psi <- [ e^{-i mu_g dt/s} sum_{j<m} coeffs[g][c][j] R_g^j ]^s psi,   R_g = -i scale_g (H_g(eps) - mu_g),
+ * with coeffs[j] = (dt / (scale_g s))^j / j! (dt signed as in krotov_set_cheby, H_g the adjoint generator backward):
+ * s times the first m terms of exp(B), B = -i dt/s (H_g - mu_g).  Exact to double-precision backward error for any
+ * generator, Hermitian or not, when (m - 1, s) are chosen for ||B||_1 (the caller's part; theta table of the paper).
+ * A fixed number of products per step, (m - 1) s, without early termination.
+ *   mu, scale : [n_gen]    shift (real; tr(H0)/d is a good choice) and row scale (> 0, e.g. 1/||H - mu||_1)
+ *   s, m      : [n_gen][n_dt_class]   repeats (>= 1) and terms (1 <= m <= m_max)
+ *   coeffs    : [n_gen][n_dt_class][m_max]
+ * KROTOV_ERR_STATE on a Chebyshev handle (and krotov_set_cheby on an Expmv handle); KROTOV_ERR_ARG for m or s out of
+ * range, a scale that is not finite and > 0 or a mu that is not finite. */
+int krotov_set_taylor(krotov_handle h, int direction, int n_dt_class, const int32_t *dt_class_of_step,
+                      const double *dt_of_class, const double *mu, const double *scale, const int32_t *s,
+                      const int32_t *m, const double *coeffs, int m_max);
 
 /* Non-linear control amplitudes.  Replaces what `evaluate(generator, tlist, n; vals_dict)` and `_eval_mu`
  * (src/optimize.jl:268-276, 337-346) do for generators whose control terms carry amplitude objects: control term l

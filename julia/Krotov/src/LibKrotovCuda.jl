@@ -13,6 +13,8 @@ const KROTOV_CHI_HOST, KROTOV_CHI_SM, KROTOV_CHI_SS, KROTOV_CHI_RE = Cint(0), Ci
 const KROTOV_PATH_WARP, KROTOV_PATH_DENSE, KROTOV_PATH_SPARSE = Cint(1), Cint(2), Cint(3)
 const KROTOV_KERNEL_TINY, KROTOV_KERNEL_PREG, KROTOV_KERNEL_SEQ_PREG, KROTOV_KERNEL_PAIR, KROTOV_KERNEL_RELOAD = Cint(1), Cint(2), Cint(3), Cint(4), Cint(5)
 const KROTOV_KERNEL_DMMA_STREAM, KROTOV_KERNEL_DENSE_SWEEP, KROTOV_KERNEL_SPARSE_SWEEP, KROTOV_KERNEL_SPARSE_STREAM = Cint(6), Cint(7), Cint(8), Cint(9)
+const KROTOV_KERNEL_TAYLOR = Cint(10)
+const KROTOV_PROP_CHEBY, KROTOV_PROP_EXPMV = Cint(0), Cint(1)
 const COMM_DESC_BYTES = 256
 
 # mirrors `krotov_problem` field by field
@@ -42,7 +44,8 @@ struct Problem
     device::Int32
     force_path::Int32
     replicated_forward::Int32
-    reserved::NTuple{6,Int32}
+    propagator::Int32
+    reserved::NTuple{5,Int32}
 end
 
 # mirrors `krotov_info` field by field
@@ -113,6 +116,14 @@ set_cheby(h, dir, dtc_of_step::Vector{Int32}, dt_of_class::Vector{Float64}, E_mi
     check(h, ccall((:krotov_set_cheby, lib), Cint,
         (Ptr{Cvoid}, Cint, Cint, Ptr{Int32}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Int32}, Ptr{Float64}, Cint),
         h.ptr, dir, length(dt_of_class), dtc_of_step, dt_of_class, E_min, Delta, m, coeffs, size(coeffs, 1)))
+
+# Taylor settings of a KROTOV_PROP_EXPMV handle: mu, scale: [n_gen]; s, m: [n_dt_class, n_gen];
+# coeffs: [m_max, n_dt_class, n_gen] (column-major == [n_gen][n_dt_class][m_max] on the wire)
+set_taylor(h, dir, dtc_of_step::Vector{Int32}, dt_of_class::Vector{Float64}, mu::Vector{Float64},
+           scale::Vector{Float64}, s::Matrix{Int32}, m::Matrix{Int32}, coeffs::Array{Float64,3}) =
+    check(h, ccall((:krotov_set_taylor, lib), Cint,
+        (Ptr{Cvoid}, Cint, Cint, Ptr{Int32}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Int32}, Ptr{Int32}, Ptr{Float64}, Cint),
+        h.ptr, dir, length(dt_of_class), dtc_of_step, dt_of_class, mu, scale, s, m, coeffs, size(coeffs, 1)))
 
 # non-linear amplitudes a_l(eps, n) = shape[n, l] * sum_p poly[p+1, l] eps^p; poly: Matrix(degree+1, L) or nothing,
 # shape: Matrix(N_T, L) or nothing

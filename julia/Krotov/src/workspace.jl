@@ -295,7 +295,7 @@ function KrotovWrk(problem::QuantumControl.ControlProblem; verbose = false)
             pointer(tlist), pointer(gen_of), C_NULL, C_NULL, Ptr{Float64}(pointer(vals)), pointer(present),
             Ptr{Float64}(pointer(psi0)), have_targets ? Ptr{Float64}(pointer(targets)) : C_NULL, pointer(weights),
             pointer(S), pointer(lambda_vals), chi_kind, 0, store_fw ? 1 : 0, get(kwargs, :device, 0),
-            get(kwargs, :force_path, 0), get(kwargs, :replicated_forward, false) ? 1 : 0, ntuple(_ -> Int32(0), 6)))
+            get(kwargs, :force_path, 0), get(kwargs, :replicated_forward, false) ? 1 : 0, LibKrotovCuda.KROTOV_PROP_CHEBY, ntuple(_ -> Int32(0), 5)))
     end
 
     pk = fw_prop_kwargs[1]

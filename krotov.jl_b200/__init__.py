@@ -15,7 +15,7 @@ from .functionals import J_T_re, J_T_sm, J_T_ss, chi_re, chi_sm, chi_ss, make_ch
 from .generators import (Generator, LogisticParametrization, LogisticSqParametrization, ParametrizedAmplitude,
                          PolynomialAmplitude, ShapedAmplitude, SquareParametrization, TanhParametrization,
                          TanhSqParametrization, hamiltonian)
-from .optimize import (Cheby, Krotov, finalize_result, krotov_initial_fw_prop, krotov_iteration,
+from .optimize import (Cheby, Expmv, Krotov, finalize_result, krotov_initial_fw_prop, krotov_iteration,
                        make_krotov_print_iters, make_print_iters, optimize, optimize_krotov, update_result,
                        update_sigma)
 from .problem import ControlProblem, Trajectory

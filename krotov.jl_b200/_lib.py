@@ -19,16 +19,17 @@ GEN_DENSE_COLMAJOR, GEN_CSR = 0, 1
 FORWARD, BACKWARD = 0, 1
 CHI_HOST, CHI_SM, CHI_SS, CHI_RE = 0, 1, 2, 3
 PATH_WARP, PATH_DENSE, PATH_SPARSE = 1, 2, 3
+PROP_CHEBY, PROP_EXPMV = 0, 1  # enum krotov_propagator (Problem.propagator)
 # enum krotov_kernel (Info.kernel)
 (KERNEL_TINY, KERNEL_PREG, KERNEL_SEQ_PREG, KERNEL_PAIR, KERNEL_RELOAD, KERNEL_DMMA_STREAM, KERNEL_DENSE_SWEEP,
- KERNEL_SPARSE_SWEEP, KERNEL_SPARSE_STREAM) = range(1, 10)
+ KERNEL_SPARSE_SWEEP, KERNEL_SPARSE_STREAM, KERNEL_TAYLOR) = range(1, 11)
 COMM_DESC_BYTES = 256
 
 # every symbol include/krotov_cuda.h declares that returns a status code or a string (tests check the .so exports all
 # of them); krotov_live_device_objects returns a count and is bound below
 EXPORTS = [
     "krotov_abi_version", "krotov_create", "krotov_destroy", "krotov_last_error", "krotov_get_info",
-    "krotov_set_cheby", "krotov_set_amplitudes", "krotov_set_amplitude_saturation", "krotov_set_control_terms", "krotov_forward", "krotov_set_chi", "krotov_set_chi_coeffs", "krotov_iterate",
+    "krotov_set_cheby", "krotov_set_taylor", "krotov_set_amplitudes", "krotov_set_amplitude_saturation", "krotov_set_control_terms", "krotov_forward", "krotov_set_chi", "krotov_set_chi_coeffs", "krotov_iterate",
     "krotov_get_states", "krotov_get_tau", "krotov_get_storage", "krotov_get_profile", "krotov_comm_export", "krotov_comm_connect",
     "krotov_group_connect", "krotov_group_iterate",
     "krotov_hermitian_extremes", "krotov_envelope_extremes", "krotov_envelope_extremes_device",
@@ -50,7 +51,8 @@ class Problem(C.Structure):
         ("gen_values", C.c_void_p), ("term_present", C.c_void_p), ("psi0", C.c_void_p), ("target", C.c_void_p),
         ("weight", C.c_void_p), ("update_shape", C.c_void_p), ("lambda_a", C.c_void_p),
         ("functional", C.c_int32), ("n_traj_global", C.c_int32), ("store_fw", C.c_int32), ("device", C.c_int32),
-        ("force_path", C.c_int32), ("replicated_forward", C.c_int32), ("reserved", C.c_int32 * 6),
+        ("force_path", C.c_int32), ("replicated_forward", C.c_int32), ("propagator", C.c_int32),
+        ("reserved", C.c_int32 * 5),
     ]
 
 
@@ -88,6 +90,7 @@ def lib():
     L.krotov_last_error.restype = C.c_char_p
     L.krotov_get_info.argtypes = [vp, C.POINTER(Info)]
     L.krotov_set_cheby.argtypes = [vp, i32, i32, vp, vp, vp, vp, vp, vp, i32]
+    L.krotov_set_taylor.argtypes = [vp, i32, i32, vp, vp, vp, vp, vp, vp, vp, i32]
     L.krotov_set_amplitudes.argtypes = [vp, i32, vp, vp]
     L.krotov_set_amplitude_saturation.argtypes = [vp, vp]
     L.krotov_set_control_terms.argtypes = [vp, vp]

@@ -26,12 +26,17 @@ void add_warp2_instances(KernelMap &t);         // pair kernel: two trajectories
 void add_warp_instances_rf(KernelMap &t);       // replicated forward sweep of several ranks (one trajectory per warp, d <= 32)
 void add_warp_instances_rf2(KernelMap &t);      // ... one / three controls, runtime L
 void add_warp_instances_rf_emul(KernelMap &t);  // the same with the ranks emulated by one launch
+// truncated-Taylor propagator (prop_method=Expmv), one warp per trajectory: the regular instances into `t`, the
+// emulated-ranks instances into `emul` (maps of their own: the Chebyshev lookups above never see them)
+void add_warp_instances_taylor(KernelMap &t, KernelMap &emul);
 
 #define KR_INST(W, LT, MT) t[KernelKey{W, LT, 32}] = (WarpKernel)krotov_warp_kernel<W, LT, MT>
 #define KR_INSTW(W, LT, MT, LPT) t[KernelKey{W, LT, LPT}] = (WarpKernel)krotov_warp_kernel<W, LT, MT, LPT>
 #define KR_INSTE(W, LT, MT) t[KernelKey{W, LT, 32}] = (WarpKernel)krotov_warp_kernel<W, LT, MT, 32, true>
 #define KR_INSTR(W, LT, MT) t[KernelKey{W, LT, 32}] = (WarpKernel)krotov_warp_kernel<W, LT, MT, 32, false, true>
 #define KR_INSTRE(W, LT, MT) t[KernelKey{W, LT, 32}] = (WarpKernel)krotov_warp_kernel<W, LT, MT, 32, true, true>
+#define KR_INSTT(W, LT, MT) t[KernelKey{W, LT, 32}] = (WarpKernel)krotov_warp_kernel<W, LT, MT, 32, false, false, true>
+#define KR_INSTTE(W, LT, MT) emul[KernelKey{W, LT, 32}] = (WarpKernel)krotov_warp_kernel<W, LT, MT, 32, true, false, true>
 #define KR_INST2(W, LT) t[KernelKey{W, LT, 32}] = (WarpKernel)krotov_warp2_kernel<W, LT>
 
 }  // namespace kr

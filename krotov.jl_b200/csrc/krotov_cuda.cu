@@ -101,6 +101,7 @@ struct krotov_handle_s : HandleStream {
     bool preg = false;
     bool pair = false;  // two trajectories of one generator per warp (warp2_kernel.cuh)
     bool mu_hermitian = false;
+    bool taylor = false;  // krotov_problem.propagator == KROTOV_PROP_EXPMV: cheb[] holds Taylor tables (krotov_set_taylor)
     int lpt = 32;  // threads (= padded rows) per trajectory on the warp path: 32, 64 or 128
     bool tiny = false;  // d <= 4, N <= 32, L <= 2: one thread per trajectory, everything in registers (tiny_kernel.cuh)
     bool tiny_imag[2] = {false, false};  // every prepared term of the direction is purely imaginary (real Hamiltonian)
@@ -254,6 +255,24 @@ const std::map<KernelKey, WarpKernel> &kernel_rf_emul_table() {
         return t;
     }();
     return tab;
+}
+
+// truncated-Taylor instances (prop_method=Expmv): regular and emulated-ranks, in maps of their own
+struct TaylorTables {
+    std::map<KernelKey, WarpKernel> regular, emul;
+};
+const TaylorTables &kernel_taylor_tables() {
+    static const TaylorTables tab = [] {
+        TaylorTables t;
+        kr::add_warp_instances_taylor(t.regular, t.emul);
+        return t;
+    }();
+    return tab;
+}
+
+// the regular instances serving the handle's propagator
+const std::map<KernelKey, WarpKernel> &warp_table(const krotov_handle h) {
+    return h->taylor ? kernel_taylor_tables().regular : kernel_table();
 }
 
 // pair kernel (two trajectories of one generator per warp): register-resident rows only
@@ -595,7 +614,7 @@ int choose_launch(krotov_handle h) {
     const int lpt = h->lpt;
     // groups per CTA (named barriers 3..15); the wide-row instances of one-warp groups are built for 256 threads
     const int cap_preg = (256 - 32) / lpt, cap = (lpt == 32 && h->Wt >= 16) ? 7 : std::min(13, (512 - 32) / lpt);
-    const bool preg_possible = kernel_table().count(KernelKey{h->Wt, h->L, lpt}) > 0;
+    const bool preg_possible = warp_table(h).count(KernelKey{h->Wt, h->L, lpt}) > 0;
     // Pair mode: when there are more trajectories than one-per-warp CTAs with register-resident rows can hold
     // (N > 7 per SM) and they come in generator-sharing pairs (ensembles over basis states), one warp runs two
     // of them interleaved and keeps the rows in registers.  Measured on B200: +19 % at N = 2048 against the
@@ -603,7 +622,7 @@ int choose_launch(krotov_handle h) {
     // with two interleaved recursions (13.7 vs 15.3 ms), so the pair kernel is not used there.
     // KROTOV_NO_PAIR=1 disables it, KROTOV_FORCE_PAIR=1 uses it whenever the pairing exists.
     h->pair = false;
-    if (lpt == 32 && kernel2_table().count(KernelKey{h->Wt, h->L, 32}) > 0 && N % 2 == 0 &&
+    if (lpt == 32 && !h->taylor && kernel2_table().count(KernelKey{h->Wt, h->L, 32}) > 0 && N % 2 == 0 &&
         (N > cap_preg * sm || getenv("KROTOV_FORCE_PAIR")) && N / 2 <= cap_preg * sm &&
         !getenv("KROTOV_NO_PAIR") && !getenv("KROTOV_NO_PREG") && !getenv("KROTOV_SEQ_PREG")) {
         bool ok = true;
@@ -620,7 +639,8 @@ int choose_launch(krotov_handle h) {
     // one warp runs `tpw` trajectories of ONE generator one after the other and keeps that generator's rows in
     // registers, instead of re-reading rows from L2 for every trajectory and time step (21 row loads of 512 bytes
     // per trajectory and step: ~5 TB/s of L2 traffic at N = 4096, which is what bound the row-reloading variant).
-    if (lpt == 32 && preg_possible && N > cap_preg * sm && !getenv("KROTOV_NO_PREG") && !getenv("KROTOV_NO_SEQ_PREG")) {
+    if (lpt == 32 && !h->taylor && preg_possible && N > cap_preg * sm && !getenv("KROTOV_NO_PREG") &&
+        !getenv("KROTOV_NO_SEQ_PREG")) {
         for (int tpw = 2; tpw <= 16; ++tpw) {
             if (N % tpw != 0 || N / tpw > cap_preg * sm) continue;
             bool ok = true;
@@ -666,7 +686,7 @@ void fill_warp_params(krotov_handle h, int mode, kr::WarpParams &p) {
     memset(&p, 0, sizeof(p));
     p.d = h->d; p.N = h->N; p.L = h->L; p.N_T = h->N_T; p.n_gen = h->n_gen;
     p.wpc = h->wpc; p.tpw = h->tpw; p.nCTA = h->nCTA; p.mode = mode; p.store_fw = h->store_fw;
-    p.mu_hermitian = (h->mu_hermitian && !getenv("KROTOV_NO_FAST")) ? 1 : 0;
+    p.mu_hermitian = (h->mu_hermitian && !h->taylor && !getenv("KROTOV_NO_FAST")) ? 1 : 0;
     p.ndtc_f = h->cheb[0].ndtc; p.ndtc_b = h->cheb[1].set ? h->cheb[1].ndtc : 1; p.mmax_f = h->cheb[0].mmax; p.mmax_b = h->cheb[1].set ? h->cheb[1].mmax : 1;
     p.gen_of_traj = h->d_gen.get<const int>();
     p.cols = h->d_cols.get<const int>();
@@ -761,6 +781,7 @@ void fill_warp_params(krotov_handle h, int mode, kr::WarpParams &p) {
 
 // enum krotov_kernel of the persistent warp kernel choose_launch selected (the tiny kernel aside)
 int warp_kernel_kind(const krotov_handle h) {
+    if (h->taylor) return KROTOV_KERNEL_TAYLOR;
     if (h->pair) return KROTOV_KERNEL_PAIR;
     if (h->preg) return h->tpw > 1 ? KROTOV_KERNEL_SEQ_PREG : KROTOV_KERNEL_PREG;
     return KROTOV_KERNEL_RELOAD;
@@ -789,7 +810,7 @@ int launch_warp(krotov_handle h, int mode) {
         return KROTOV_OK;
     }
     KernelKey key{h->Wt, h->preg ? h->L : 0, h->pair ? 32 : h->lpt};
-    const auto &table = h->pair ? kernel2_table() : kernel_table();
+    const auto &table = h->pair ? kernel2_table() : warp_table(h);
     auto it = table.find(key);
     if (it == table.end()) return fail(h, KROTOV_ERR_UNSUPPORTED, "no kernel instance for this (W, L)");
     WarpKernel fn = it->second;
@@ -863,7 +884,13 @@ static int create_handle(krotov_handle h, const krotov_problem *pb) {
     h->N_global = pb->n_traj_global > 0 ? pb->n_traj_global : pb->n_traj;
     h->store_fw = pb->store_fw; h->device = pb->device;
     h->rf_wanted = pb->replicated_forward != 0;
+    if (pb->propagator != KROTOV_PROP_CHEBY && pb->propagator != KROTOV_PROP_EXPMV)
+        return fail(h, KROTOV_ERR_ARG, "unknown krotov_problem.propagator");
+    h->taylor = pb->propagator == KROTOV_PROP_EXPMV;
     const int d = h->d, N = h->N, L = h->L, N_T = h->N_T;
+    if (h->taylor && (d > 32 || (pb->force_path != 0 && pb->force_path != KROTOV_PATH_WARP) || h->rf_wanted))
+        return fail(h, KROTOV_ERR_UNSUPPORTED, "KROTOV_PROP_EXPMV runs on the persistent one-warp-per-trajectory kernel "
+                                               "only (d <= 32, no replicated_forward)");
     if (cudaSetDevice(h->device) != cudaSuccess) return fail(h, KROTOV_ERR_CUDA, "cudaSetDevice failed");
     cudaDeviceProp prop;
     cudaGetDeviceProperties(&prop, h->device);
@@ -999,6 +1026,8 @@ static int create_handle(krotov_handle h, const krotov_problem *pb) {
         }
     }
     h->path = path;
+    if (h->taylor && path != KROTOV_PATH_WARP)
+        return fail(h, KROTOV_ERR_UNSUPPORTED, "KROTOV_PROP_EXPMV: the generator does not fit the persistent warp kernel");
 
     if (path != KROTOV_PATH_SPARSE && h->Hdense.empty()) fill_dense();
 
@@ -1057,7 +1086,11 @@ static int create_handle(krotov_handle h, const krotov_problem *pb) {
             if ((rc = upload(h, h->d_rawb, raw, true))) return rc;
         }
         choose_launch(h);
-        h->tiny = d >= 2 && d <= 4 && N <= 32 && tiny_kernel_for(d, L) != nullptr && !getenv("KROTOV_NO_TINY");
+        if (h->taylor && h->tpw > 1)  // (several trajectories per warp, one after another: not served by the Taylor step)
+            return fail(h, KROTOV_ERR_UNSUPPORTED, "KROTOV_PROP_EXPMV: more trajectories than one per warp of a co-resident "
+                                                   "grid (" + std::to_string(N) + ")");
+        // (the one-thread kernel propagates with the Chebyshev series only: Expmv problems run on the warp kernel)
+        h->tiny = !h->taylor && d >= 2 && d <= 4 && N <= 32 && tiny_kernel_for(d, L) != nullptr && !getenv("KROTOV_NO_TINY");
         // padded state arrays [N][32]
         auto pad_states = [&](const double *src, std::vector<cplx> &dst) {
             dst.assign((size_t)N * h->lpt, cplx(0, 0));
@@ -1187,6 +1220,7 @@ int krotov_set_cheby(krotov_handle h, int direction, int n_dt_class, const int32
     if (direction != KROTOV_FORWARD && direction != KROTOV_BACKWARD) return fail(h, KROTOV_ERR_ARG, "bad direction");
     if (n_dt_class < 1 || !dt_class_of_step || !dt_of_class || !E_min || !Delta || !m || !coeffs || m_max < 1)
         return fail(h, KROTOV_ERR_ARG, "bad argument to krotov_set_cheby");
+    if (h->taylor) return fail(h, KROTOV_ERR_STATE, "the handle propagates with KROTOV_PROP_EXPMV: use krotov_set_taylor");
     Trace tr("set_cheby");
     cudaSetDevice(h->device);
     ChebyTables &ct = h->cheb[direction];
@@ -1273,6 +1307,80 @@ int krotov_set_cheby(krotov_handle h, int direction, int n_dt_class, const int32
     return KROTOV_OK;
 }
 
+int krotov_set_taylor(krotov_handle h, int direction, int n_dt_class, const int32_t *dt_class_of_step,
+                      const double *dt_of_class, const double *mu, const double *scale, const int32_t *s,
+                      const int32_t *m, const double *coeffs, int m_max) {
+    if (!h) return KROTOV_ERR_ARG;
+    if (direction != KROTOV_FORWARD && direction != KROTOV_BACKWARD) return fail(h, KROTOV_ERR_ARG, "bad direction");
+    if (n_dt_class < 1 || !dt_class_of_step || !dt_of_class || !mu || !scale || !s || !m || !coeffs || m_max < 1)
+        return fail(h, KROTOV_ERR_ARG, "bad argument to krotov_set_taylor");
+    if (!h->taylor) return fail(h, KROTOV_ERR_STATE, "krotov_set_taylor needs a handle created with KROTOV_PROP_EXPMV");
+    cudaSetDevice(h->device);
+    for (int n = 0; n < h->N_T; ++n)
+        if (dt_class_of_step[n] < 0 || dt_class_of_step[n] >= n_dt_class)
+            return fail(h, KROTOV_ERR_ARG, "dt_class_of_step out of range");
+    for (int c = 0; c < n_dt_class; ++c) {
+        if (direction == KROTOV_FORWARD && !(dt_of_class[c] > 0)) return fail(h, KROTOV_ERR_ARG, "forward dt must be > 0");
+        if (direction == KROTOV_BACKWARD && !(dt_of_class[c] < 0)) return fail(h, KROTOV_ERR_ARG, "backward dt must be < 0");
+    }
+    const int n_gen = h->n_gen;
+    for (int g = 0; g < n_gen; ++g) {
+        if (!(std::isfinite(scale[g]) && scale[g] > 0)) return fail(h, KROTOV_ERR_ARG, "scale must be finite and > 0");
+        if (!std::isfinite(mu[g])) return fail(h, KROTOV_ERR_ARG, "mu must be finite");
+        for (int c = 0; c < n_dt_class; ++c) {
+            const size_t i = (size_t)g * n_dt_class + c;
+            if (m[i] < 1 || m[i] > m_max) return fail(h, KROTOV_ERR_ARG, "m out of range");
+            if (s[i] < 1) return fail(h, KROTOV_ERR_ARG, "s must be >= 1");
+        }
+    }
+    // the tables of krotov_set_cheby, with (m, s) pairs in the count table and the phase of one repeat
+    ChebyTables &ct = h->cheb[direction];
+    ct.ndtc = n_dt_class;
+    ct.mmax = m_max;
+    ct.m_host.resize((size_t)2 * n_gen * n_dt_class);
+    ct.phase_host.resize((size_t)n_gen * n_dt_class);
+    ct.m_max_used = 0;
+    for (int g = 0; g < n_gen; ++g)
+        for (int c = 0; c < n_dt_class; ++c) {
+            const size_t i = (size_t)g * n_dt_class + c;
+            ct.m_host[2 * i] = m[i];
+            ct.m_host[2 * i + 1] = s[i];
+            ct.m_max_used = (int)std::min<long long>(INT32_MAX, std::max<long long>(ct.m_max_used, (long long)m[i] * s[i]));
+            ct.phase_host[i] = std::exp(cplx(0.0, -mu[g] * dt_of_class[c] / s[i]));
+        }
+    ct.coef_host.assign(coeffs, coeffs + (size_t)n_gen * n_dt_class * m_max);
+    ct.dtc_of_step.assign(dt_class_of_step, dt_class_of_step + h->N_T);
+    int rc;
+    if ((rc = upload(h, ct.dtc, ct.dtc_of_step, false))) return rc;
+    if ((rc = upload(h, ct.coef, ct.coef_host, false))) return rc;
+    if ((rc = upload(h, ct.m, ct.m_host, false))) return rc;
+    if ((rc = upload(h, ct.phase, ct.phase_host, true))) return rc;  // (waits for all four: the next call rewrites ct)
+    ct.set = true;
+    // R_t = -i scale_g (H_t - mu_g delta_t0) in both directions (the backward rows hold the adjoint generator and the
+    // coefficients carry the negative dt): scale_rows_kernel with (fy, beta) = (-scale_g, mu_g)
+    std::vector<double> fb((size_t)2 * n_gen);
+    for (int g = 0; g < n_gen; ++g) {
+        fb[2 * g] = -scale[g];
+        fb[2 * g + 1] = mu[g];
+    }
+    if ((rc = upload(h, h->d_rowscale, fb, true))) return rc;
+    DevBuf &dP = direction == KROTOV_FORWARD ? h->d_Pf : h->d_Pb;
+    const DevBuf &raw = direction == KROTOV_FORWARD ? h->d_rawf : h->d_rawb;
+    const size_t total = (size_t)n_gen * (1 + h->L) * (h->Wt + 1) * h->lpt;
+    if ((rc = dev_alloc(h, dP, total * 16))) return rc;
+    scale_rows_kernel<<<(unsigned)((total + 255) / 256), 256, 0, h->stream>>>(
+        raw.get<const double2>(), h->d_rowscale.get<const double2>(), dP.get<double2>(), 1 + h->L, h->Wt, h->lpt, h->d, total);
+    KR_CUDA(h, cudaStreamSynchronize(h->stream));  // the next call may rewrite d_rowscale
+    KR_CUDA(h, cudaGetLastError());
+    h->launches_total += 1;
+    if (direction == KROTOV_FORWARD) {  // overlaps: Im<chi|H_l|psi> = Re<chi|R_l psi> / scale
+        std::vector<double> inv_s(n_gen);
+        for (int g = 0; g < n_gen; ++g) inv_s[g] = 1.0 / scale[g];
+        if ((rc = upload(h, h->d_inv_s, inv_s, true))) return rc;
+    }
+    return KROTOV_OK;
+}
+
 // a_l(eps_old) and a_l'(eps_old) for the pulses of the coming sweep: O(L N_T) host work, uploaded on the launch stream
 static int prepare_amplitudes(krotov_handle h, const double *pulses) {
     if (!h->amp_set) return KROTOV_OK;
@@ -1349,7 +1457,9 @@ static int end_timed(krotov_handle h) {
 
 int krotov_forward(krotov_handle h, const double *pulses) {
     if (!h || !pulses) return KROTOV_ERR_ARG;
-    if (!h->cheb[0].set) return fail(h, KROTOV_ERR_STATE, "krotov_set_cheby(FORWARD) must be called before krotov_forward");
+    if (!h->cheb[0].set)
+        return fail(h, KROTOV_ERR_STATE, h->taylor ? "krotov_set_taylor(FORWARD) must be called before krotov_forward"
+                                                   : "krotov_set_cheby(FORWARD) must be called before krotov_forward");
     cudaSetDevice(h->device);
     KR_CUDA(h, cudaMemcpyAsync(h->d_eps_old.get<void>(), pulses, (size_t)h->L * h->N_T * 8, cudaMemcpyHostToDevice, h->stream));
     int rc;
@@ -1404,7 +1514,8 @@ int krotov_set_chi_coeffs(krotov_handle h, const double *coef) {
 // exchange arrays reset.  Leaves the timed region open (begin_timed).
 static int iterate_prepare(krotov_handle h, const double *guess_pulses) {
     if (!h->cheb[0].set || !h->cheb[1].set)
-        return fail(h, KROTOV_ERR_STATE, "krotov_set_cheby must be called for both directions before krotov_iterate");
+        return fail(h, KROTOV_ERR_STATE, h->taylor ? "krotov_set_taylor must be called for both directions before krotov_iterate"
+                                                   : "krotov_set_cheby must be called for both directions before krotov_iterate");
     cudaSetDevice(h->device);
     const bool need_device_coef = !h->chiT_valid && !h->chicoef_valid;
     if (need_device_coef) {
@@ -1534,7 +1645,8 @@ int krotov_group_connect(krotov_handle *hs, int world) {
         if (h->path != KROTOV_PATH_WARP || h->pair || (h->tiny && world == 1))
             return fail(h, KROTOV_ERR_UNSUPPORTED, "krotov_group_connect: warp path (one trajectory per warp) only");
         if (h->device != hs[0]->device || h->L != hs[0]->L || h->N_T != hs[0]->N_T || h->Wt != hs[0]->Wt ||
-            h->lpt != hs[0]->lpt || h->preg != hs[0]->preg || h->wpc != hs[0]->wpc || h->tpw != hs[0]->tpw)
+            h->lpt != hs[0]->lpt || h->preg != hs[0]->preg || h->wpc != hs[0]->wpc || h->tpw != hs[0]->tpw ||
+            h->taylor != hs[0]->taylor)
             return fail(h, KROTOV_ERR_ARG, "krotov_group_connect: ranks must share device, grid shape and kernel instance");
         total += h->nCTA;
         mx = std::max(mx, h->nCTA);
@@ -1604,8 +1716,9 @@ int krotov_group_iterate(krotov_handle *hs, int world, const double *guess_pulse
     p0.emul_ranks = world;
     p0.wpc = h0->wpc;
     const KernelKey key{h0->Wt, h0->preg ? h0->L : 0, h0->lpt};
-    auto it = kernel_emul_table().find(key);
-    if (it == kernel_emul_table().end())
+    const auto &emul_table = h0->taylor ? kernel_taylor_tables().emul : kernel_emul_table();
+    auto it = emul_table.find(key);
+    if (it == emul_table.end())
         return fail(h0, KROTOV_ERR_UNSUPPORTED, "no emulated-ranks instance of this kernel (W, L)");
     size_t smem = 0;
     for (int r = 0; r < world; ++r) smem = std::max(smem, warp_smem_bytes(hs[r]));

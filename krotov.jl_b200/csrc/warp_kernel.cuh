@@ -269,6 +269,93 @@ __device__ __forceinline__ StepMeta load_meta(const int *dtc, const int *m_tab, 
     return s;
 }
 
+// One truncated-Taylor step with scaling (Al-Mohy & Higham 2011; prop_method=Expmv): the rows g hold
+// R = -i scale (H(eps) - mu) and a[j] = (dt / (scale s))^j / j!, so that each of the s repeats applies
+//   v <- e^{-i mu dt/s} sum_{j<m} a_j R^j v  =  e^{-i mu dt/s} sum_{j<m} B^j / j! v,   B = -i dt/s (H - mu).
+// m and s are fixed per (generator, dt class): (m-1) s products, no early termination, so the instruction stream and
+// the bits are the same on every CTA and rank.  Same buffers as cheby_step: v0buf holds psi (written + synced by the
+// caller); every product reads the buffer written behind the previous one and writes the other.
+template <int W, int LPT = 32>
+__device__ __forceinline__ double2 taylor_step(const double2 psi, const double2 (&g)[W + 1], const int (&col)[W],
+                                               const double2 *v0buf, double2 *bufA, double2 *bufB,
+                                               const double *__restrict__ a, const int m, const int s,
+                                               const double2 phase, const int lane, const int bar_id = 0) {
+    double2 v = psi;
+    const double2 *cur = v0buf;
+    double2 *nxt = bufB, *oth = bufA;
+    for (int r = 0; r < s; ++r) {
+        const double a0 = a[0];
+        double outr = a0 * v.x, outi = a0 * v.y;
+        double2 vj = v;
+        for (int j = 1; j < m; ++j) {
+            double ar = 0.0, ai = 0.0;
+            row_dot<W>(g, col, cur, vj, ar, ai);
+            const double aj = a[j];
+            outr = fma(aj, ar, outr);
+            outi = fma(aj, ai, outi);
+            vj = make_double2(ar, ai);
+            // behind the last product of a repeat the buffer takes the next repeat's input
+            if (j + 1 == m) vj = make_double2(phase.x * outr - phase.y * outi, phase.x * outi + phase.y * outr);
+            double2 *const w = nxt;
+            w[lane] = vj;
+            grp_sync<LPT>(bar_id);
+            cur = w;
+            nxt = oth;
+            oth = w;
+        }
+        v = (m > 1) ? vj : make_double2(phase.x * outr - phase.y * outi, phase.x * outi + phase.y * outr);
+    }
+    return v;
+}
+
+// Taylor tables: m_tab holds (m, s) per (generator, dt class)
+struct TaylorMeta {
+    int m, s;
+    double2 phase;
+    const double *a;
+};
+__device__ __forceinline__ TaylorMeta load_meta_taylor(const int *dtc, const int *ms_tab, const double2 *ph_tab,
+                                                       const double *coef, int ndtc, int mmax, int gi, int n) {
+    const int ci = gi * ndtc + dtc[n];
+    TaylorMeta s;
+    const int2 ms = reinterpret_cast<const int2 *>(ms_tab)[ci];
+    s.m = ms.x;
+    s.s = ms.y;
+    s.phase = ph_tab[ci];
+    s.a = coef + (size_t)ci * mmax;
+    return s;
+}
+
+// the step of the kernel's propagator: Chebyshev (StepMeta) or Taylor (TaylorMeta)
+template <bool TAYLOR>
+struct Prop {
+    using Meta = StepMeta;
+    static __device__ __forceinline__ Meta load(const int *dtc, const int *m_tab, const double2 *ph_tab, const double *coef,
+                                                int ndtc, int mmax, int gi, int n) {
+        return load_meta(dtc, m_tab, ph_tab, coef, ndtc, mmax, gi, n);
+    }
+    template <int W, int LPT>
+    static __device__ __forceinline__ double2 step(const double2 psi, const double2 (&g)[W + 1], const int (&col)[W],
+                                                   const double2 *v0buf, double2 *bufA, double2 *bufB, const Meta &mt,
+                                                   const int lane, const int bar_id) {
+        return cheby_step<W, LPT>(psi, g, col, v0buf, bufA, bufB, mt.a, mt.m, mt.phase, lane, bar_id);
+    }
+};
+template <>
+struct Prop<true> {
+    using Meta = TaylorMeta;
+    static __device__ __forceinline__ Meta load(const int *dtc, const int *m_tab, const double2 *ph_tab, const double *coef,
+                                                int ndtc, int mmax, int gi, int n) {
+        return load_meta_taylor(dtc, m_tab, ph_tab, coef, ndtc, mmax, gi, n);
+    }
+    template <int W, int LPT>
+    static __device__ __forceinline__ double2 step(const double2 psi, const double2 (&g)[W + 1], const int (&col)[W],
+                                                   const double2 *v0buf, double2 *bufA, double2 *bufB, const Meta &mt,
+                                                   const int lane, const int bar_id) {
+        return taylor_step<W, LPT>(psi, g, col, v0buf, bufA, bufB, mt.a, mt.m, mt.s, mt.phase, lane, bar_id);
+    }
+};
+
 // Same recursion, but the first term v_1 = G v_0 / 2 was assembled by the caller from products that do not
 // depend on the pulse value (computed while the warp waited for the grid-wide sum).
 template <int W, int LPT = 32>
@@ -1075,9 +1162,11 @@ struct RfProducer<true> {
 
 // RF: instance with the replicated forward sweep of several ranks compiled in (sharded backward sweep, forwarder warps, rank
 // barrier); the regular instances carry none of it (at 254 registers per thread every extra live value costs the sweeps).
+// TAYLOR: the step is taylor_step (prop_method=Expmv; WarpParams::m_f / m_b then hold (m, s) pairs) instead of cheby_step.
 template <int W, int LT /*0 = runtime L, rows reloaded from L1/L2 per use*/, int MAXTHREADS, int LPT = 32, bool EMUL = false,
-          bool RF = false>
+          bool RF = false, bool TAYLOR = false>
 __global__ void __launch_bounds__(MAXTHREADS, 1) krotov_warp_kernel(const __grid_constant__ WarpParams p0) {
+    using Step = Prop<TAYLOR>;
     const WarpParams &p = select_params<EMUL>(p0);
     const int cta = EMUL ? (int)blockIdx.x - p.cta_base : (int)blockIdx.x;
     constexpr bool PREG = (LT > 0);
@@ -1185,13 +1274,13 @@ __global__ void __launch_bounds__(MAXTHREADS, 1) krotov_warp_kernel(const __grid
                 mypsi[t * LPT + lane] = chi;
                 grp_sync<LPT>(gbar);
             }
-            StepMeta meta = load_meta(p.dtc_b, p.m_b, p.phase_b, p.coef_b, p.ndtc_b, p.mmax_b, gi, N_T - 1);
+            typename Step::Meta meta = Step::load(p.dtc_b, p.m_b, p.phase_b, p.coef_b, p.ndtc_b, p.mmax_b, gi, N_T - 1);
             double e_cur[kMaxCtrl];
 #pragma unroll
             for (int l = 0; l < kMaxCtrl; ++l) e_cur[l] = (l < L) ? p.amp_old[(size_t)l * N_T + N_T - 1] : 0.0;
             for (int n = N_T - 1; n >= 0; --n) {
                 const int nn = n > 0 ? n - 1 : 0;  // prefetch the next step's metadata and pulse values
-                const StepMeta meta_next = load_meta(p.dtc_b, p.m_b, p.phase_b, p.coef_b, p.ndtc_b, p.mmax_b, gi, nn);
+                const typename Step::Meta meta_next = Step::load(p.dtc_b, p.m_b, p.phase_b, p.coef_b, p.ndtc_b, p.mmax_b, gi, nn);
                 double e_next[kMaxCtrl];
 #pragma unroll
                 for (int l = 0; l < kMaxCtrl; ++l) e_next[l] = (l < L) ? p.amp_old[(size_t)l * N_T + nn] : 0.0;
@@ -1222,9 +1311,9 @@ __global__ void __launch_bounds__(MAXTHREADS, 1) krotov_warp_kernel(const __grid
                 }
                 if constexpr (RF) {
                     rfp.peek();  // (consumer's progress: used when the next record is put)
-                    chi = cheby_step<W, LPT>(chi, g, col, rfp.v0, bufA, bufB, meta.a, meta.m, meta.phase, lane, gbar);
+                    chi = Step::template step<W, LPT>(chi, g, col, rfp.v0, bufA, bufB, meta, lane, gbar);
                 } else {
-                    chi = cheby_step<W, LPT>(chi, g, col, mypsi + t * LPT, bufA, bufB, meta.a, meta.m, meta.phase, lane, gbar);
+                    chi = Step::template step<W, LPT>(chi, g, col, mypsi + t * LPT, bufA, bufB, meta, lane, gbar);
                 }
                 meta = meta_next;
 #pragma unroll
@@ -1271,7 +1360,7 @@ __global__ void __launch_bounds__(MAXTHREADS, 1) krotov_warp_kernel(const __grid
         for (int q = 0; q < NT; ++q) load_row<W, LPT>(Pg + q * rowstride, P[q], lane);
     }
     const double inv_s0 = (k0 < p.N) ? p.inv_s_f[g0] : 0.0;
-    StepMeta fmeta = load_meta(p.dtc_f, p.m_f, p.phase_f, p.coef_f, p.ndtc_f, p.mmax_f, g0, 0);
+    typename Step::Meta fmeta = Step::load(p.dtc_f, p.m_f, p.phase_f, p.coef_f, p.ndtc_f, p.mmax_f, g0, 0);
     double2 chi_next = make_double2(0.0, 0.0);
     if (p.mode == 1 && k0 < p.N) chi_next = p.X[(size_t)k0 * (N_T + 1) * LPT + lane];
     // FAST: register-resident rows, one trajectory per warp, Hermitian control terms.  Then
@@ -1279,7 +1368,7 @@ __global__ void __launch_bounds__(MAXTHREADS, 1) krotov_warp_kernel(const __grid
     // so xi_l = P_l chi(t_n) can be formed BEFORE psi(t_n) exists, and the overlap on the critical path is a
     // plain dot product; and the products w_t = P_t psi(t_n) that make up the first Chebyshev term
     // v_1 = (w_0 + sum_l eps_l w_l) / 2 are formed while the warp waits for eps.
-    const bool FAST = PREG && tpw == 1 && p.mode == 1 && p.mu_hermitian != 0;
+    const bool FAST = !TAYLOR && PREG && tpw == 1 && p.mode == 1 && p.mu_hermitian != 0;
     double2 *chibuf = chibufs + (size_t)warp * LPT;
     double2 xi[PREG ? (LT > 0 ? LT : 1) : 1];
     double2 wv[PREG ? NT : 1];
@@ -1373,13 +1462,13 @@ __global__ void __launch_bounds__(MAXTHREADS, 1) krotov_warp_kernel(const __grid
                 if (l < L) eps[l] = p.amp_old[(size_t)l * N_T + n];
         }
         // ---- forward step with the (updated) pulse value  (src/optimize.jl:360-368)
-        const StepMeta fmeta_next =
-            load_meta(p.dtc_f, p.m_f, p.phase_f, p.coef_f, p.ndtc_f, p.mmax_f, g0, n + 1 < N_T ? n + 1 : n);
+        const typename Step::Meta fmeta_next =
+            Step::load(p.dtc_f, p.m_f, p.phase_f, p.coef_f, p.ndtc_f, p.mmax_f, g0, n + 1 < N_T ? n + 1 : n);
         for (int t = 0; t < tpw; ++t) {
             const int k = kbase + t;
             if (k >= p.N) break;
             const int gi = (t == 0) ? g0 : p.gen_of_traj[k];
-            const StepMeta sm = (t == 0) ? fmeta : load_meta(p.dtc_f, p.m_f, p.phase_f, p.coef_f, p.ndtc_f, p.mmax_f, gi, n);
+            const typename Step::Meta sm = (t == 0) ? fmeta : Step::load(p.dtc_f, p.m_f, p.phase_f, p.coef_f, p.ndtc_f, p.mmax_f, gi, n);
             if (PREG) {
 #pragma unroll
                 for (int s = 0; s <= W; ++s) g[s] = P[0][s];
@@ -1405,7 +1494,7 @@ __global__ void __launch_bounds__(MAXTHREADS, 1) krotov_warp_kernel(const __grid
                 }
             }
             double2 psi = (tpw == 1) ? psi_reg : mypsi[t * LPT + lane];
-            if (PREG && FAST) {
+            if (PREG && FAST) {  // (never in the TAYLOR instances)
                 double v1r = wv[0].x, v1i = wv[0].y;
 #pragma unroll
                 for (int l = 0; l < NT - 1; ++l) {
@@ -1415,7 +1504,7 @@ __global__ void __launch_bounds__(MAXTHREADS, 1) krotov_warp_kernel(const __grid
                 psi = cheby_step_from_v1<W, LPT>(psi, make_double2(0.5 * v1r, 0.5 * v1i), g, col, bufA, bufB, sm.a, sm.m,
                                             sm.phase, lane, gbar);
             } else {
-                psi = cheby_step<W, LPT>(psi, g, col, mypsi + t * LPT, bufA, bufB, sm.a, sm.m, sm.phase, lane, gbar);
+                psi = Step::template step<W, LPT>(psi, g, col, mypsi + t * LPT, bufA, bufB, sm, lane, gbar);
             }
             mypsi[t * LPT + lane] = psi;
             if (t == 0) psi_reg = psi;

@@ -18,7 +18,7 @@ def _ptr(a):
 class KrotovCuda:
     def __init__(self, *, tlist, H0, Hc, gen_of_traj, psi0, target=None, weight=None, update_shape, lambda_a,
                  functional=B.CHI_HOST, n_traj_global=0, store_fw=False, device=0, force_path=0, csr=False,
-                 replicated_forward=False):
+                 replicated_forward=False, propagator=B.PROP_CHEBY):
         """H0: (n_gen, d, d) complex, Hc: (n_gen, L, d, d) complex with ``None`` entries allowed
         (as zeros + term_present=0); psi0/target: (N, d); update_shape: (L, N_T); lambda_a: (L,)."""
         lib = B.lib()
@@ -92,6 +92,7 @@ class KrotovCuda:
         p.functional, p.n_traj_global = int(functional), int(n_traj_global)
         p.store_fw, p.device, p.force_path = int(bool(store_fw)), int(device), int(force_path)
         p.replicated_forward = int(bool(replicated_forward))
+        p.propagator = int(propagator)
         rc = lib.krotov_create(C.byref(p), C.byref(self._h))
         if rc != B.KROTOV_OK:
             msg = lib.krotov_last_error(None).decode()
@@ -132,6 +133,20 @@ class KrotovCuda:
         Dl = np.ascontiguousarray(Delta, np.float64).reshape(n_gen)
         self._check(self._lib.krotov_set_cheby(self._h, int(direction), ndtc, _ptr(dtc), _ptr(dts), _ptr(Emin),
                                                _ptr(Dl), _ptr(m), _ptr(tab), m_max))
+
+    def set_taylor(self, direction, dt_class_of_step, dt_of_class, mu, scale, s, m, tab):
+        """Taylor settings of a ``propagator=PROP_EXPMV`` handle (``krotov_set_taylor``): mu, scale: (n_gen,); s, m:
+        (n_gen, n_dt_class) repeats and terms; tab: (n_gen, n_dt_class, m_max) zero-padded coefficients."""
+        n_gen, ndtc = self.n_gen, len(dt_of_class)
+        s = np.ascontiguousarray(s, np.int32).reshape(n_gen, ndtc)
+        m = np.ascontiguousarray(m, np.int32).reshape(n_gen, ndtc)
+        tab = np.ascontiguousarray(tab, np.float64).reshape(n_gen, ndtc, -1)
+        dtc = np.ascontiguousarray(dt_class_of_step, np.int32)
+        dts = np.ascontiguousarray(dt_of_class, np.float64)
+        mu = np.ascontiguousarray(mu, np.float64).reshape(n_gen)
+        sc = np.ascontiguousarray(scale, np.float64).reshape(n_gen)
+        self._check(self._lib.krotov_set_taylor(self._h, int(direction), ndtc, _ptr(dtc), _ptr(dts), _ptr(mu), _ptr(sc),
+                                                _ptr(s), _ptr(m), _ptr(tab), int(tab.shape[2])))
 
     def set_amplitudes(self, poly=None, shape=None):
         """Non-linear amplitudes ``a_l(eps, n) = shape[l][n] * sum_p poly[l][p] eps^p`` (``krotov_set_amplitudes``);
@@ -266,6 +281,11 @@ class KrotovCudaGroup:
         m, tab = np.asarray(m), np.asarray(tab)
         for e, g in zip(self.engines, self.gens):
             e.set_cheby(direction, dt_class_of_step, dt_of_class, E_min[g], Delta[g], m[g], tab[g])  # (replicated: g = all)
+
+    def set_taylor(self, direction, dt_class_of_step, dt_of_class, mu, scale, s, m, tab):
+        mu, scale, s, m, tab = (np.asarray(a) for a in (mu, scale, s, m, tab))
+        for e, g in zip(self.engines, self.gens):
+            e.set_taylor(direction, dt_class_of_step, dt_of_class, mu[g], scale[g], s[g], m[g], tab[g])
 
     def set_amplitudes(self, poly=None, shape=None):
         for e in self.engines:

@@ -28,7 +28,7 @@ from .workspace import KrotovWrk
 log = logging.getLogger("krotov_jl_b200")
 
 __all__ = ["optimize", "optimize_krotov", "krotov_initial_fw_prop", "krotov_iteration", "update_result", "update_sigma",
-           "finalize_result", "detached_result", "make_krotov_print_iters", "make_print_iters", "Krotov", "Cheby"]
+           "finalize_result", "detached_result", "make_krotov_print_iters", "make_print_iters", "Krotov", "Cheby", "Expmv"]
 
 
 class _Method:
@@ -41,6 +41,7 @@ class _Method:
 
 Krotov = _Method("Krotov")  # `optimize(problem; method=Krotov)`
 Cheby = _Method("Cheby")  # `prop_method=Cheby`
+Expmv = _Method("Expmv")  # `prop_method=Expmv`: truncated Taylor series with scaling (expmv.py), any generator
 
 
 # --------------------------------------------------------------------------------------------

@@ -20,6 +20,7 @@ import numpy as np
 
 from . import _lib as B
 from .cheby import ChebyDirection
+from .expmv import TaylorDirection
 from .controls import discretize_on_midpoints, get_control_derivs, get_control_terms, get_controls
 from .engine import KrotovCuda
 from .errors import ArgumentError, ErrorException
@@ -109,6 +110,7 @@ def _takes_tau(fn):
 
 
 _CHEBY_NAMES = {"cheby", "Cheby", ":Cheby", ":cheby"}
+_EXPMV_NAMES = {"expmv", "Expmv", ":Expmv", ":expmv"}
 
 
 def _is_cheby(method):
@@ -117,6 +119,13 @@ def _is_cheby(method):
     if isinstance(method, str):
         return method in _CHEBY_NAMES
     return getattr(method, "__name__", "").split(".")[-1] in _CHEBY_NAMES
+
+
+def _is_expmv(method):
+    if method is None:
+        return False
+    name = method if isinstance(method, str) else getattr(method, "__name__", "").split(".")[-1]
+    return name in _EXPMV_NAMES
 
 
 def _prop_kwargs(traj, kwargs, prefixes):
@@ -288,10 +297,11 @@ class KrotovWrk:
         for pk in self.fw_prop_kwargs + self.bw_prop_kwargs:
             if "method" not in pk:
                 raise ArgumentError("The propagation method must be specified (`prop_method=Cheby`)")
-            if not _is_cheby(pk["method"]):
+            if not (_is_cheby(pk["method"]) or _is_expmv(pk["method"])):
                 raise ArgumentError(
-                    f"prop_method={pk['method']!r}: libkrotov_cuda serves the `Cheby` propagator only "
-                    "(there is no CPU fallback for other methods)")
+                    f"prop_method={pk['method']!r}: libkrotov_cuda serves the `Cheby` propagator and `Expmv` (truncated "
+                    "Taylor series, exact for non-Hermitian generators such as Liouvillians) only; there is no CPU "
+                    "fallback for other methods")
             if "callback" in pk:
                 raise ArgumentError("per-step propagation callbacks cannot run inside the device sweep")
         for name, pks in (("fw", self.fw_prop_kwargs), ("bw", self.bw_prop_kwargs)):
@@ -301,6 +311,11 @@ class KrotovWrk:
                 if _comparable(pk) != _comparable(pks[0]):
                     raise ArgumentError(f"{name}_prop_kwargs differ between trajectories; the batched device "
                                         "propagator needs the same propagator settings for all of them")
+        # both directions run in one persistent kernel, which carries one propagator
+        self._expmv = _is_expmv(self.fw_prop_kwargs[0]["method"])
+        if self._expmv != _is_expmv(self.bw_prop_kwargs[0]["method"]):
+            raise ArgumentError("the forward and backward propagators must use the same method (`Cheby` or `Expmv`): "
+                                f"got fw {self.fw_prop_kwargs[0]['method']!r}, bw {self.bw_prop_kwargs[0]['method']!r}")
         if "J_T" not in kwargs:
             raise ArgumentError("`optimize` for `method=Krotov` must be passed the functional `J_T`.")
         J_T = kwargs["J_T"]
@@ -400,10 +415,24 @@ class KrotovWrk:
         return saturated_corners(self._amp_poly[l] if self._amp_poly is not None else [0.0, 1.0], s, lo, hi,
                                  None if self._amp_shape is None else float(np.max(np.abs(self._amp_shape[l]))))
 
+    def _amp_abs_max(self, l, lo, hi):
+        """Largest |coefficient of H_l| over the control range [lo, hi] (the Taylor norm bound): the corners of
+        ``_amp_envelope_corners`` and, for a polynomial amplitude, its value at every critical point inside the range."""
+        v = max(abs(c) for c in self._amp_envelope_corners(l, lo, hi))
+        if self._amp_poly is not None and (self._amp_sat is None or self._amp_sat[l] == 0.0):
+            q = np.polynomial.Polynomial(self._amp_poly[l])
+            shp = 1.0 if self._amp_shape is None else float(np.max(np.abs(self._amp_shape[l])))
+            for x in q.deriv().roots():
+                if abs(x.imag) < 1e-12 and lo <= x.real <= hi:
+                    v = max(v, shp * abs(q(x.real)))
+        return v
+
     def _build_device_side(self, tlist, comm):
         trajs = self.trajectories
         N, L = self.N, len(self._terms)  # (the device counts control terms)
         d = trajs[0].initial_state.shape[0]
+        if self._expmv and d > 32:
+            raise ArgumentError(f"prop_method=Expmv runs on the one-warp-per-trajectory kernel, d <= 32 (got d = {d})")
         # distinct generators by identity: ensemble members sharing a Hamiltonian share its storage
         gen_ids, gens, gen_of_traj = {}, [], np.zeros(N, np.int32)
         for k, t in enumerate(trajs):
@@ -450,10 +479,12 @@ class KrotovWrk:
         n_ranks_wanted = max(world, int(self.kwargs.get("emulate_ranks", 0) or 0))
         any_sparse = any(hasattr(m, "tocsr") for m in H0)
         if mode == "auto":
-            mode = "replicate" if (n_ranks_wanted > 1 and d <= 32 and N <= 7 * 148 and not any_sparse and
-                                   int(self.kwargs.get("force_path", 0)) in (0, 1)) else "shard"
+            mode = "replicate" if (n_ranks_wanted > 1 and d <= 32 and N <= 7 * 148 and not any_sparse and not self._expmv
+                                   and int(self.kwargs.get("force_path", 0)) in (0, 1)) else "shard"
         if mode not in ("shard", "replicate"):
             raise ArgumentError(f"multi_gpu={mode!r}: expected 'auto', 'shard' or 'replicate'")
+        if self._expmv and mode == "replicate":
+            raise ArgumentError("prop_method=Expmv has no replicated forward sweep: use multi_gpu='shard' (or 'auto')")
         self._replicated = mode == "replicate" and n_ranks_wanted > 1
 
         def make_engine(lo, hi):
@@ -465,7 +496,8 @@ class KrotovWrk:
                 psi0=psi0[lo:hi], target=None if target is None else target[lo:hi], weight=weight[lo:hi],
                 update_shape=S, lambda_a=lam, functional=functional, n_traj_global=N,
                 store_fw=self.store_fw, device=device, force_path=int(self.kwargs.get("force_path", 0)),
-                csr=bool(self.kwargs.get("csr_generators", False)), replicated_forward=self._replicated)
+                csr=bool(self.kwargs.get("csr_generators", False)), replicated_forward=self._replicated,
+                propagator=B.PROP_EXPMV if self._expmv else B.PROP_CHEBY)
             return eng, local_gens
 
         emulate = int(self.kwargs.get("emulate_ranks", 0) or 0)
@@ -497,7 +529,7 @@ class KrotovWrk:
             self.engine.set_amplitudes(self._amp_poly, self._amp_shape)
         if self._amp_sat is not None:
             self.engine.set_amplitude_saturation(self._amp_sat)
-        # ---- Chebyshev settings of both directions (init_prop: un-widened ranges of the guess pulses)
+        # ---- propagator settings of both directions (Chebyshev or Taylor) (init_prop: un-widened ranges of the guess pulses)
         adj = lambda m: m.conj().T.tocsr() if hasattr(m, "tocsr") else m.conj().T  # noqa: E731
         same = lambda a, b: (abs(a - b).max() == 0) if hasattr(a, "tocsr") else np.array_equal(a, b)  # noqa: E731
         terms = list(self._H0) + [h for row in self._Hc for h in row if h is not None]
@@ -518,6 +550,9 @@ class KrotovWrk:
         def settings(pk, backward):
             H0s = [adj(h) for h in self._H0] if backward else self._H0
             Hcs = [[None if h is None else adj(h) for h in row] for row in self._Hc] if backward else self._Hc
+            if self._expmv:
+                return TaylorDirection(H0s, Hcs, tlist, backward, self._term_rows(self._init_pulses),
+                                       amplitude_max=self._amp_abs_max if nonlinear else None)
             return ChebyDirection(
                 H0s, Hcs, tlist, backward, self._term_rows(self._init_pulses),
                 limit=pk.get("cheby_coeffs_limit", 1e-12), specrange_buffer=pk.get("specrange_buffer", 0.01),

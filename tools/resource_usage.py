@@ -57,7 +57,7 @@ worst = max(spills.values()) if spills else 0
 print(f"\nlargest LDL/STL count in one kernel: {worst}")
 
 # ---- where the local-memory instructions of the C4 instance sit: address histogram of its SASS --------------------------
-KEY = "_ZN2kr18krotov_warp_kernelILi6ELi2ELi256ELi32ELb0ELb0EEEvNS_10WarpParamsE"
+KEY = "_ZN2kr18krotov_warp_kernelILi6ELi2ELi256ELi32ELb0ELb0ELb0EEEvNS_10WarpParamsE"
 k = subprocess.run(["cuobjdump", "-sass", "-fun", KEY, LIB], capture_output=True, text=True).stdout
 ins = []
 for line in k.splitlines():
